@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port, all host threads)
+    python bench.py ... --dump-outputs DIR                   # also write a seeded sample of the output
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d config 2): a synthetic
 TIMIT-TRAIN-sized corpus -- 4620 utterances, lengths U(32000, 64000) samples at 16 kHz,
@@ -39,6 +40,7 @@ N_UTTS, LEN_LO, LEN_HI = 4620, 32000, 64000
 FLOP_PER_CS = 80.0  # 40 FP32 FMA per channel-sample: filterbank + envelope + LPF (SURVEY.md 8d)
 TRAFFIC_1GPU = 11.520e9  # bytes per fused_kernel launch (window-store mode): 4.08 GB read + 7.44 GB written (ncu, DESIGN.md section 5)
 KERNELS_PER_STEP = 2  # ring_cluster_kernel (whole pre-pass of the corpus sizes), fused_kernel (stores the windows)
+DUMP_ROWS = 8192  # --dump-outputs: 8192 x 11 x 128 float32 = 46 MB of the 7.5 GB windows tensor
 
 
 def parse():
@@ -53,7 +55,16 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the side configs (single utterance, 600 s stream, evalnoise)")
     ap.add_argument("--no-verify", action="store_true", help="N > 1: skip the bit-for-bit check against the 1-GPU result")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write DIR/windows.npy: %d seeded rows (sorted, rows in corpus order) of "
+                         "the float32 (N, 11, %d) windows the last timed step stored" % (DUMP_ROWS, C))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the CPU arm times a bounded sample of "
+                 "the corpus and has no output of the whole step to write")
+    return args
 
 
 def dist_env():
@@ -238,6 +249,40 @@ def other_configs(coefs128):
     return out
 
 
+def dump_windows(path, windows, shards, nwin_all, rank):
+    """--dump-outputs: a fixed, seeded sample of the corpus's windows, rows numbered as in the whole corpus.
+    Rank r's `windows` holds the rows of its utterances shards[r]; every sampled row is copied from the rank
+    that computed it, so the file is the same, bit for bit, for any number of GPUs."""
+    import torch
+    import torch.distributed as dist
+    first = np.concatenate([[0], np.cumsum(nwin_all)])
+    rows = np.sort(np.random.default_rng(0).choice(int(first[-1]), size=min(DUMP_ROWS, int(first[-1])), replace=False))
+    owner = np.empty(len(nwin_all), dtype=np.int64)        # utterance -> rank
+    local_first = np.empty(len(nwin_all), dtype=np.int64)  # utterance -> its first row in its rank's `windows`
+    for r, utts in enumerate(shards):
+        owner[utts] = r
+        local_first[utts] = np.cumsum(nwin_all[utts]) - nwin_all[utts]
+    utt = np.searchsorted(first, rows, side="right") - 1
+    src = local_first[utt] + rows - first[utt]
+
+    def of_rank(r):
+        return torch.from_numpy(np.flatnonzero(owner[utt] == r)).to(windows.device)
+
+    sample = torch.zeros((len(rows),) + tuple(windows.shape[1:]), dtype=windows.dtype, device=windows.device)
+    mine = of_rank(rank)
+    sample[mine] = windows[torch.from_numpy(src).to(windows.device)[mine]]
+    if len(shards) > 1:
+        parts = [torch.empty_like(sample) for _ in shards] if rank == 0 else None
+        dist.gather(sample, parts, dst=0)
+        if rank == 0:
+            for r in range(1, len(shards)):
+                sel = of_rank(r)
+                sample[sel] = parts[r][sel]
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "windows.npy"), sample.cpu().numpy())
+
+
 def main():
     args = parse()
     rank, local_rank, world = dist_env()
@@ -284,7 +329,8 @@ def main():
     flat, offsets = synth.corpus_waves_i16(lengths, seed=1)
     total_samples = int(offsets[-1])
     cs_per_step = float(C) * total_samples          # the WHOLE job, whatever the number of GPUs
-    mine = engine.shard_utterances(lengths, world)[rank]
+    shards = engine.shard_utterances(lengths, world)
+    mine = shards[rank]
     my_lengths = lengths[mine]
 
     plan = engine.plan_for(coefs, local_rank)
@@ -356,6 +402,8 @@ def main():
     ms_step = max_over_ranks(t_start.elapsed_ms(t_stop)) / args.steps
     value = cs_per_step / (ms_step * 1e-3)
     windows_head = windows[:64].cpu() if rank == 0 else None
+    if args.dump_outputs:
+        dump_windows(args.dump_outputs, windows, shards, nwin_all, rank)
     del windows, dec, check
 
     # ---- e2e: THE PUBLIC CALL, host int16 waves in, host float32 input tensor out ---------------------
@@ -392,7 +440,7 @@ def main():
         call(out_arr)                     # first call: builds and caches the pipeline, touches `out`
         cold_ms = max_over_ranks((time.perf_counter() - t0) * 1e3)
         call(out_arr)
-        k = max(2, min(args.steps, 5))
+        k = args.steps
         barrier()
         t0 = time.perf_counter()
         for _ in range(k):

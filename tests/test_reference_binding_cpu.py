@@ -1,5 +1,5 @@
-"""The reference's OWN entry points on the drop-in (CPU box: needs /root/reference, skipped on the
-GPU box where it does not exist): after dropin.install() the reference's unmodified f2cnn.py imports,
+"""The reference's OWN entry points on the drop-in (needs a checkout of the original F2CNN tree named by
+F2CNN_REFERENCE; skipped without one): after dropin.install() the reference's unmodified f2cnn.py imports,
 every dispatch name it binds (f2cnn.py:4-9, 27-45) resolves to this package, a late install()
 re-binds the names PlottingProcessing.py:12-15 imported by value, and every public function of the
 shadowed modules has the reference's signature."""
@@ -11,8 +11,9 @@ import types
 
 import pytest
 
-REF = os.environ.get("F2CNN_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "f2cnn.py")), reason="reference tree not present")
+REF = os.environ.get("F2CNN_REFERENCE", "")
+pytestmark = pytest.mark.skipif(not (REF and os.path.isfile(os.path.join(REF, "f2cnn.py"))),
+                                reason="F2CNN_REFERENCE does not name a reference tree")
 
 SHADOWED = ["gammatone.filters", "scripts.processing.GammatoneFiltering", "scripts.processing.EnvelopeExtraction",
             "scripts.processing.InputGenerator", "scripts.processing.LabelDataGenerator",

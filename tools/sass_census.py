@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """SASS census of the SHIPPED library: per kernel, how many of the instructions that prove what the
 code runs on (packed FP32 math, bulk-TMA copies, mbarriers, tensor-core / tensor-memory ops,
-shuffles).  __graft_entry__.build() rewrites profiles/sass_census.txt from the .so it just built,
-so the file can never describe a stale kernel.   usage: tools/sass_census.py [lib.so] [out.txt]"""
+shuffles).  __graft_entry__.build() writes build/sass_census.txt from the .so it just built, so that
+file never describes a stale kernel; run this tool by hand to refresh the committed snapshot
+profiles/sass_census.txt with a kernel change.   usage: tools/sass_census.py [lib.so] [out.txt]"""
 import collections
 import os
 import re
@@ -34,10 +35,10 @@ def census(lib):
     return counts
 
 
-def main():
-    lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "f2cnn_b200", "libf2cnn_b200.so")
-    dst = sys.argv[2] if len(sys.argv) > 2 else os.path.join(ROOT, "profiles", "sass_census.txt")
-    rows = ["# cuobjdump -sass %s: instruction counts per kernel (tools/sass_census.py; rewritten by build())" %
+def main(lib=None, dst=None):
+    lib = lib or os.path.join(ROOT, "f2cnn_b200", "libf2cnn_b200.so")
+    dst = dst or os.path.join(ROOT, "profiles", "sass_census.txt")
+    rows = ["# cuobjdump -sass %s: instruction counts per kernel (tools/sass_census.py)" %
             os.path.relpath(lib, ROOT), "# kernel | total | " + " ".join(MNEMONICS)]
     for kernel, c in census(lib).items():
         rows.append("%s | %d | %s" % (kernel, c["_all"], " ".join("%s=%d" % (m, c[m]) for m in MNEMONICS if c[m])))
@@ -47,4 +48,4 @@ def main():
 
 
 if __name__ == "__main__":
-    print(main())
+    print(main(*sys.argv[1:3]))
