@@ -948,6 +948,8 @@ int f2_cnn_create(int device, const float* const* arrays, int dots, int channels
     cudaDeviceProp prop;
     F2_CUDA(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) return fail(F2_ERR_UNSUPPORTED, "device %d is sm_%d%d; tcgen05 needs sm_100a", device, prop.major, prop.minor);
+    // the kernels' shared-memory limit is a per-device attribute: set it for the device this network lives on
+    F2_CUDA(f2::configure_cnn_kernels());
     // Keras order: conv kernels HWIO + biases (Training.py:95-108), dense kernels (in, out) + biases (:111-114)
     const float *k1 = arrays[0], *b1 = arrays[1], *k2 = arrays[2], *b2 = arrays[3], *k3 = arrays[4], *b3 = arrays[5],
                 *k4 = arrays[6], *b4 = arrays[7], *W5 = arrays[8], *b5 = arrays[9], *W6 = arrays[10], *b6 = arrays[11];

@@ -657,18 +657,18 @@ size_t cnn_workspace_bytes(long long chunk_frames) {
     return ((pooled + 255) / 256 + (feat + 255) / 256) * 256 + 256;
 }
 
+cudaError_t configure_cnn_kernels() {
+    using namespace cnn;
+    cudaError_t e = cudaFuncSetAttribute(cnn_front_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FrontSmem::total);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cnn_mid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MidSmem::total);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cnn_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DenseSmem::total);
+    return e;
+}
+
 cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, long long frame0, long long n_frames,
                                long long chunk_frames, float* scores, int* bad_flag, int* status, void* workspace,
                                int sm_count, cudaStream_t stream) {
     using namespace cnn;
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(cnn_front_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FrontSmem::total);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(cnn_mid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MidSmem::total);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(cnn_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DenseSmem::total);
-        if (e != cudaSuccess) return e;
-        configured = true;
-    }
     uint8_t* pooled2 = (uint8_t*)(((size_t)workspace + 255) / 256 * 256);
     const size_t pooled_bytes = ((size_t)chunk_frames * 4 * kPool2 * 16 + 255) / 256 * 256;
     __nv_bfloat16* feat = (__nv_bfloat16*)(pooled2 + pooled_bytes);

@@ -23,6 +23,10 @@ struct CnnWeights {
 };
 
 size_t cnn_workspace_bytes(long long chunk_frames);
+// Raises the dynamic shared-memory limit of the three CNN kernels on the CURRENT device.  A function
+// attribute belongs to one device's copy of the kernel, so every device that runs the network needs this
+// once (f2_cnn_create calls it under its device guard).
+cudaError_t configure_cnn_kernels();
 // Frames frame0 .. frame0 + n_frames - 1 of the time-major envelope env_t ([rows][128] float32): frame i =
 // rows i + k*step, k < 11 (Evaluating.py:70-78).  scores: [n_frames][2] float32 softmax.
 cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, long long frame0, long long n_frames,
