@@ -14,6 +14,7 @@ F2_I16, F2_F32, F2_F64 = 0, 1, 2
 F2_ROWS_ENVELOPE, F2_ROWS_HILBERT, F2_ROWS_LOWPASS = 0, 1, 2
 F2_ERR_INVALID, F2_ERR_CUDA, F2_ERR_WORKSPACE, F2_ERR_UNSUPPORTED, F2_ERR_INDEX = 1, 2, 3, 4, 5
 ABI_VERSION = 6
+F2_PLAN_FLOAT64_SECTIONS = 1
 
 
 class F2Error(RuntimeError):
@@ -63,6 +64,11 @@ SIGNATURES = {
                                       ctypes.POINTER(ctypes.c_void_p)]),
     "f2_bank_check": (ctypes.c_int, [ctypes.POINTER(ctypes.c_double), ctypes.c_int, ctypes.POINTER(ctypes.c_double),
                                      ctypes.POINTER(ctypes.c_int)]),
+    "f2_plan_create_ex": (ctypes.c_int, [ctypes.POINTER(ctypes.c_double), ctypes.c_int, ctypes.c_int, ctypes.c_uint,
+                                         ctypes.POINTER(ctypes.c_void_p)]),
+    "f2_bank_check_groups": (ctypes.c_int, [ctypes.POINTER(ctypes.c_double), ctypes.c_int,
+                                            ctypes.POINTER(ctypes.c_double)]),
+    "f2_plan_float64_groups": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_ubyte), ctypes.c_int]),
     "f2_plan_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "f2_plan_channels": (ctypes.c_int, [ctypes.c_void_p]),
     "f2_plan_set_warmup": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int]),

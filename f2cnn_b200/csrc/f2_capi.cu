@@ -57,6 +57,10 @@ int round_up_tile(double v) { return (int)(ceil(v / f2::kTile) * f2::kTile); }
 constexpr float kDirectMinCyGfb = 0.25f;
 constexpr float kDirectMinCyEnv = 0.035f;
 constexpr double kDirectCost = 0.85;  // time per sample of a direct-form group / delta-form group (measured)
+// the same for a FORM 2 (float64) group: 20.3 ms for the float64 group of a 16 kHz / 128 ch / LOW_FREQ 20 bank over
+// the bench corpus against ~11.7 ms for the same group in float32 delta form (B200 at 1000 W,
+// tools/float64_sections_bench.py, profiles/r03b_float64_sections.log)
+constexpr double kForm2Cost = 1.75;
 
 // Per-stage float32 rounding whose SUM over the four stages is as close to 4*c as the
 // float32 lattice allows.  The four sections share their poles, so the first-order error of
@@ -141,16 +145,23 @@ double probe_channel(const ProbeChan& p, const float* x, int n, double loudest_r
     return scale > 0.0 ? err / scale : 0.0;
 }
 
-// worst predicted error of the bank, in units of the 1e-4 tolerance
-double bank_float32_error(const double* coefs, int C, int* worst_channel) {
-    constexpr int kProbeLen = 8192, kChannels = 6;
-    constexpr double kAmp = 8000.0;
-    // the channels nearest to z = 1
-    std::vector<int> order((size_t)C);
-    for (int c = 0; c < C; ++c) order[(size_t)c] = c;
+constexpr int kProbeChannels = 6;
+
+// the (up to kProbeChannels) channels of [c0, c1) nearest to z = 1
+std::vector<int> nearest_to_one(const double* coefs, int c0, int c1) {
+    std::vector<int> order;
+    for (int c = c0; c < c1; ++c) order.push_back(c);
     auto cy_of = [&](int c) { return 1.0 + (coefs[(size_t)c * 10 + 7] + coefs[(size_t)c * 10 + 8]) / coefs[(size_t)c * 10 + 6]; };
     std::sort(order.begin(), order.end(), [&](int a, int b) { return cy_of(a) < cy_of(b); });
-    order.resize((size_t)std::min(C, kChannels));
+    order.resize((size_t)std::min(c1 - c0, kProbeChannels));
+    return order;
+}
+
+// worst predicted error of the channels `order`, in units of the 1e-4 tolerance
+double probe_float32_error(const double* coefs, int C, const std::vector<int>& order, int* worst_channel) {
+    constexpr int kProbeLen = 8192;
+    constexpr double kAmp = 8000.0;
+    auto cy_of = [&](int c) { return 1.0 + (coefs[(size_t)c * 10 + 7] + coefs[(size_t)c * 10 + 8]) / coefs[(size_t)c * 10 + 6]; };
     std::vector<float> x((size_t)kProbeLen);
     double worst = 0.0;
     if (worst_channel) *worst_channel = order.empty() ? 0 : order[0];
@@ -199,6 +210,26 @@ double bank_float32_error(const double* coefs, int C, int* worst_channel) {
     return worst;
 }
 
+// worst predicted error of the bank: its channels nearest to z = 1
+double bank_float32_error(const double* coefs, int C, int* worst_channel) {
+    return probe_float32_error(coefs, C, nearest_to_one(coefs, 0, C), worst_channel);
+}
+
+// the same per group of 32 channels (one warp of the fused kernel): the group's channels nearest to z = 1
+void group_float32_errors(const double* coefs, int C, double* per_group) {
+    for (int g = 0; g * 32 < C; ++g)
+        per_group[g] = probe_float32_error(coefs, C, nearest_to_one(coefs, g * 32, std::min(C, g * 32 + 32)), nullptr);
+}
+
+int check_coefs(const double* coefs, int n_channels) {
+    for (int c = 0; c < n_channels; ++c) {
+        const double* k = coefs + (size_t)c * 10;
+        if (!(k[6] != 0.0) || !(k[0] != 0.0) || !(k[9] > 0.0) || !isfinite(k[9]))
+            return fail(F2_ERR_INVALID, "channel %d: A0 == 0, B0 == 0 or gain <= 0", c);
+    }
+    return F2_OK;
+}
+
 }  // namespace
 
 // error channel of the other translation units of the library (f2_host.cpp); not exported
@@ -220,7 +251,19 @@ struct f2_plan {
     long long id = 0;
     int w_imag = 0, w_edge = 0, w_casc = 0;
     double min_neg_log_r = 0.0;
+    double* d_chan64 = nullptr;  // [kNumChanPar64][c_pad] float64 block of the FORM 2 groups (null: none)
+    std::vector<unsigned char> f64_group;  // per group of 32 channels: runs FORM 2
+    int n_f64 = 0;
 };
+
+namespace {
+// time per sample of a channel group relative to a delta-form group: direct form kDirectCost, FORM 2 kForm2Cost
+double group_cost(const f2_plan* plan, int cb) {
+    const float cy = plan->h_chan[(size_t)f2::P_FORM * plan->c_pad + (size_t)cb * 32];
+    if (cy == f2::kForm2Marker) return kForm2Cost;
+    return cy >= kDirectMinCyEnv ? kDirectCost : 1.0;
+}
+}  // namespace
 
 struct f2_batch {
     f2_plan* plan = nullptr;
@@ -236,6 +279,8 @@ struct f2_batch {
     // channel group costs the same per sample); null when the two decompositions coincide
     f2::Item* d_items_uniform = nullptr;
     long long n_items_uniform = 0;
+    // the last n_items_f64 (n_items_uniform_f64) of each list belong to FORM 2 groups
+    long long n_items_f64 = 0, n_items_uniform_f64 = 0;
     long long total_samples = 0, total_frames = 0, total_ring = 0;
     int max_n = 0;
     int min_log2 = 0, max_log2 = 0;
@@ -256,17 +301,25 @@ int f2_lowpass_coefficients(double cutoff_hz, double* b0, double* a1) {
 
 int f2_bank_check(const double* coefs, int n_channels, double* predicted, int* worst_channel) {
     if (!coefs || n_channels <= 0 || !predicted) return fail(F2_ERR_INVALID, "f2_bank_check: bad arguments");
-    for (int c = 0; c < n_channels; ++c) {
-        const double* k = coefs + (size_t)c * 10;
-        if (!(k[6] != 0.0) || !(k[0] != 0.0) || !(k[9] > 0.0) || !isfinite(k[9]))
-            return fail(F2_ERR_INVALID, "channel %d: A0 == 0, B0 == 0 or gain <= 0", c);
-    }
+    if (const int rc = check_coefs(coefs, n_channels)) return rc;
     *predicted = bank_float32_error(coefs, n_channels, worst_channel);
     return F2_OK;
 }
 
+int f2_bank_check_groups(const double* coefs, int n_channels, double* per_group) {
+    if (!coefs || n_channels <= 0 || !per_group) return fail(F2_ERR_INVALID, "f2_bank_check_groups: bad arguments");
+    if (const int rc = check_coefs(coefs, n_channels)) return rc;
+    group_float32_errors(coefs, n_channels, per_group);
+    return F2_OK;
+}
+
 int f2_plan_create(const double* coefs, int n_channels, int device, f2_plan** out) {
+    return f2_plan_create_ex(coefs, n_channels, device, 0u, out);
+}
+
+int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned flags, f2_plan** out) {
     if (!coefs || !out || n_channels <= 0) return fail(F2_ERR_INVALID, "f2_plan_create: bad arguments");
+    if (flags & ~(unsigned)F2_PLAN_FLOAT64_SECTIONS) return fail(F2_ERR_INVALID, "f2_plan_create_ex: unknown flags 0x%x", flags);
     int ndev = 0;
     F2_CUDA(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(F2_ERR_INVALID, "device %d out of range (%d visible)", device, ndev);
@@ -328,7 +381,32 @@ int f2_plan_create(const double* coefs, int n_channels, int device, f2_plan** ou
         const float scale = (float)std::min(1.0, min_nlr / nlr * (1.0 + 1e-6));
         for (int c = g0; c < g0 + 32; ++c) par[(size_t)f2::P_WSCALE * c_pad + c] = scale;
     }
-    {
+    // F2_PLAN_FLOAT64_SECTIONS: in a bank f2_bank_check refuses, the groups predicted to leave the tolerance in
+    // float32 run FORM 2.  A bank it accepts keeps float32 everywhere, so that the flag never changes its
+    // outputs.  A refused bank always flags a group: its worst channel is among the probed channels of its
+    // own group, so that group's prediction is at least the bank's.
+    const int n_groups = c_pad / 32;
+    std::vector<unsigned char> f64_group((size_t)n_groups, 0);
+    std::vector<double> par64;
+    if ((flags & F2_PLAN_FLOAT64_SECTIONS) && bank_float32_error(coefs, C, nullptr) > 1.0) {
+        std::vector<double> per_group((size_t)n_groups);
+        group_float32_errors(coefs, C, per_group.data());
+        for (int g = 0; g < n_groups; ++g) f64_group[(size_t)g] = per_group[(size_t)g] > 1.0;
+        par64.assign((size_t)f2::kNumChanPar64 * c_pad, 0.0);
+        for (int c = 0; c < C; ++c) {
+            if (!f64_group[(size_t)(c / 32)]) continue;
+            const double* k = coefs + (size_t)c * 10;
+            const double a0n = k[0] / k[6];
+            par64[(size_t)f2::P64_G4 * c_pad + c] = a0n * a0n * a0n * a0n / k[9];
+            for (int s = 0; s < 4; ++s) par64[(size_t)(f2::P64_Z + s) * c_pad + c] = k[1 + s] / k[0];
+            par64[(size_t)f2::P64_B1 * c_pad + c] = k[7] / k[6];
+            par64[(size_t)f2::P64_B2 * c_pad + c] = k[8] / k[6];
+        }
+        for (int c = 0; c < c_pad; ++c)
+            if (f64_group[(size_t)(c / 32)]) par[(size_t)f2::P_FORM * c_pad + c] = f2::kForm2Marker;
+    }
+    const int n_f64 = (int)std::count(f64_group.begin(), f64_group.end(), (unsigned char)1);
+    if (!(flags & F2_PLAN_FLOAT64_SECTIONS)) {
         // a bank whose float32 result would leave the stated tolerance is refused, not answered quietly
         int bad = 0;
         const double predicted = bank_float32_error(coefs, C, &bad);
@@ -348,6 +426,8 @@ int f2_plan_create(const double* coefs, int n_channels, int device, f2_plan** ou
     p->C = C;
     p->c_pad = c_pad;
     p->min_neg_log_r = min_nlr;
+    p->f64_group = f64_group;
+    p->n_f64 = n_f64;
     // truncated-history lengths.  The cascade's impulse response decays like t^3 r^t, so for an
     // input that adds up coherently (a tone on the slowest channel's centre) the part of the steady
     // state older than W samples is Gamma(4, -W ln r)/6 of the whole: 7e-7 at 21.5/-ln r (w_imag),
@@ -364,10 +444,16 @@ int f2_plan_create(const double* coefs, int n_channels, int device, f2_plan** ou
     if (e == cudaSuccess) e = cudaMalloc(&p->d_scan_mats, mats.size() * sizeof(float));
     if (e == cudaSuccess)
         e = cudaMemcpy(p->d_scan_mats, mats.data(), mats.size() * sizeof(float), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && n_f64 > 0) {
+        e = cudaMalloc(&p->d_chan64, par64.size() * sizeof(double));
+        if (e == cudaSuccess)
+            e = cudaMemcpy(p->d_chan64, par64.data(), par64.size() * sizeof(double), cudaMemcpyHostToDevice);
+    }
     if (e == cudaSuccess) e = f2::init_twiddles(0);
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         if (p->d_chan) cudaFree(p->d_chan);
+        if (p->d_chan64) cudaFree(p->d_chan64);
         if (p->d_scan_mats) cudaFree(p->d_scan_mats);
         delete p;
         return fail(F2_ERR_CUDA, "plan upload: %s", cudaGetErrorString(e));
@@ -380,12 +466,22 @@ int f2_plan_destroy(f2_plan* plan) {
     if (!plan) return F2_OK;
     DeviceGuard guard(plan->device);
     if (plan->d_chan) cudaFree(plan->d_chan);
+    if (plan->d_chan64) cudaFree(plan->d_chan64);
     if (plan->d_scan_mats) cudaFree(plan->d_scan_mats);
     delete plan;
     return F2_OK;
 }
 
 int f2_plan_channels(const f2_plan* plan) { return plan ? plan->C : 0; }
+
+int f2_plan_float64_groups(const f2_plan* plan, unsigned char* mask, int n_groups) {
+    if (!plan || n_groups < 0 || (n_groups > 0 && !mask)) {
+        fail(F2_ERR_INVALID, "f2_plan_float64_groups: bad arguments");
+        return -1;
+    }
+    for (int g = 0; g < n_groups; ++g) mask[g] = g < (int)plan->f64_group.size() ? plan->f64_group[(size_t)g] : 0;
+    return plan->n_f64;
+}
 
 int f2_plan_set_warmup(f2_plan* plan, int w_imag, int w_edge, int w_casc) {
     if (!plan) return fail(F2_ERR_INVALID, "null plan");
@@ -488,8 +584,7 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
         std::vector<double> cost((size_t)cblocks), W((size_t)cblocks);
         for (int cb = 0; cb < cblocks; ++cb) {
             const size_t c0 = (size_t)cb * 32;
-            const bool direct = plan->h_chan[(size_t)f2::P_FORM * plan->c_pad + c0] >= kDirectMinCyEnv;
-            cost[(size_t)cb] = direct ? kDirectCost : 1.0;
+            cost[(size_t)cb] = group_cost(plan, cb);
             W[(size_t)cb] = (double)f2::group_warmup(plan->w_casc, plan->h_chan[(size_t)f2::P_WSCALE * plan->c_pad + c0]) + 2048.0;
         }
         auto seg_at = [&](double T, int cb) { return std::max(2048.0, T / cost[(size_t)cb] - W[(size_t)cb]); };
@@ -544,7 +639,7 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
         for (int cb = 0; cb < cblocks; ++cb) {
             const size_t c0 = (size_t)cb * 32;
             const float wscale = plan->h_chan[(size_t)f2::P_WSCALE * plan->c_pad + c0];
-            gcost[(size_t)cb] = plan->h_chan[(size_t)f2::P_FORM * plan->c_pad + c0] >= kDirectMinCyEnv ? kDirectCost : 1.0;
+            gcost[(size_t)cb] = group_cost(plan, cb);
             gwarm[(size_t)cb] = 0.6 * (f2::group_warmup(plan->w_imag, wscale) + f2::group_warmup(plan->w_edge, wscale));
         }
         const bool whole_utterances = seg >= ((long long)1 << 40);
@@ -576,6 +671,15 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
     std::vector<f2::Item> items = build_items(seg_of, !equal_cost);
     std::vector<f2::Item> items_uniform;
     if (equal_cost) items_uniform = build_items(seg_same, true);
+    // the items of FORM 2 groups go last: the second launch (launch_fused64) runs them
+    auto split_form2 = [&](std::vector<f2::Item>& v) {
+        if (plan->n_f64 == 0) return 0LL;
+        auto mid = std::stable_partition(v.begin(), v.end(),
+                                         [&](const f2::Item& it) { return !plan->f64_group[(size_t)it.cblock]; });
+        return (long long)(v.end() - mid);
+    };
+    b->n_items_f64 = split_form2(items);
+    b->n_items_uniform_f64 = split_form2(items_uniform);
     b->n_items = (long long)items.size();
     b->n_items_uniform = (long long)items_uniform.size();
     b->n_whole = whole / units * cblocks;  // same utterance count, in CTAs
@@ -652,6 +756,11 @@ static size_t ws_edge_bytes(const f2_batch* b) {
     return align_up((size_t)b->n_utts * (size_t)b->plan->C * 8 * sizeof(float), 256);
 }
 
+// float64 edge residuals of the FORM 2 groups (none without such groups)
+static size_t ws_edge64_bytes(const f2_batch* b) {
+    return b->plan->n_f64 ? align_up((size_t)b->n_utts * (size_t)b->plan->C * 8 * sizeof(double), 256) : 0;
+}
+
 // Ring sections of the workspace: xz (two floats per ring sample) always; the two FFT scratch rings (the
 // second doubles as the per-utterance injection table) only when some utterance needs them -- a batch whose
 // rings are all transformed by the cluster kernel and read shared injection tables (every corpus batch)
@@ -663,7 +772,7 @@ static int ws_ring_units(const f2_batch* b) {
 
 size_t f2_batch_workspace_bytes(const f2_batch* b, int want_full_gfb, int want_full_env) {
     if (!b) return 0;
-    size_t s = (size_t)ws_ring_units(b) * ws_ring_bytes(b->total_ring) + ws_edge_bytes(b);
+    size_t s = (size_t)ws_ring_units(b) * ws_ring_bytes(b->total_ring) + ws_edge_bytes(b) + ws_edge64_bytes(b);
     if (want_full_gfb) s += ws_full_bytes(b);
     if (want_full_env) s += ws_full_bytes(b);
     return s + 256;
@@ -715,7 +824,8 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     float2* xz = (float2*)(units == 4 ? ws + rb : ws);
     float* G = units == 4 ? (float*)(ws + 3 * rb) : nullptr;
     float* edge = (float*)(ws + (size_t)units * rb);
-    char* cur = ws + (size_t)units * rb + ws_edge_bytes(b);
+    double* edge64 = (double*)(ws + (size_t)units * rb + ws_edge_bytes(b));
+    char* cur = ws + (size_t)units * rb + ws_edge_bytes(b) + ws_edge64_bytes(b);
     float* gfb_t = nullptr;
     float* env_t = a->env_t;
     if (want_gfb) {
@@ -762,6 +872,8 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     fp.win_off = reinterpret_cast<const long long*>(a->win_offsets);
     fp.win_dots = a->win_dots;
     fp.edge = nullptr;
+    fp.chan64 = plan->d_chan64;
+    fp.edge64 = nullptr;
     if (need_env && b->n_items > b->n_whole) {
         // time-chunked batch: the edge residuals are per utterance, compute them once instead of
         // in every chunk.  Few (utterance, channel) pairs -> chunked scan (low latency), many ->
@@ -774,6 +886,9 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
             F2_CUDA(f2::launch_edge(b->d_utts, b->n_utts, plan->d_chan, plan->C, plan->c_pad, xz, plan->w_edge, edge,
                                     stream));
         fp.edge = edge;
+        if (plan->n_f64)
+            F2_CUDA(f2::launch_edge64(b->d_utts, b->n_utts, plan->d_chan, plan->d_chan64, plan->C, plan->c_pad, xz,
+                                      plan->w_edge, edge64, stream));
     }
     fp.C = plan->C;
     fp.c_pad = plan->c_pad;
@@ -793,7 +908,15 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     // low-pass warm-up of a mid-signal chunk: |a1|^W < 1e-7
     fp.w_lpf = a->lpf ? round_up_tile(log(1e-7) / log(-a1)) : 0;
     if (a->ev_fused_start) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_start, stream));
-    F2_CUDA(f2::launch_fused(fp, (int)(uniform_chunks ? b->n_items_uniform : b->n_items), stream));
+    const long long n_items = uniform_chunks ? b->n_items_uniform : b->n_items;
+    const long long n_f64 = uniform_chunks ? b->n_items_uniform_f64 : b->n_items_f64;
+    F2_CUDA(f2::launch_fused(fp, (int)(n_items - n_f64), stream));
+    if (n_f64 > 0) {
+        f2::FusedParams fp64 = fp;
+        fp64.items = fp.items + (n_items - n_f64);
+        fp64.edge64 = fp.edge ? edge64 : nullptr;
+        F2_CUDA(f2::launch_fused64(fp64, (int)n_f64, stream));
+    }
     if (a->ev_fused_stop) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_stop, stream));
 
     if (a->gfb && !direct_cn)

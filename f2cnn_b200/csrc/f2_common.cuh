@@ -37,6 +37,14 @@ constexpr int kNumChanPar = 19;   // floats per channel in the parameter block
 //                    the 100 Hz channels the plan's lengths are derived from
 enum ChanPar { P_G4 = 0, P_Z = 1, P_CQ = 5, P_NCY = 9, P_NB1 = 13, P_FORM = 17, P_WSCALE = 18 };
 
+// Groups whose float32 error is predicted above the tolerance (f2_plan_create_ex with
+// F2_PLAN_FLOAT64_SECTIONS) run their cascade in float64 (FORM 2): their group_cy entry holds this
+// marker, and their exact design coefficients live in a second block of doubles, par64[i * c_pad + c]:
+//   0 g4 = A0^4/gain   1..4 z[k] = A1k/A0   5 b1 = B1/B0   6 b2 = B2/B0
+constexpr float kForm2Marker = -1.0f;
+constexpr int kNumChanPar64 = 7;
+enum ChanPar64 { P64_G4 = 0, P64_Z = 1, P64_B1 = 5, P64_B2 = 6 };
+
 // A plan-wide truncated-history length scaled to one channel group, in whole tiles (never longer than
 // the plan's, never shorter than one tile).  Host and device use the same expression.
 __host__ __device__ __forceinline__ int group_warmup(int w_plan, float wscale) {

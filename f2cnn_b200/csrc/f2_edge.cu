@@ -94,6 +94,67 @@ cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, int 
     return cudaGetLastError();
 }
 
+// ---- FORM 2 groups: float64 direct-form residuals ---------------------------------------------
+// One CTA per (utterance, group of 32 channels); groups that are not FORM 2 leave at once.  The same
+// recurrence as cascade_real / edge_residuals of the fused kernel's FORM 2, from zero state w_edge
+// samples before the end.
+__global__ void __launch_bounds__(32) edge_kernel64(const UttDesc* utts, const float* __restrict__ chan,
+                                                    const double* __restrict__ chan64, int C, int c_pad,
+                                                    const float2* __restrict__ xz, int w_edge,
+                                                    double* __restrict__ edge) {
+    const UttDesc ut = utts[blockIdx.x];
+    const int c = blockIdx.y * 32 + threadIdx.x;
+    if (chan[P_FORM * c_pad + blockIdx.y * 32] != kForm2Marker || c >= C || ut.n <= 0) return;
+    double z[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) z[i] = chan64[(P64_Z + i) * c_pad + c];
+    const double b1 = chan64[P64_B1 * c_pad + c], b2 = chan64[P64_B2 * c_pad + c];
+    double y[4] = {0.0, 0.0, 0.0, 0.0}, y2[4] = {0.0, 0.0, 0.0, 0.0};
+    double up = 0.0;
+    const int n = ut.n;
+    const int t0 = n - w_edge > 0 ? n - w_edge : 0;
+    const float2* src = xz + ut.ring_off;
+    if (ut.N2 > 2) {
+#pragma unroll 4
+        for (int t = t0; t < n; ++t) {
+            double u = __ldg(&src[t].x), upi = up;
+            up = u;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const double yn = fma(-b1, y[i], fma(-b2, y2[i], fma(z[i], upi, u)));
+                upi = y[i];
+                y2[i] = y[i];
+                y[i] = yn;
+                u = yn;
+            }
+        }
+    }
+    double e0[4], e1[4];
+    double uprev = up;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const bool real_only = ut.N2 <= 2;
+        e0[i] = real_only ? 0.0 : fma(b1, y[i], b2 * y2[i]) - z[i] * uprev;
+        e1[i] = real_only ? 0.0 : b2 * y[i];
+        uprev = y[i];
+    }
+    const bool n_odd = (n & 1) != 0;  // (t - n) odd -> e0 multiplies G[t]
+    double* o = edge + ((size_t)blockIdx.x * C + c) * 8;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        o[i] = n_odd ? e0[i] : e1[i];
+        o[4 + i] = n_odd ? e1[i] : e0[i];
+    }
+}
+
+cudaError_t launch_edge64(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
+                          const float2* xz, int w_edge, double* edge, cudaStream_t stream) {
+    if (n_utts <= 0) return cudaSuccess;
+    dim3 grid(n_utts, (C + 31) / 32);
+    edge_kernel64<<<grid, 32, 0, stream>>>(utts, chan, chan64, C, c_pad, xz, w_edge, edge);
+    return cudaGetLastError();
+}
+
 // ---- scan version ----------------------------------------------------------------------------
 constexpr int kScanWarps = 4;                  // channels per CTA (they share the staged window)
 constexpr int kScanPitch = kScanBlock + 1;     // floats per lane block in shared memory (bank spread)

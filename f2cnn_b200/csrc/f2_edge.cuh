@@ -12,6 +12,10 @@ constexpr int kScanWindow = 32 * kScanBlock;  // 2048 samples: the last w_edge s
 // seq: one thread per channel runs the real cascade over the last w_edge samples.
 cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, int C, int c_pad, const float2* xz,
                         int w_edge, float* edge, cudaStream_t stream);
+// FORM 2 groups (P_FORM == kForm2Marker): float64 sequential pass over the last w_edge samples into a
+// float64 table [utt][C][8] (same layout); the entries of other groups are not written.
+cudaError_t launch_edge64(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
+                          const float2* xz, int w_edge, double* edge, cudaStream_t stream);
 // scan: one warp per (utterance, channel); lane = block of 64 samples run from zero state;
 // the 8-state cascade carries are composed across lanes with precomputed block transition
 // powers M^(2^d) (lower block-triangular, 2x2 blocks per biquad) and warp shuffles.

@@ -26,6 +26,8 @@
 // The delta form keeps float32 round-off and coefficient quantisation harmless for poles
 // 0.039 rad from z=1 (SURVEY.md H2); the direct form is used where 1+B1+B2 = |1-pole|^2 is
 // large enough for it to be as accurate (FusedParams::direct_min_cy, DESIGN.md section 3).
+// FORM 2 (float64 direct form, exact coefficients) runs the groups a plan created with
+// F2_PLAN_FLOAT64_SECTIONS found float32 unable to hold to the tolerance, in fused_kernel64 (DESIGN.md 2 (iii)).
 // Every stage is computed WITHOUT its common numerator gain a0 = A0/gain^(1/4): stage k holds
 // y_k / a0^k, and the single factor a0^4 = A0^4/gain is applied where a value leaves the
 // kernel (folded into the low-pass b0 when the low-pass is on).  In delta form that is 40
@@ -200,6 +202,159 @@ __device__ __forceinline__ void edge_residuals(const Coef& k, const State& s, fl
     }
 }
 
+// ---- FORM 2: float64 direct-form sections (groups float32 cannot hold to the tolerance) ----------------
+// Exact design coefficients (no dither), y = in - b1*y[t-1] - b2*y[t-2] with the same zn = z' - b1 trick as
+// FORM 1.  Ring samples and G stay float and are widened when read; the injection e*G is formed in double;
+// g4 is applied in double, so the value that leaves the cascade is the float of the scaled output and the
+// float code after it (magnitude, low-pass, stores) runs with a unit scale.
+struct Coef64 {
+    double z[4];
+    double nb1, nb2;  // -b1, -b2
+    double zn[3];     // z[i+1] - b1
+    double gd;        // A0^4/gain
+    float g4;         // 1: the float-side output scale of run_tile
+};
+
+struct State64 {
+    double yr[4], yi[4];    // y[t-1]
+    double qr[4], qi[4];    // y[t-2]
+    double upr, upi;        // previous stage-1 input
+    float l;
+    float wprev;
+};
+
+__device__ __forceinline__ void reset(State64& s) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) s.yr[i] = s.yi[i] = s.qr[i] = s.qi[i] = 0.0;
+    s.upr = s.upi = 0.0;
+    s.l = 0.f;
+    s.wprev = 0.f;
+}
+
+template <int FORM>
+__device__ __forceinline__ float2 cascade(const Coef64& k, State64& s, float2 u, float g, const double (&e)[4]) {
+    const double ur = u.x, ui = u.y, gd = g;
+    double inr = fma(k.z[0], s.upr, ur);
+    double ini = fma(e[0], gd, fma(k.z[0], s.upi, ui));
+    s.upr = ur;
+    s.upi = ui;
+    double yr = 0.0, yi = 0.0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const double ar = fma(k.nb2, s.qr[i], inr), ai = fma(k.nb2, s.qi[i], ini);
+        const double yor = s.yr[i], yoi = s.yi[i];
+        yr = fma(k.nb1, yor, ar);
+        yi = fma(k.nb1, yoi, ai);
+        if (i < 3) {
+            inr = fma(k.zn[i], yor, ar);
+            ini = fma(e[i + 1], gd, fma(k.zn[i], yoi, ai));
+        }
+        s.qr[i] = yor;
+        s.qi[i] = yoi;
+        s.yr[i] = yr;
+        s.yi[i] = yi;
+    }
+    return make_float2((float)(k.gd * yr), (float)(k.gd * yi));
+}
+
+template <int FORM>
+__device__ __forceinline__ void cascade_real(const Coef64& k, State64& s, float u) {
+    const double ur = u;
+    double in = fma(k.z[0], s.upr, ur);
+    s.upr = ur;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const double a = fma(k.nb2, s.qr[i], in);
+        const double yo = s.yr[i];
+        if (i < 3) in = fma(k.zn[i], yo, a);
+        s.qr[i] = yo;
+        s.yr[i] = fma(k.nb1, yo, a);
+    }
+}
+
+template <int FORM>
+__device__ __forceinline__ void cascade_imag(const Coef64& k, State64& s, float u, float g, const double (&e)[4]) {
+    const double ui = u, gd = g;
+    double in = fma(e[0], gd, fma(k.z[0], s.upi, ui));
+    s.upi = ui;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const double a = fma(k.nb2, s.qi[i], in);
+        const double yo = s.yi[i];
+        if (i < 3) in = fma(e[i + 1], gd, fma(k.zn[i], yo, a));
+        s.qi[i] = yo;
+        s.yi[i] = fma(k.nb1, yo, a);
+    }
+}
+
+// e0 = b1*y[n-1] + b2*y[n-2] - z_k*u[n-1],  e1 = b2*y[n-1]  (as FORM 1, in double)
+template <int FORM>
+__device__ __forceinline__ void edge_residuals(const Coef64& k, const State64& s, double (&e0)[4], double (&e1)[4]) {
+    double uprev = s.upr;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        e0[i] = -fma(k.nb1, s.yr[i], k.nb2 * s.qr[i]) - k.z[i] * uprev;
+        e1[i] = -k.nb2 * s.yr[i];
+        uprev = s.yr[i];
+    }
+}
+
+// Coefficients of this thread's channel (inactive lanes: zeros, as the float forms do)
+template <int FORM>
+__device__ __forceinline__ void load_coef(const FusedParams& p, int c, bool active, Coef& k) {
+    const float* cp = p.chan + (active ? c : 0);
+    const float on = active ? 1.f : 0.f;
+    k.g4 = on * cp[P_G4 * p.c_pad];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const float z = on * cp[(P_Z + i) * p.c_pad];
+        const float cq = on * (FORM == 1 ? -cp[(P_CQ + i) * p.c_pad] : cp[(P_CQ + i) * p.c_pad]);
+        const float ncy = on * cp[((FORM == 1 ? P_NB1 : P_NCY) + i) * p.c_pad];
+        k.z[i] = make_float2(z, z);
+        k.cq[i] = make_float2(cq, cq);
+        k.ncy[i] = make_float2(ncy, ncy);
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        const float zn = FORM == 1 ? k.z[i + 1].x + k.ncy[i].x : 0.f;
+        k.zn[i] = make_float2(zn, zn);
+    }
+}
+
+template <int FORM>
+__device__ __forceinline__ void load_coef(const FusedParams& p, int c, bool active, Coef64& k) {
+    const double* cp = p.chan64 + (active ? c : 0);
+    const double on = active ? 1.0 : 0.0;
+    k.gd = on * cp[P64_G4 * p.c_pad];
+    k.g4 = 1.f;
+    k.nb1 = -on * cp[P64_B1 * p.c_pad];
+    k.nb2 = -on * cp[P64_B2 * p.c_pad];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) k.z[i] = on * cp[(P64_Z + i) * p.c_pad];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) k.zn[i] = k.z[i + 1] + k.nb1;
+}
+
+// Time-chunked batches: this channel's edge residuals from the per-utterance table
+__device__ __forceinline__ void load_edge(const FusedParams& p, int utt, int c, float (&ee)[4], float (&eo)[4]) {
+    const float4* e = reinterpret_cast<const float4*>(p.edge + ((size_t)utt * p.C + c) * 8);
+    const float4 v0 = __ldg(e), v1 = __ldg(e + 1);
+    ee[0] = v0.x; ee[1] = v0.y; ee[2] = v0.z; ee[3] = v0.w;
+    eo[0] = v1.x; eo[1] = v1.y; eo[2] = v1.z; eo[3] = v1.w;
+}
+
+__device__ __forceinline__ void load_edge(const FusedParams& p, int utt, int c, double (&ee)[4], double (&eo)[4]) {
+    const double* e = p.edge64 + ((size_t)utt * p.C + c) * 8;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        ee[i] = __ldg(e + i);
+        eo[i] = __ldg(e + 4 + i);
+    }
+}
+
+template <int FORM> struct SectionTypes { using K = Coef; using S = State; using E = float; };
+template <> struct SectionTypes<2> { using K = Coef64; using S = State64; using E = double; };
+
 // ENV: 0 = cascade only, 1 = magnitude, 2 = magnitude + low-pass.
 // OUT: 0 = nothing leaves the kernel (warm-up), 1 = decimated frames only, 2 = full-rate
 //      time-major stores (and decimated frames when asked), 3 = every decimated frame goes
@@ -280,8 +435,8 @@ __device__ __forceinline__ void store_window_entries(const FusedParams& p, OutCt
 // butter(1) low-pass output is b0*(w[t] + w[t-1]) (same transfer function (1+z^-1)/(1-k*z^-1) as
 // the reference's lfilter, EnvelopeExtraction.py:47-48), and that sum is only formed for the
 // samples that are stored -- one FMA per sample instead of an add and an FMA.
-template <int ENV>
-__device__ __forceinline__ float envelope(const FusedParams& p, State& s, float2 y) {
+template <int ENV, class S>
+__device__ __forceinline__ float envelope(const FusedParams& p, S& s, float2 y) {
     float e = fast_sqrt(fmaf(y.x, y.x, y.y * y.y));
     if (ENV == 2) {
         e = fmaf(p.lp_k, s.l, e);
@@ -290,9 +445,9 @@ __device__ __forceinline__ float envelope(const FusedParams& p, State& s, float2
     return e;
 }
 
-template <int FORM, int ENV, int OUT, bool ZEROX, int U, bool CN = false>
-__device__ __forceinline__ void run_tile(const FusedParams& p, const Coef& k, State& s, const float (&ee)[4],
-                                         const float (&eo)[4], const float2* __restrict__ sxz,
+template <int FORM, int ENV, int OUT, bool ZEROX, int U, bool CN = false, class K, class S, class E>
+__device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s, const E (&ee)[4],
+                                         const E (&eo)[4], const float2* __restrict__ sxz,
                                          const float* __restrict__ sg, int t, int cnt, bool active, OutCtx& o) {
     int i = 0;
     for (; i + U <= cnt; i += U) {
@@ -431,26 +586,9 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
     const int mask = N2 - 1;
     const bool big = N2 >= kTile;  // TMA path: tiles never straddle the ring wrap
 
-    Coef k;
-    {
-        const float* cp = p.chan + (active ? c : 0);
-        const float on = active ? 1.f : 0.f;
-        k.g4 = on * cp[P_G4 * p.c_pad];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float z = on * cp[(P_Z + i) * p.c_pad];
-            const float cq = on * (FORM == 1 ? -cp[(P_CQ + i) * p.c_pad] : cp[(P_CQ + i) * p.c_pad]);
-            const float ncy = on * cp[((FORM == 1 ? P_NB1 : P_NCY) + i) * p.c_pad];
-            k.z[i] = make_float2(z, z);
-            k.cq[i] = make_float2(cq, cq);
-            k.ncy[i] = make_float2(ncy, ncy);
-        }
-#pragma unroll
-        for (int i = 0; i < 3; ++i) {
-            const float zn = FORM == 1 ? k.z[i + 1].x + k.ncy[i].x : 0.f;
-            k.zn[i] = make_float2(zn, zn);
-        }
-    }
+    using E = typename SectionTypes<FORM>::E;
+    typename SectionTypes<FORM>::K k;
+    load_coef<FORM>(p, c, active, k);
 
     // ---- tile schedule: E stream [tE0, n) (edge residuals), then M stream [ts, t1) ----
     // truncated-history lengths of THIS channel group (uniform in the CTA): the plan's lengths belong to
@@ -497,15 +635,10 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
         for (int kk = 0; kk < pre; ++kk) issue(kk);
     }
 
-    State s;
+    typename SectionTypes<FORM>::S s;
     reset(s);
-    float ee[4] = {0.f, 0.f, 0.f, 0.f}, eo[4] = {0.f, 0.f, 0.f, 0.f};
-    if (EDGE && need_imag && active) {
-        const float4* e = reinterpret_cast<const float4*>(p.edge + ((size_t)item.utt * p.C + c) * 8);
-        const float4 v0 = __ldg(e), v1 = __ldg(e + 1);
-        ee[0] = v0.x; ee[1] = v0.y; ee[2] = v0.z; ee[3] = v0.w;
-        eo[0] = v1.x; eo[1] = v1.y; eo[2] = v1.z; eo[3] = v1.w;
-    }
+    E ee[4] = {0, 0, 0, 0}, eo[4] = {0, 0, 0, 0};
+    if (EDGE && need_imag && active) load_edge(p, item.utt, c, ee, eo);
     OutCtx o;
     o.C = (size_t)p.C;
     o.step = p.step;
@@ -563,7 +696,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
             const int cnt = min(kTile, n - t);
             for (int i = 0; i < cnt; ++i) cascade_real<FORM>(k, s, sxz[i].x);
             if (kk == nE - 1) {
-                float e0[4], e1[4];
+                E e0[4], e1[4];
                 edge_residuals<FORM>(k, s, e0, e1);
                 // (t - n) odd -> e0 multiplies G[t]; even -> e1
                 const bool n_odd = (n & 1) != 0;
@@ -652,6 +785,43 @@ static void launch_variant(const FusedParams& p, int n_items, cudaStream_t strea
         if (p.edge) fused_kernel<MINB, U, true, false, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
         else fused_kernel<MINB, U, false, false, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
     }
+}
+
+// FORM 2 (float64 sections) in its own kernel: a third branch in fused_kernel would raise the register
+// count of the float32 forms for every bank.
+template <int MINB, int U, bool EDGE, bool WIN, bool CN>
+__global__ void __launch_bounds__(kChanPerBlock, MINB) fused_kernel64(const FusedParams p) {
+    __shared__ __align__(128) float2 s_xz[kStages][kTile];
+    __shared__ __align__(128) float s_g[kStages][kTile];
+    __shared__ __align__(8) uint64_t s_full[kStages];
+    extern __shared__ float s_tr[];
+    if (threadIdx.x == 0) {
+        for (int b = 0; b < kStages; ++b) mbar_init(&s_full[b], 1);
+        mbar_fence_init();
+    }
+    __syncwarp();
+    const Item item = p.items[blockIdx.x];
+    const int c = item.cblock * kChanPerBlock + threadIdx.x;
+    const Smem sm{s_xz, s_g, s_full, s_tr};
+    fused_body<2, U, EDGE, WIN, CN>(p, item, sm, c);
+}
+
+cudaError_t launch_fused64(const FusedParams& p, int n_items, cudaStream_t stream) {
+    if (n_items <= 0) return cudaSuccess;
+    constexpr int MINB = 12, U = 8;
+    const bool edge = p.edge64 != nullptr;
+    if (p.win) {
+        if (edge) fused_kernel64<MINB, U, true, true, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
+        else fused_kernel64<MINB, U, false, true, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
+    } else if (p.gfb_cn || p.env_cn) {
+        const size_t tiles = ((p.gfb_cn ? 1 : 0) + (p.env_cn ? 1 : 0)) * (size_t)(32 * kCnP) * sizeof(float);
+        if (edge) fused_kernel64<MINB, U, true, false, true><<<n_items, kChanPerBlock, tiles, stream>>>(p);
+        else fused_kernel64<MINB, U, false, false, true><<<n_items, kChanPerBlock, tiles, stream>>>(p);
+    } else {
+        if (edge) fused_kernel64<MINB, U, true, false, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
+        else fused_kernel64<MINB, U, false, false, false><<<n_items, kChanPerBlock, 0, stream>>>(p);
+    }
+    return cudaGetLastError();
 }
 
 cudaError_t launch_fused(const FusedParams& p, int n_items, cudaStream_t stream) {

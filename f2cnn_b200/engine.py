@@ -52,10 +52,33 @@ def bank_check(coefs):
     return pred.value, chan.value
 
 
-class Plan:
-    """One gammatone filterbank on one device.  coefs = make_erb_filters output (C,10)."""
+def bank_check_groups(coefs):
+    """Predicted float32 error of every group of 32 channels, in units of the 1e-4 x RMS tolerance (numpy
+    array, host only, f2_bank_check_groups).  Plan(..., float64_sections=True) runs the groups above 1.0
+    in float64."""
+    coefs = np.ascontiguousarray(coefs, dtype=np.float64)
+    if coefs.ndim != 2 or coefs.shape[1] != 10:
+        raise ValueError("coefs must be (n_channels, 10) as returned by make_erb_filters")
+    out = np.zeros(max(1, (coefs.shape[0] + 31) // 32), dtype=np.float64)
+    check(_native.lib().f2_bank_check_groups(coefs.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                                             int(coefs.shape[0]), out.ctypes.data_as(ctypes.POINTER(ctypes.c_double))))
+    return out
 
-    def __init__(self, coefs, device=None):
+
+def float64_sections_default():
+    """The float64_sections setting of Plan(..., float64_sections=None): F2CNN_B200_FLOAT64_SECTIONS=1."""
+    return os.environ.get("F2CNN_B200_FLOAT64_SECTIONS", "0") == "1"
+
+
+class Plan:
+    """One gammatone filterbank on one device.  coefs = make_erb_filters output (C,10).
+
+    float64_sections: the kernels compute in float32, and a bank float32 cannot hold to the 1e-4 x RMS
+    tolerance (bank_check > 1: poles very near z = 1, e.g. LOW_FREQ = 20 Hz) is refused.  With True, the
+    groups of 32 channels that bank_check_groups puts above 1 run their sections in float64 instead and
+    the bank is accepted; the others are unchanged.  None: F2CNN_B200_FLOAT64_SECTIONS=1 (off by default)."""
+
+    def __init__(self, coefs, device=None, float64_sections=None):
         _require_cuda()
         coefs = np.ascontiguousarray(coefs, dtype=np.float64)
         if coefs.ndim != 2 or coefs.shape[1] != 10:
@@ -63,9 +86,16 @@ class Plan:
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
         self.n_channels = int(coefs.shape[0])
         self.coefs = coefs
+        self.float64_sections = float64_sections_default() if float64_sections is None else bool(float64_sections)
         self._h = ctypes.c_void_p()
-        check(_native.lib().f2_plan_create(coefs.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), self.n_channels,
-                                           self.device.index, ctypes.byref(self._h)))
+        flags = _native.F2_PLAN_FLOAT64_SECTIONS if self.float64_sections else 0
+        check(_native.lib().f2_plan_create_ex(coefs.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), self.n_channels,
+                                              self.device.index, flags, ctypes.byref(self._h)))
+        n_groups = (self.n_channels + 31) // 32
+        mask = (ctypes.c_ubyte * n_groups)()
+        if _native.lib().f2_plan_float64_groups(self._h, mask, n_groups) < 0:
+            raise _native.F2Error(_native.F2_ERR_INVALID, _native.lib().f2_last_error().decode())
+        self.float64_groups = tuple(g for g in range(n_groups) if mask[g])
         self._ws = {}
         self._ws_lock = threading.Lock()
         self._frozen = False  # plan_for() hands the same object to every caller: no mutation there
@@ -703,15 +733,17 @@ _plans_lock = threading.Lock()
 
 
 def plan_for(coefs, device=None):
-    """One shared, immutable plan per (coefficient matrix, device)."""
+    """One shared, immutable plan per (coefficient matrix, device, float64 sections setting): the setting is
+    F2CNN_B200_FLOAT64_SECTIONS at the time of the call (Plan)."""
     _require_cuda()
     coefs = np.ascontiguousarray(coefs, dtype=np.float64)
     dev = torch.cuda.current_device() if device is None else int(device)
-    key = (hashlib.sha1(coefs.tobytes()).hexdigest(), coefs.shape, dev)
+    f64 = float64_sections_default()
+    key = (hashlib.sha1(coefs.tobytes()).hexdigest(), coefs.shape, dev, f64)
     with _plans_lock:
         p = _plans.get(key)
         if p is None:
-            p = Plan(coefs, dev)
+            p = Plan(coefs, dev, float64_sections=f64)
             p._frozen = True
             _plans[key] = p
         return p
@@ -724,7 +756,7 @@ def any_plan(device=None):
     """A plan is only a device handle for the filterbank-independent entry points."""
     dev = torch.cuda.current_device() if device is None else int(device)
     with _plans_lock:
-        for (k, shape, d), p in _plans.items():
+        for (k, shape, d, f64), p in _plans.items():
             if d == dev:
                 return p
     from .gammatone import filters

@@ -56,8 +56,21 @@ F2_API int f2_abi_version(void);
  * coefs: HOST pointer to the (n_channels, 10) float64 matrix returned by
  * gammatone.filters.make_erb_filters (gammatone/filters.py:186-190: columns
  * A0, A11, A12, A13, A14, A2, B0, B1, B2, gain).  Derives the float32 per-channel
- * parameter block in float64 and uploads it to `device`. */
+ * parameter block in float64 and uploads it to `device`.  The kernels compute in float32: a bank whose
+ * predicted float32 error (f2_bank_check) exceeds the 1e-4 x RMS tolerance is refused with
+ * F2_ERR_UNSUPPORTED, unless the environment sets F2CNN_B200_ALLOW_IMPRECISE.  Same as
+ * f2_plan_create_ex with flags 0. */
 F2_API int f2_plan_create(const double* coefs, int n_channels, int device, f2_plan** out);
+/* flags of f2_plan_create_ex */
+#define F2_PLAN_FLOAT64_SECTIONS 1u /* in a bank f2_bank_check refuses (> 1), the groups of 32 channels
+                                       predicted above the tolerance in float32 (f2_bank_check_groups > 1)
+                                       run their four sections in float64; the bank is accepted and
+                                       F2CNN_B200_ALLOW_IMPRECISE plays no part.  A bank f2_bank_check
+                                       accepts runs in float32 exactly as without the flag. */
+F2_API int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned flags, f2_plan** out);
+/* Which groups of 32 channels run in float64: mask[g] = 1 or 0 for g < n_groups (mask may be null when
+ * n_groups == 0).  Returns how many groups do, or -1 for a null plan or bad arguments (f2_last_error). */
+F2_API int f2_plan_float64_groups(const f2_plan* plan, unsigned char* mask, int n_groups);
 /* Host-only check f2_plan_create applies (no device needed).  The kernels compute in float32 and are
  * held to 1e-4 x channel RMS against the reference's float64: the real cascade of the channels
  * nearest to z = 1 is run on the host in float32 with the kernel's exact operations and in float64,
@@ -66,6 +79,9 @@ F2_API int f2_plan_create(const double* coefs, int n_channels, int device, f2_pl
  * (make_erb_filters(fs, cf, width) is public API, gammatone/filters.py:89: e.g. LOW_FREQ = 20 Hz with
  * width = 2), unless the environment sets F2CNN_B200_ALLOW_IMPRECISE. */
 F2_API int f2_bank_check(const double* coefs, int n_channels, double* predicted, int* worst_channel);
+/* The same prediction per group of 32 channels (one warp of the fused kernel), host only:
+ * per_group[g] for g < ceil(n_channels / 32), from the group's own channels nearest to z = 1. */
+F2_API int f2_bank_check_groups(const double* coefs, int n_channels, double* per_group);
 F2_API int f2_plan_destroy(f2_plan* plan);
 F2_API int f2_plan_channels(const f2_plan* plan);
 /* Warm-up lengths in samples (rounded up to multiples of 256); <= 0 keeps the default that
