@@ -4,7 +4,6 @@ Each function stages its inputs through pinned host memory, launches the C-ABI s
 the current CUDA stream and returns freshly allocated numpy arrays of the reference's dtype
 and layout.  All arithmetic happens in libf2cnn_b200.so."""
 import hashlib
-import os
 import threading
 from collections import OrderedDict
 
@@ -300,8 +299,6 @@ def _pipeline_for(plan, lengths, dots, step, phase, LPF, CUTOFF, src_offsets=Non
             # `share` processes of this box run a pipeline each: split the host cores between their pools
             # (one core stays free for the CUDA host-callback thread that hands frames to the pool)
             threads = max(1, engine.host_cores() // max(int(share), 1) - (1 if int(share) == 1 else 0))
-            if os.environ.get("F2CNN_B200_PLACER_THREADS"):   # development knob
-                threads = max(1, int(os.environ["F2CNN_B200_PLACER_THREADS"]))
             pipe = engine.WindowPipeline(plan, lengths, dots=dots, step=step, phase=phase, lpf=LPF, cutoff=CUTOFF,
                                          src_offsets=src_offsets, placer=engine.Placer(threads))
             _pipelines[key] = pipe

@@ -650,9 +650,7 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
         };
         std::stable_sort(out.begin(), out.end(), by_length);
         if (whole_utterances) {   // time chunks are cut to equal cost already
-            const char* tail_env = getenv("F2CNN_B200_TAIL_ITEMS");   // development knob
-            const size_t want = tail_env ? (size_t)atoll(tail_env) : (size_t)sm_count * 16 * 2;
-            const size_t tail = std::min(out.size(), want);
+            const size_t tail = std::min(out.size(), (size_t)sm_count * 16 * 2);
             std::stable_sort(out.end() - (long)tail, out.end(), by_cost);
         }
         // One wave or less (a shard of the corpus on one of eight GPUs): the CTAs are handed to the SMs round
@@ -896,7 +894,6 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     // the direct form grows like 1/(1+B1+B2).  The envelope stays at the delta form's error level
     // (<= 1e-5 of the channel RMS) down to 0.035; the filterbank output itself only down to 0.25.
     fp.direct_min_cy = a->gfb ? kDirectMinCyGfb : kDirectMinCyEnv;
-    if (const char* v = getenv("F2_DIRECT_MIN_CY")) fp.direct_min_cy = (float)atof(v);  // development knob
     fp.step = b->step;
     fp.phase = b->phase;
     fp.lpf = a->lpf ? 1 : 0;

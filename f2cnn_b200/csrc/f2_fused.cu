@@ -385,10 +385,7 @@ struct OutCtx {
 
 // (C, n) staging tile: 32 channels x kCnW samples (+1 column of padding).  Longer runs per channel row make
 // the stores friendlier to DRAM pages (every row of a tile lands in a different page of the (C, n) matrix).
-#ifndef F2_CN_W
-#define F2_CN_W 128
-#endif
-constexpr int kCnW = F2_CN_W;
+constexpr int kCnW = 128;
 constexpr int kCnP = kCnW + 1;
 
 // rows of the staged tile -> global: samples [tb, tb + cnt) of every channel of this CTA
@@ -762,13 +759,8 @@ __global__ void __launch_bounds__(kChanPerBlock, MINB) fused_kernel(const FusedP
     const Smem sm{s_xz, s_g, s_full, s_tr};
     // per group of 32 channels (c_pad = C rounded up to 32): min over the group of 1 + B1 + B2
     const float group_cy = p.chan[P_FORM * p.c_pad + c];
-#ifdef F2_SINGLE_FORM
-    (void)group_cy;
-    fused_body<F2_SINGLE_FORM, U, EDGE, WIN, CN>(p, item, sm, c);
-#else
     if (group_cy >= p.direct_min_cy) fused_body<1, U, EDGE, WIN, CN>(p, item, sm, c);
     else fused_body<0, U, EDGE, WIN, CN>(p, item, sm, c);
-#endif
 }
 
 template <int MINB, int U>
@@ -826,22 +818,6 @@ cudaError_t launch_fused64(const FusedParams& p, int n_items, cudaStream_t strea
 
 cudaError_t launch_fused(const FusedParams& p, int n_items, cudaStream_t stream) {
     if (n_items <= 0) return cudaSuccess;
-#ifdef F2_FUSED_TUNING
-    // development build (make EXTRA=-DF2_FUSED_TUNING): F2_FUSED_VARIANT = "<min CTAs per SM><unroll>"
-    static int variant = -1;
-    if (variant < 0) {
-        const char* v = getenv("F2_FUSED_VARIANT");
-        variant = v ? atoi(v) : 0;
-    }
-    if (variant == 168) {
-        launch_variant<16, 8>(p, n_items, stream);
-        return cudaGetLastError();
-    }
-    if (variant == 208) {
-        launch_variant<20, 8>(p, n_items, stream);
-        return cudaGetLastError();
-    }
-#endif
     // 16 one-warp CTAs per SM, 16 samples per loop trip (profiles/r01j_tune_*.log, r01m); the
     // window-store mode is its own instantiation so that the other modes keep their code
     launch_variant<16, 16>(p, n_items, stream);

@@ -179,9 +179,6 @@ __device__ __forceinline__ void smem_fft(float2* s, int pitch, int logL, int bat
 // N2 = 32768 / 65536 / 131072 are transformed by one cluster kernel (ring_cluster_kernel, ring_cluster8_kernel below)
 __host__ __device__ inline bool ring_cluster_size(int log2N2) { return log2N2 >= 15 && log2N2 <= 17; }
 
-// legs of 128 / 256 points have a register-pass implementation (see the fast kernels below)
-__host__ __device__ inline bool fast_leg(int l) { return l == 7 || l == 8; }
-
 __device__ __forceinline__ int bitrev(int v, int bits) { return bits ? (int)(__brev((unsigned)v) >> (32 - bits)) : 0; }
 
 __host__ __device__ inline void fft_split(int log2M, int& l1, int& l2) {
@@ -205,7 +202,7 @@ __global__ void __launch_bounds__(kFftThreads) fft_cols_kernel(PrepParams p, flo
     if (log2M <= kTwLog) return;  // single-pass sizes skip the column pass
     int l1, l2;
     fft_split(log2M, l1, l2);
-    if (fast_leg(l1) && fast_leg(l2)) return;  // taken by fft_cols_fast_kernel
+    if (p.cluster && ring_cluster_size(ut.log2N2)) return;  // taken by ring_cluster_kernel
     const int M1 = 1 << l1, M2 = 1 << l2;
     int B = kFftSmemPts >> l1;
     if (B > M2) B = M2;
@@ -246,7 +243,7 @@ __global__ void __launch_bounds__(kFftThreads) fft_rows_kernel(PrepParams p, con
     fft_split(log2M, l1, l2);
     if (SRC_WAVE && l1 != 0) return;   // two-pass sizes were packed by the column pass
     if (!SRC_WAVE && !INV && l1 == 0) return;  // forward single-pass sizes take the SRC_WAVE launch
-    if (l1 != 0 && fast_leg(l1) && fast_leg(l2)) return;  // taken by fft_rows_fast_kernel
+    if (p.cluster && ring_cluster_size(ut.log2N2)) return;  // taken by ring_cluster_kernel
     const int M1 = 1 << l1, M2 = 1 << l2;
     int B = kFftSmemPts >> l2;
     if (B > M1) B = M1;
@@ -282,7 +279,7 @@ __global__ void __launch_bounds__(kFftThreads) fft_rows_kernel(PrepParams p, con
 }
 
 // =============================================================================================
-// Fast legs for the sizes real utterances use (legs of 128 and 256 points: N2 = 32768 ... 131072).
+// Register transforms for the legs of the cluster kernel below (128 and 256 points: N2 = 32768 ... 131072).
 // Each leg is two register passes -- L = R1 x R2 with R1 = 16, R2 = L/16 -- around ONE
 // shared-memory exchange, instead of log4(L) shared-memory passes:
 //   pass 1: thread (fft b, n2) loads x[n1*R2 + n2], n1 < 16, runs a 16-point FFT in registers,
@@ -372,135 +369,6 @@ __device__ __forceinline__ float2 leg_twiddle(int m, int logL) {  // w_L^m for 0
     }
     if (INV) w.y = -w.y;
     return w;
-}
-
-constexpr int kFastPts = 4096;  // complex points per CTA in the fast kernels
-
-// Shared layout A[b][k1][n2]: b * PB + k1 * (R2 + 1) + n2, PB odd.
-template <int LOGL>
-struct LegShape {
-    static constexpr int L = 1 << LOGL;
-    static constexpr int R2 = L / 16;
-    static constexpr int B = kFastPts / L;
-    static constexpr int P1 = R2 + 1;
-    static constexpr int PB = 16 * P1 + (((16 * P1) & 1) ? 0 : 1);
-};
-
-// Both passes of one leg for the B transforms of a CTA.  LOAD(b, n) -> float2 input element n
-// of transform b; STORE(b, k, value) consumes output frequency k.  256 threads.
-template <bool INV, int LOGL, typename LoadF, typename StoreF>
-__device__ __forceinline__ void leg_fft(float2* sA, bool b_fastest, LoadF load, StoreF store) {
-    using S = LegShape<LOGL>;
-    const int tid = threadIdx.x;
-    {   // pass 1: S::B * S::R2 == 256 threads
-        const int b = b_fastest ? tid % S::B : tid / S::R2;
-        const int n2 = b_fastest ? tid / S::B : tid % S::R2;
-        float2 v[16];
-#pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) v[n1] = load(b, n1 * S::R2 + n2);
-        fft16<INV>(v);
-#pragma unroll
-        for (int r = 0; r < 16; ++r) {
-            const int k1 = out16(r);
-            sA[b * S::PB + k1 * S::P1 + n2] = cmul(v[r], leg_twiddle<INV>(n2 * k1, LOGL));
-        }
-    }
-    __syncthreads();
-    // pass 2: S::B * 16 threads of work (256 for L = 256, 512 for L = 128)
-#pragma unroll 1
-    for (int t2 = tid; t2 < S::B * 16; t2 += kFftThreads) {
-        const int b = t2 % S::B, k1 = t2 / S::B;
-        const float2* a = sA + b * S::PB + k1 * S::P1;
-        if (S::R2 == 16) {
-            float2 v[16];
-#pragma unroll
-            for (int n2 = 0; n2 < 16; ++n2) v[n2] = a[n2];
-            fft16<INV>(v);
-#pragma unroll
-            for (int r = 0; r < 16; ++r) store(b, k1 + 16 * out16(r), v[r]);
-        } else {
-            float2 v[8];
-#pragma unroll
-            for (int n2 = 0; n2 < 8; ++n2) v[n2] = a[n2];
-            fft8<INV>(v);
-#pragma unroll
-            for (int r = 0; r < 8; ++r) store(b, k1 + 16 * out8(r), v[r]);
-        }
-    }
-}
-
-template <bool INV, bool SRC_WAVE, int LOGL>
-__device__ __forceinline__ void cols_fast_body(const PrepParams& p, const UttDesc& ut, float* buf, float2* sA, int l2) {
-    using S = LegShape<LOGL>;
-    const int M2 = 1 << l2;
-    const int c0 = blockIdx.y * S::B;
-    if (c0 >= M2) return;
-    float2* z = reinterpret_cast<float2*>(buf + ut.ring_off);
-    const float sgn = INV ? 2.0f : -2.0f;
-    const float invM = 1.0f / (float)(1 << (LOGL + l2));
-    leg_fft<INV, LOGL>(
-        sA, true,
-        [&](int b, int n) {
-            const int e = n * M2 + c0 + b;
-            return SRC_WAVE ? load_pair(p.wave, p.wave_dtype, ut.wave_off, e, ut.n) : z[e];
-        },
-        [&](int b, int k, float2 v) {
-            const int n2 = c0 + b;
-            float sn, cs;
-            sincospif(sgn * (float)(n2 * k) * invM, &sn, &cs);
-            z[(size_t)k * M2 + n2] = cmul(v, make_float2(cs, sn));
-        });
-}
-
-// The pass that reads the int16 wave is latency-bound at 3 CTAs per SM (74 registers): capped at 64
-// registers it runs 4 CTAs per SM and 15 % faster; the other passes lose from the same cap.
-template <bool INV, bool SRC_WAVE>
-__global__ void __launch_bounds__(kFftThreads, SRC_WAVE ? 4 : 3) fft_cols_fast_kernel(PrepParams p, float* buf) {
-    __shared__ float2 sA[kFastPts + kFastPts / 8 + 64];
-    const UttDesc ut = p.utts[blockIdx.x];
-    const int log2M = ut.log2N2 - 1;
-    int l1, l2;
-    fft_split(log2M, l1, l2);
-    if (log2M <= kTwLog || !fast_leg(l1) || !fast_leg(l2)) return;
-    if (p.cluster && ring_cluster_size(ut.log2N2)) return;  // taken by ring_cluster_kernel
-    if (l1 == 7) cols_fast_body<INV, SRC_WAVE, 7>(p, ut, buf, sA, l2);
-    else cols_fast_body<INV, SRC_WAVE, 8>(p, ut, buf, sA, l2);
-}
-
-template <bool INV, bool DST_RING, int LOGL>
-__device__ __forceinline__ void rows_fast_body(const PrepParams& p, const UttDesc& ut, const float* in_buf,
-                                               float* out_buf, float2* sA, int l1) {
-    using S = LegShape<LOGL>;
-    const int M1 = 1 << l1;
-    const int r0 = blockIdx.y * S::B;
-    if (r0 >= M1) return;
-    const float2* zin = reinterpret_cast<const float2*>(in_buf + ut.ring_off);
-    float2* zout = DST_RING ? nullptr : reinterpret_cast<float2*>(out_buf + ut.ring_off);
-    float4* ring = DST_RING ? reinterpret_cast<float4*>(p.xz + ut.ring_off) : nullptr;
-    leg_fft<INV, LOGL>(
-        sA, false, [&](int b, int n) { return zin[(size_t)(r0 + b) * S::L + n]; },
-        [&](int b, int k, float2 v) {
-            const int m = k * M1 + r0 + b;
-            if (DST_RING) {
-                const float2 x = load_pair(p.wave, p.wave_dtype, ut.wave_off, m, ut.n);
-                ring[m] = make_float4(x.x, v.x, x.y, v.y);
-            } else {
-                zout[m] = v;
-            }
-        });
-}
-
-template <bool INV, bool DST_RING>
-__global__ void __launch_bounds__(kFftThreads) fft_rows_fast_kernel(PrepParams p, const float* in_buf, float* out_buf) {
-    __shared__ float2 sA[kFastPts + kFastPts / 8 + 64];
-    const UttDesc ut = p.utts[blockIdx.x];
-    const int log2M = ut.log2N2 - 1;
-    int l1, l2;
-    fft_split(log2M, l1, l2);
-    if (log2M <= kTwLog || !fast_leg(l1) || !fast_leg(l2)) return;
-    if (p.cluster && ring_cluster_size(ut.log2N2)) return;  // taken by ring_cluster_kernel
-    if (l2 == 7) rows_fast_body<INV, DST_RING, 7>(p, ut, in_buf, out_buf, sA, l1);
-    else rows_fast_body<INV, DST_RING, 8>(p, ut, in_buf, out_buf, sA, l1);
 }
 
 // One pair (Z[k], Z[M-k]) of the packed spectrum -> the pair (W[k], W[M-k]) the inverse packed transform
@@ -911,17 +779,12 @@ __device__ __forceinline__ void ring_cluster_body(const PrepParams& p, const Utt
     }
 }
 
-#ifndef F2_RING_CL
-#define F2_RING_CL 4
-#endif
-#ifndef F2_RING_CTAS
-#define F2_RING_CTAS 2
-#endif
-constexpr int kRingCl = F2_RING_CL;   // CTAs per cluster
+constexpr int kRingCl = 4;            // CTAs per cluster
+constexpr int kRingCtas = 2;          // CTAs per SM
 constexpr int kRingClThreads = 512;
-constexpr int kRingAhead = 148 * F2_RING_CTAS / F2_RING_CL;   // clusters resident at a time
+constexpr int kRingAhead = 148 * kRingCtas / kRingCl;   // clusters resident at a time
 constexpr int kRingCl8 = 8;           // CTAs per cluster for rings of 131072 samples (M = 256 x 256)
-constexpr int kRingAhead8 = 148 * F2_RING_CTAS / kRingCl8;
+constexpr int kRingAhead8 = 148 * kRingCtas / kRingCl8;
 constexpr int kRingClElems = RingCl<7, 8, kRingCl, kRingClThreads>::kElems > RingCl<7, 7, kRingCl, kRingClThreads>::kElems
                                  ? RingCl<7, 8, kRingCl, kRingClThreads>::kElems
                                  : RingCl<7, 7, kRingCl, kRingClThreads>::kElems;
@@ -943,7 +806,7 @@ __device__ __forceinline__ void prefetch_next_wave(const PrepParams& p, int u, i
         asm volatile("prefetch.global.L2 [%0];" ::"l"(base + o));
 }
 
-__global__ void __cluster_dims__(kRingCl, 1, 1) __launch_bounds__(kRingClThreads, F2_RING_CTAS) ring_cluster_kernel(PrepParams p) {
+__global__ void __cluster_dims__(kRingCl, 1, 1) __launch_bounds__(kRingClThreads, kRingCtas) ring_cluster_kernel(PrepParams p) {
     extern __shared__ float2 s_fft[];
     const int u = blockIdx.x / kRingCl, n_utts = gridDim.x / kRingCl;
     const UttDesc ut = p.utts[u];
@@ -953,7 +816,7 @@ __global__ void __cluster_dims__(kRingCl, 1, 1) __launch_bounds__(kRingClThreads
 }
 
 // rings of 131072 samples (utterances of 4.1 ... 8.2 s): M = 256 x 256 packed points, a cluster of 8 CTAs
-__global__ void __cluster_dims__(kRingCl8, 1, 1) __launch_bounds__(kRingClThreads, F2_RING_CTAS) ring_cluster8_kernel(PrepParams p) {
+__global__ void __cluster_dims__(kRingCl8, 1, 1) __launch_bounds__(kRingClThreads, kRingCtas) ring_cluster8_kernel(PrepParams p) {
     extern __shared__ float2 s_fft[];
     const int u = blockIdx.x / kRingCl8, n_utts = gridDim.x / kRingCl8;
     const UttDesc ut = p.utts[u];
@@ -1035,7 +898,6 @@ cudaError_t launch_prep(const PrepParams& p_in, const HostPrepInfo& h, cudaStrea
         cudaFuncSetAttribute(fft_rows_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         cudaFuncSetAttribute(fft_rows_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         cudaFuncSetAttribute(fft_rows_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        cudaFuncSetAttribute(fft_cols_fast_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         cudaFuncSetAttribute(ring_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRingClSmem);
         cudaFuncSetAttribute(ring_cluster8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRingCl8Smem);
         if (dev < 64) attr_done[dev] = true;
@@ -1049,24 +911,10 @@ cudaError_t launch_prep(const PrepParams& p_in, const HostPrepInfo& h, cudaStrea
         if (p.G) hilbert_mask_kernel<<<g_ew, 256, 0, stream>>>(p.utts, nullptr, p.G, 0);  // N2 <= 2: G = 0
         return cudaGetLastError();
     }
-    const bool two = (h.max_log2N2 - 1) > kTwLog;
     const bool one = h.min_log2N2 - 1 <= kTwLog;  // some utterances take the single-pass path
-    // sizes with 128/256-point legs (N2 = 2^15 .. 2^17) take the register-pass kernels
-    bool fast = false, slow2 = false;
-    int fast_blocks = 1;
-    for (int lg = h.min_log2N2; lg <= h.max_log2N2; ++lg) {
-        if (lg - 1 <= kTwLog) continue;
-        if (p.cluster && ring_cluster_size(lg)) continue;
-        int l1, l2;
-        fft_split(lg - 1, l1, l2);
-        if (fast_leg(l1) && fast_leg(l2)) {
-            fast = true;
-            fast_blocks = std::max(fast_blocks, std::max((1 << l2) / (kFastPts >> l1), (1 << l1) / (kFastPts >> l2)));
-        } else {
-            slow2 = true;
-        }
-    }
-    const dim3 g_fast(h.n_utts, fast_blocks);
+    bool two = false;                              // some take the two-pass path: not a cluster kernel's size
+    for (int lg = h.min_log2N2; lg <= h.max_log2N2; ++lg)
+        if (lg - 1 > kTwLog && !(p.cluster && ring_cluster_size(lg))) two = true;
     const dim3 g_cols(h.n_utts, max_blocks(h, true));
     const dim3 g_rows(h.n_utts, max_blocks(h, false));
     float* A = p.bufA;
@@ -1076,19 +924,15 @@ cudaError_t launch_prep(const PrepParams& p_in, const HostPrepInfo& h, cudaStrea
     if (p.cluster && h.min_log2N2 <= 16) ring_cluster_kernel<<<kRingCl * h.n_utts, kRingClThreads, kRingClSmem, stream>>>(p);
     if (p.cluster && h.max_log2N2 >= 17) ring_cluster8_kernel<<<kRingCl8 * h.n_utts, kRingClThreads, kRingCl8Smem, stream>>>(p);
     // forward
-    if (fast) fft_cols_fast_kernel<false, true><<<g_fast, kFftThreads, 0, stream>>>(p, A);
-    if (fast) fft_rows_fast_kernel<false, false><<<g_fast, kFftThreads, 0, stream>>>(p, A, B);
-    if (two && slow2) fft_cols_kernel<false, true><<<g_cols, kFftThreads, smem, stream>>>(p, A);
-    if (two && slow2) fft_rows_kernel<false, false, false><<<g_rows, kFftThreads, smem, stream>>>(p, A, B);
+    if (two) fft_cols_kernel<false, true><<<g_cols, kFftThreads, smem, stream>>>(p, A);
+    if (two) fft_rows_kernel<false, false, false><<<g_rows, kFftThreads, smem, stream>>>(p, A, B);
     if (one) fft_rows_kernel<false, true, false><<<g_rows, kFftThreads, smem, stream>>>(p, nullptr, B);
     // Hilbert multiplier in place on B; the injection kernel goes to A (free from here on)
     const bool all_cluster = p.cluster && h.min_log2N2 >= 15 && h.max_log2N2 <= 17;
     if (!all_cluster || (p.G && h.private_g > 0)) hilbert_mask_kernel<<<g_ew, 256, 0, stream>>>(p.utts, B, p.G, p.cluster);
     // inverse, last pass writes the (x, xi) ring
-    if (fast) fft_cols_fast_kernel<true, false><<<g_fast, kFftThreads, 0, stream>>>(p, B);
-    if (fast) fft_rows_fast_kernel<true, true><<<g_fast, kFftThreads, 0, stream>>>(p, B, nullptr);
-    if (two && slow2) fft_cols_kernel<true, false><<<g_cols, kFftThreads, smem, stream>>>(p, B);
-    if (one || slow2) fft_rows_kernel<true, false, true><<<g_rows, kFftThreads, smem, stream>>>(p, B, nullptr);
+    if (two) fft_cols_kernel<true, false><<<g_cols, kFftThreads, smem, stream>>>(p, B);
+    if (one || two) fft_rows_kernel<true, false, true><<<g_rows, kFftThreads, smem, stream>>>(p, B, nullptr);
     if (h.min_log2N2 < 2) plain_ring_kernel<<<g_ew, 256, 0, stream>>>(p, 1);
     return cudaGetLastError();
 }

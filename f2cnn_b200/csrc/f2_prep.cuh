@@ -19,7 +19,7 @@ struct PrepParams {
     float* G;          // out: injection kernel rings; must alias bufA (free once the forward
                        // transform is done) or be null (plain Hilbert, no table)
     int hilbert;       // 0: filterbank-only run, skip the FFTs and leave xi = 0
-    int cluster;       // set by launch_prep: N2 = 32768 / 65536 go through ring_cluster_kernel
+    int cluster;       // set by launch_prep: N2 = 32768 ... 131072 go through the cluster kernels
 };
 
 struct HostPrepInfo {

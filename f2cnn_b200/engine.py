@@ -436,8 +436,8 @@ class WindowPipeline:
     kernel stores its decimated frames STRAIGHT INTO THE PINNED HOST BUFFER (posted PCIe writes
     spread over the kernel's run time: 16 GB/s on average; a device buffer plus one D2H copy per
     sub-batch arrives in bursts that fight the placement threads for the host's DRAM and was 3 ms
-    slower per corpus -- `zero_copy = False` / F2CNN_B200_ZERO_COPY_FRAMES=0 brings it back).  The
-    end of each sub-batch's kernels is followed, in stream order, by the host placement of its rows
+    slower per corpus).  The end of each sub-batch's kernels is followed, in stream order, by the
+    host placement of its rows
     (cudaLaunchHostFunc -> thread pool), so the host never waits between sub-batches.  Consecutive sub-batches run on two alternating compute
     streams (each with its own ring workspace), so the tail of one launch overlaps the head of the
     next.
@@ -466,20 +466,12 @@ class WindowPipeline:
         # sub-batches of total/n_sub samples, except that the first few grow from an eighth of that (nothing
         # can be placed before the first sub-batch is uploaded, filtered and downloaded) and the last few
         # shrink to a quarter (the rows of the last sub-batch are placed after the GPU has gone idle)
-        if n_sub is None and os.environ.get("F2CNN_B200_NSUB"):
-            n_sub = int(os.environ["F2CNN_B200_NSUB"])   # development knob
         if n_sub is None:
             # a sub-batch should still fill the device: 592 utterances x 4 channel groups = one wave of CTAs
             n_sub = min(U // 576, 8)
         n_sub = max(1, min(int(n_sub), 32, max(U, 1)))
         per_sub = cum[-1] / n_sub
         head, size, at = [], per_sub / 8, 0.0
-        ramp = os.environ.get("F2CNN_B200_RAMP")   # development knob: head sub-batches as fractions 1/d of the corpus
-        if ramp:
-            for d in ramp.split(","):
-                at += cum[-1] / float(d)
-                head.append(at)
-            size = per_sub
         while size < per_sub and at + size < cum[-1] / 2:
             at += size
             head.append(at)
@@ -515,7 +507,6 @@ class WindowPipeline:
         self._wave_dev = None
         self._stage = None      # pinned staging for pageable input
         with torch.cuda.device(dev):
-            self._dec_dev = None    # only the copy mode (zero_copy = False) needs a device-side frames buffer
             self._dec_host = _pinned_empty(max(self.total_frames, 1) * C, torch.float32).view(-1, C)
             self._s_in, self._s_out = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
             # consecutive sub-batches alternate between two compute streams: a launch ends with a tail
@@ -523,12 +514,8 @@ class WindowPipeline:
             self._s_comp = [torch.cuda.Stream(dev), torch.cuda.Stream(dev)]
             self._ev_in = [torch.cuda.Event(enable_timing=True) for _ in self.subs]
             self._ev_done = [torch.cuda.Event(enable_timing=True) for _ in self.subs]
-            self._ev_out = [torch.cuda.Event(enable_timing=True) for _ in self.subs]
             self._ev_start = torch.cuda.Event(enable_timing=True)
             self._ev_end = torch.cuda.Event(blocking=True)
-        # True: the fused kernel stores the decimated frames straight into the pinned host buffer (posted PCIe
-        # writes spread over the kernel's run time) instead of a device buffer + one D2H copy per sub-batch
-        self.zero_copy = os.environ.get("F2CNN_B200_ZERO_COPY_FRAMES", "1") == "1"
         self.timing = False     # True: run() synchronises first and keeps a timeline (see timeline())
         self._t0 = None
         self.placer = placer if placer is not None else Placer()
@@ -576,8 +563,7 @@ class WindowPipeline:
     def _run(self, wave_host, runs, out_host, keep_frames, gc_was_on):
         caller = torch.cuda.current_stream(self.plan.device)
         dev = self.plan.device
-        C = self.plan.n_channels
-        listed = isinstance(wave_host, (list, tuple))
+        listed =isinstance(wave_host, (list, tuple))
         if listed:
             dt = torch.from_numpy(wave_host[0][:0]).dtype if len(wave_host) else torch.int16
             pinned = False
@@ -626,9 +612,7 @@ class WindowPipeline:
                     self._ev_in[i].record(self._s_in)
             comp = self._s_comp[i & 1]
             comp.wait_event(self._ev_in[i])
-            if not self.zero_copy and self._dec_dev is None:
-                self._dec_dev = torch.empty((max(self.total_frames, 1), C), dtype=torch.float32, device=dev)
-            dec = (self._dec_host if self.zero_copy else self._dec_dev)[sub["f0"]:sub["f1"]]
+            dec = self._dec_host[sub["f0"]:sub["f1"]]
             sub["batch"].run(self._wave_dev[sub["s0"]:sub["s1"]], lpf=self.lpf, cutoff=self.cutoff, out={"dec": dec},
                              stream=comp)
             self._ev_done[i].record(comp)
@@ -641,9 +625,6 @@ class WindowPipeline:
         with torch.cuda.stream(self._s_out):
             for i, sub in enumerate(self.subs):
                 self._s_out.wait_event(self._ev_done[i])
-                if sub["f1"] > sub["f0"] and not self.zero_copy:
-                    self._dec_host[sub["f0"]:sub["f1"]].copy_(self._dec_dev[sub["f0"]:sub["f1"]], non_blocking=True)
-                self._ev_out[i].record(self._s_out)
                 if per_sub[i].shape[0]:
                     self.placer.submit(self._dec_host, per_sub[i], out_flat, dots=self.dots, stream=self._s_out)
             self._ev_end.record(self._s_out)
@@ -659,15 +640,15 @@ class WindowPipeline:
 
     def timeline(self):
         """After a run() with timing = True: per sub-batch, milliseconds since the start of the run at
-        which its waves were on the device, its kernels had finished, its frames were on the host (CUDA
-        events), and at which its rows became runnable / were placed (host clock of the worker pool)."""
+        which its waves were on the device and its kernels had finished, which is also when its frames
+        were on the host (CUDA events), and at which its rows became runnable / were placed (host clock
+        of the worker pool)."""
         torch.cuda.synchronize(self.plan.device)
         trace = self.placer.trace(clear=True)
         rows = []
         for i, sub in enumerate(self.subs):
             rows.append(dict(utterances=sub["u1"] - sub["u0"], h2d=self._ev_start.elapsed_time(self._ev_in[i]),
-                             kernels=self._ev_start.elapsed_time(self._ev_done[i]),
-                             d2h=self._ev_start.elapsed_time(self._ev_out[i])))
+                             kernels=self._ev_start.elapsed_time(self._ev_done[i])))
         jobs = [dict(runnable=(t[1] - self._t0) * 1e3, placed=(t[2] - self._t0) * 1e3, rows=int(t[3])) for t in trace]
         return rows, jobs
 

@@ -708,9 +708,10 @@ def test_frame_windows_are_views_of_the_decimated_frames(gpu, monkeypatch):
 
 
 def test_multi_pass_prepass_agrees_with_the_cluster_kernels(gpu):
-    """F2CNN_B200_RING_CLUSTER=0 sends rings of 32768 / 65536 / 131072 samples through the five-kernel
-    pre-pass the cluster kernels replaced (kept as their cross-check): a child process computes the same
-    decimated envelopes that way; the two agree far inside the tolerance (different FFT factorisations)."""
+    """F2CNN_B200_RING_CLUSTER=0 sends rings of 32768 / 65536 / 131072 samples through the generic
+    multi-pass kernels (fft_cols / fft_rows / hilbert_mask, which serve every other ring size and are kept
+    as the cluster kernels' cross-check): a child process computes the same decimated envelopes that way;
+    the two agree far inside the tolerance (different FFT factorisations)."""
     import os
     import subprocess
     import sys

@@ -27,6 +27,6 @@ for i in range(14):
     pipe.run(wave_host, runs, out)
     total = (time.perf_counter() - t) * 1e3
     subs, jobs = pipe.timeline()
-    print("run %2d total %.2f ms | kernels end %.2f | frames %.2f | first runnable %.2f last placed %.2f | per-sub place ms %s | gc %s" % (
-        i, total, max(s["kernels"] for s in subs), max(s["d2h"] for s in subs), jobs[0]["runnable"], max(j["placed"] for j in jobs),
+    print("run %2d total %.2f ms | kernels end %.2f | first runnable %.2f last placed %.2f | per-sub place ms %s | gc %s" % (
+        i, total, max(s["kernels"] for s in subs), jobs[0]["runnable"], max(j["placed"] for j in jobs),
         " ".join("%.1f" % (j["placed"] - j["runnable"]) for j in jobs), g0), flush=True)

@@ -1,5 +1,5 @@
 """The public call on the bench corpus, N times: per-call wall times (ms), median and min.
-usage: tools/e2e_repeat.py [calls]   (F2CNN_B200_ZERO_COPY_FRAMES=0/1 selects how the frames travel)"""
+usage: tools/e2e_repeat.py [calls]"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -20,6 +20,6 @@ for i in range(calls + 2):
     api.features_to_windows((wave, lengths), co, centers, True, 50, 5, 160, out=out, counts=nwin)
     ms.append((time.perf_counter() - t) * 1e3)
 warm = np.array(ms[2:])
-print("zero_copy=%s first %.1f ms; warm calls: %s -> median %.2f min %.2f ms; checksum %.6e" % (
-    os.environ.get("F2CNN_B200_ZERO_COPY_FRAMES", "1"), ms[0], " ".join("%.1f" % m for m in warm), np.median(warm), warm.min(),
+print("first %.1f ms; warm calls: %s -> median %.2f min %.2f ms; checksum %.6e" % (
+    ms[0], " ".join("%.1f" % m for m in warm), np.median(warm), warm.min(),
     float(out[::997].astype(np.float64).sum())))

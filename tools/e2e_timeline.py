@@ -1,5 +1,5 @@
-"""Timeline of one corpus-sized pipeline run: when each sub-batch's waves, kernels, frames and rows
-were done (ms since the start of the call)."""
+"""Timeline of one corpus-sized pipeline run: when each sub-batch's waves, kernels (and with them its
+frames, which the fused kernel stores into host memory) and rows were done (ms since the start of the call)."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -26,8 +26,8 @@ pipe.run(wave_host, runs, out)
 total = (time.perf_counter() - t) * 1e3
 subs, jobs = pipe.timeline()
 print("placement threads %d, total %.2f ms (includes the leading synchronize)" % (pipe.placer.threads, total))
-print("sub  utts   waves-on-device  kernels-done  frames-on-host | rows runnable   placed   (rows)")
+print("sub  utts   waves-on-device  kernels-done | rows runnable   placed   (rows)")
 for i, s in enumerate(subs):
     j = jobs[i] if i < len(jobs) else dict(runnable=float("nan"), placed=float("nan"), rows=0)
-    print("%3d %5d %12.2f %14.2f %14.2f | %12.2f %10.2f %9d" % (i, s["utterances"], s["h2d"], s["kernels"], s["d2h"],
-                                                              j["runnable"], j["placed"], j["rows"]))
+    print("%3d %5d %12.2f %14.2f | %12.2f %10.2f %9d" % (i, s["utterances"], s["h2d"], s["kernels"],
+                                                       j["runnable"], j["placed"], j["rows"]))

@@ -1,6 +1,6 @@
 """The one-kernel ring transform (ring_cluster_kernel) against scipy.signal.hilbert on rows that pad to
-N2 = 32768 and 65536, and the pre-pass time of a corpus slice with and without it
-(F2CNN_B200_RING_CLUSTER=0 in a child process)."""
+N2 = 32768 and 65536, and the per-utterance frame checksums of a corpus slice with and without it
+(F2CNN_B200_RING_CLUSTER=0 in a child process: the multi-pass kernels)."""
 import os, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -18,7 +18,7 @@ def errors():
         print("n=%6d N2=%6d  max |xi - scipy| / rms = %.2e" % (n, N2, np.max(np.abs(got - want)) / np.sqrt(np.mean(want ** 2))), flush=True)
 
 
-def timing():
+def checksums():
     from f2cnn_b200 import engine, synth
     from f2cnn_b200.gammatone import filters
     coefs = filters.make_erb_filters(16000, filters.centre_freqs(16000, 128, 100))
@@ -29,28 +29,22 @@ def timing():
     plan = engine.plan_for(coefs)
     batch = plan.batch(lengths, step=160, phase=0)
     out = {"dec": torch.empty((batch.total_frames, 128), dtype=torch.float32, device="cuda")}
-    ev = (engine.DeviceEvent(), engine.DeviceEvent())
-    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _ in range(4):
-        t0.record()
-        batch.run(flat, lpf=True, cutoff=50, dec=True, out=out, fused_events=ev)
-        t1.record()
-        torch.cuda.synchronize()
-    total, fused = t0.elapsed_time(t1), ev[0].elapsed_ms(ev[1])
+    batch.run(flat, lpf=True, cutoff=50, dec=True, out=out)
+    torch.cuda.synchronize()
     sums = torch.stack([out["dec"][int(a):int(b)].double().sum() for a, b in zip(batch.frame_offsets[:-1], batch.frame_offsets[1:])]).cpu().numpy()
     np.save("gpurun_out/ring_sums_%s.npy" % os.environ.get("F2CNN_B200_RING_CLUSTER", "1"), sums)
     np.save("gpurun_out/ring_lengths.npy", lengths)
-    print("cluster=%s  step %.3f ms = pre-pass %.3f + fused %.3f   checksum %.9e" % (
-        os.environ.get("F2CNN_B200_RING_CLUSTER", "1"), total, total - fused, fused, float(out["dec"].double().sum())), flush=True)
+    print("cluster=%s  checksum %.9e" % (os.environ.get("F2CNN_B200_RING_CLUSTER", "1"), float(out["dec"].double().sum())),
+          flush=True)
 
 
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "timing":
-        timing()
+    if len(sys.argv) > 1 and sys.argv[1] == "checksums":
+        checksums()
     else:
         errors()
         for v in ("1", "0"):
-            subprocess.run([sys.executable, __file__, "timing"], env=dict(os.environ, F2CNN_B200_RING_CLUSTER=v))
+            subprocess.run([sys.executable, __file__, "checksums"], env=dict(os.environ, F2CNN_B200_RING_CLUSTER=v))
         a, b = np.load("gpurun_out/ring_sums_1.npy"), np.load("gpurun_out/ring_sums_0.npy")
         lengths = np.load("gpurun_out/ring_lengths.npy")
         rel = np.abs(a - b) / np.abs(b)
