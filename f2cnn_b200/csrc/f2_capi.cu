@@ -975,8 +975,8 @@ int f2_envelope_rows(f2_plan* plan, const void* matrix, int dtype, int64_t rows,
 
 int f2_rows_op(f2_plan* plan, const void* matrix, int dtype, int64_t rows, int64_t n, int op, int lpf,
                double cutoff_hz, void* out, int out_dtype, void* workspace, size_t workspace_bytes, void* stream_) {
-    if (!plan || rows < 0 || n < 0 || op < F2_ROWS_ENVELOPE || op > F2_ROWS_LOWPASS)
-        return fail(F2_ERR_INVALID, "f2_rows_op: bad arguments");
+    if (!plan || rows < 0 || n < 0 || op < F2_ROWS_ENVELOPE || op > F2_ROWS_LOWPASS || (op == F2_ROWS_LOWPASS && !lpf))
+        return fail(F2_ERR_INVALID, "f2_rows_op: bad arguments (F2_ROWS_LOWPASS needs lpf = 1)");
     if (rows == 0 || n == 0) return F2_OK;
     if (!matrix || !out || dtype < F2_I16 || dtype > F2_F64 || (out_dtype != F2_F32 && out_dtype != F2_F64))
         return fail(F2_ERR_INVALID, "f2_envelope_rows: pointer/dtype");

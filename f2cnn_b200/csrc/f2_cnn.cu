@@ -204,11 +204,24 @@ cnn_front_kernel(const float* __restrict__ env_t, int step, long long frame0, in
                 hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
             }
             if (!(lo > 0.f) && tid == 0) atomicOr(bad_flag, 1);   // the reference raises ValueError
-            const float llo = logf(lo), inv = hi > lo ? 1.0f / (logf(hi) - llo) : 0.f;
+            // Within a factor 2 of lo, v - lo and hi - lo are exact and log1pf keeps the digits that
+            // logf(v) - logf(lo) would cancel (a frame spanning a few ulps gave NaN or several times its span);
+            // beyond it (hi - lo) / lo may overflow and the log difference has no cancellation to speak of.
+            const bool close = hi <= 2.f * lo;
+            const float llo = logf(lo);
+            const float inv = hi > lo ? 1.0f / (close ? log1pf((hi - lo) / lo) : logf(hi) - llo) : 0.f;
+            if (close) {   // the same lo and hi in every worker thread: a uniform branch
 #pragma unroll
-            for (int j = 0; j < 3; ++j) {
-                const int k = k0 + 4 * j;
-                if (k < kDots) g0[(k + 1) * kW0 + c + 1] = __float2bfloat16(hi > lo ? (logf(v[j]) - llo) * inv : 0.f);
+                for (int j = 0; j < 3; ++j) {
+                    const int k = k0 + 4 * j;
+                    if (k < kDots) g0[(k + 1) * kW0 + c + 1] = __float2bfloat16(log1pf((v[j] - lo) / lo) * inv);
+                }
+            } else {
+#pragma unroll
+                for (int j = 0; j < 3; ++j) {
+                    const int k = k0 + 4 * j;
+                    if (k < kDots) g0[(k + 1) * kW0 + c + 1] = __float2bfloat16((logf(v[j]) - llo) * inv);
+                }
             }
             worker_sync();
             for (int q = tid; q < kRows1; q += kWorkers) {

@@ -71,16 +71,23 @@ __global__ void __launch_bounds__(128) label_fit_kernel(const double* __restrict
     for (int k = 0; k < dots; ++k) sv += v[k];
     const double mv = sv / dots;
     const double mx = x0 + 0.5 * (dots - 1) * step;  // x is an arithmetic progression
-    double sxx = 0.0, sxv = 0.0, svv = 0.0;
+    double sxx = 0.0, svv = 0.0, sdv = 0.0;
     bool constant = true;
     for (int k = 0; k < dots; ++k) {
         const double dx = (x0 + (double)k * step) - mx;
         const double dv = v[k] - mv;
         sxx += dx * dx;
-        sxv += dx * dv;
         svv += dv * dv;
+        sdv += dv;
         constant = constant && (v[k] == v[0]);
     }
+    // mv is the mean rounded to float64: on a track whose spread is a few ulps of its level (one value 1 ulp
+    // off a constant) the deviations from it are off by as much as they are wide.  The corrected two-pass sum
+    // removes that from svv.  sxv pairs the abscissae +-j*step around the centre, so it takes no mean at all and
+    // is exactly 0 on a track symmetric about its centre (slope 0: r = p = NaN, as lstsq + pearsonr give).
+    svv -= sdv * sdv / dots;
+    double sxv = 0.0;
+    for (int j = 1; j <= radius; ++j) sxv += (double)j * step * (v[radius + j] - v[radius - j]);
     const double a = sxv / sxx;
     const double b = mv - a * mx;
     double r, p;

@@ -180,14 +180,18 @@ __global__ void dense_frames_kernel(const float* __restrict__ env_t, int C, int 
         }
         if (threadIdx.x == 0 && !(mn > 0.f)) atomicOr(bad_flag, 1);
     }
+    // In double: in float32, log(max) - log(min) of a frame whose span is a few ulps cancels to 0 (then
+    // NaN) or to one ulp of log(min), several times the true span.
     const bool flat = normalize && (mn == mx);
-    const float lmn = normalize ? logf(mn) : 0.f;
-    const float inv = normalize ? 1.0f / (logf(mx) - lmn) : 1.f;
+    const double lmn = normalize ? log((double)mn) : 0.0;
+    const double inv = normalize ? 1.0 / (log((double)mx) - lmn) : 1.0;
     for (int e = threadIdx.x; e < total; e += blockDim.x) {
         const int k = e / C, c = e - k * C;
-        float v = src[(size_t)k * step * C + c];
-        if (normalize) v = flat ? 0.f : (logf(v) - lmn) * inv;
-        o[e] = (T)v;
+        const float v = src[(size_t)k * step * C + c];
+        if (normalize)
+            o[e] = (T)(flat ? 0.0 : (log((double)v) - lmn) * inv);
+        else
+            o[e] = (T)v;
     }
 }
 

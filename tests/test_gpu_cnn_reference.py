@@ -269,7 +269,10 @@ def test_flat_single_value_and_wide_range_frames(setup, net):
     g = torch.Generator(device="cuda").manual_seed(9)
     wide = torch.pow(10.0, torch.rand((rows, 128), device="cuda", generator=g) * 40 - 20)
     wide[400, 0], wide[1000, 127] = 1e-20, 1e20
-    for what, env in (("flat", flat), ("single", single), ("1e-20 .. 1e20", wide)):
+    # every value within 16 ulps of 3000: a float32 log(hi) - log(lo) would cancel to nothing or to one ulp of it
+    near = 3000.0 + 2.0 ** -12 * torch.randint(0, 17, (rows, 128), device="cuda", generator=g).float()
+    near[:, 0], near[:, 127] = 3000.0, 3000.0 + 16 * 2.0 ** -12
+    for what, env in (("flat", flat), ("single", single), ("1e-20 .. 1e20", wide), ("near-flat", near)):
         scores = tc.predict_envelope(env, 160, frames=(0, nf))
         _check(_stage_local(tc, ref, env, 160, 0, nf, scores), "%s %s" % (name, what))
         _chained(ref, env, 160, 0, nf, scores, "%s %s" % (name, what))
