@@ -18,6 +18,7 @@
 #include "f2_label.cuh"
 #include "f2_post.cuh"
 #include "f2_prep.cuh"
+#include "f2_sections.cuh"
 
 static_assert(F2_I16 == F2_DT_I16 && F2_F32 == F2_DT_F32 && F2_F64 == F2_DT_F64, "dtype codes");
 
@@ -84,61 +85,85 @@ void butter1(double cutoff_hz, double* b0, double* a1) {
     *a1 = -(4.0 - w) / (4.0 + w);
 }
 
+// ---- section coefficients of a make_erb_filters row k = [A0, A11, A12, A13, A14, A2, B0, B1, B2, gain] -----
+// 1 + B1 + B2 = |1 - pole|^2: how close the channel's poles come to z = 1
+double chan_cy(const double* k) { return 1.0 + (k[7] + k[8]) / k[6]; }
+
+// min of 1 + B1 + B2 over group g of 32 channels (one warp of the fused kernel, whose section form the
+// group takes from it)
+double group_min_cy(const double* coefs, int C, int g) {
+    double cy = 1e300;
+    for (int c = g * 32; c < std::min(C, g * 32 + 32); ++c) cy = std::min(cy, chan_cy(coefs + (size_t)c * 10));
+    return cy;
+}
+
+// The exact values of one channel's sections (FORM 2 runs them; the probe's float64 reference too)
+struct Sections {
+    double g4;     // A0^4/gain (A0 = A0/B0)
+    double z[4];   // A1k/A0
+    double b1, b2; // B1/B0, B2/B0
+    double nlr;    // -ln |pole|
+};
+
+// The channel's float32 entries of the parameter block (g4, z, dithered cq / ncy / nb1) written to
+// col[i * stride], and its exact values.
+Sections chan_sections(const double* k, float* col, size_t stride) {
+    Sections d;
+    const double a0n = k[0] / k[6];
+    d.g4 = a0n * a0n * a0n * a0n / k[9];
+    d.b1 = k[7] / k[6];
+    d.b2 = k[8] / k[6];
+    d.nlr = -0.5 * log(d.b2);
+    float cq[4], ncy[4], nb1[4];
+    dither4(d.b2, cq);
+    dither4(-(1.0 + d.b1 + d.b2), ncy);
+    dither4(-d.b1, nb1);
+    col[(size_t)f2::P_G4 * stride] = (float)d.g4;
+    for (int s = 0; s < 4; ++s) {
+        d.z[s] = k[1 + s] / k[0];
+        col[(size_t)(f2::P_Z + s) * stride] = (float)d.z[s];
+        col[(size_t)(f2::P_CQ + s) * stride] = cq[s];
+        col[(size_t)(f2::P_NCY + s) * stride] = ncy[s];
+        col[(size_t)(f2::P_NB1 + s) * stride] = nb1[s];
+    }
+    return d;
+}
+
 // ---- float32 tolerance guard -------------------------------------------------------------------
 // The kernels compute in float32 and are held to 1e-4 x channel RMS against the reference's float64
 // (north star).  How close a bank's poles may come to z = 1 before float32 round-off breaks that
 // depends on more than 1 + B1 + B2 (LOW_FREQ = 20 Hz passes at width 1 and 0.5 and fails at width 2
 // under a loud tone in the stop band, profiles/r01o_fuzz.log), so instead of a formula the plan is
 // TRIED: the real cascade of the channels nearest to z = 1 is run here on the host, once in float32
-// with exactly the kernel's operations (fmaf = FFMA, same order, same dithered coefficients, same
-// section form per channel group) and once in float64, on probe signals that cover the observed worst
-// cases -- loud tones far above the channel and white noise.  The error is measured the way the
-// parity tests measure it: max |y32 - y64| over max(channel RMS, 1 % of the loudest channel's).
-struct ProbeChan {
-    float z[4], cq[4], ncy[4], nb1[4], g4;
-    double zd[4], b1, b2, g4d;
-    bool direct;
-};
-
-double probe_channel(const ProbeChan& p, const float* x, int n, double loudest_rms) {
-    float y[4] = {0, 0, 0, 0}, q[4] = {0, 0, 0, 0}, up0 = 0.f;
+// through the kernels' own cascade_real (f2_sections.cuh: same fmaf calls in the same order, on the
+// parameter-block column the plan uploads, in the section form of the channel's group) and once in
+// float64, on probe signals that cover the observed worst cases -- loud tones far above the channel and
+// white noise.  The error is measured the way the parity tests measure it: max |y32 - y64| over
+// max(channel RMS, 1 % of the loudest channel's).
+template <int FORM>
+double probe_channel(const float* col, const Sections& d, const float* x, int n, double loudest_rms) {
+    f2::Coef k;
+    f2::load_coef<FORM>(col, nullptr, 1, 0, true, k);
+    f2::State s;
+    f2::reset(s);
     double Y[4] = {0, 0, 0, 0}, Y2[4] = {0, 0, 0, 0}, UP0 = 0.0;
     double err = 0.0, power = 0.0;
     for (int t = 0; t < n; ++t) {
-        // float32, as cascade_real<FORM> of f2_fused.cu
-        float u = x[t], up = up0;
-        up0 = u;
-        for (int i = 0; i < 4; ++i) {
-            const float in = fmaf(p.z[i], up, u);
-            const float yo = y[i];
-            float yn;
-            if (!p.direct) {
-                float qn = fmaf(p.cq[i], q[i], in);
-                qn = fmaf(p.ncy[i], yo, qn);
-                yn = yo + qn;
-                q[i] = qn;
-            } else {
-                yn = fmaf(p.nb1[i], yo, fmaf(-p.cq[i], q[i], in));
-                q[i] = yo;
-            }
-            y[i] = yn;
-            up = yo;
-            u = yn;
-        }
+        f2::cascade_real<FORM>(k, s, x[t]);
         // float64, exact coefficients: y[t] = in - b1 y[t-1] - b2 y[t-2]
         double U = x[t], UP = UP0;
         UP0 = U;
         for (int i = 0; i < 4; ++i) {
-            const double in = U + p.zd[i] * UP;
+            const double in = U + d.z[i] * UP;
             const double yo = Y[i];
-            const double yn = in - p.b1 * yo - p.b2 * Y2[i];
+            const double yn = in - d.b1 * yo - d.b2 * Y2[i];
             Y2[i] = yo;
             Y[i] = yn;
             UP = yo;
             U = yn;
         }
-        const double ref = Y[3] * p.g4d;
-        err = std::max(err, fabs((double)(p.g4 * y[3]) - ref));
+        const double ref = Y[3] * d.g4;
+        err = std::max(err, fabs((double)(k.g4 * s.y[3].x) - ref));
         power += ref * ref;
     }
     const double scale = std::max(sqrt(power / n), 0.01 * loudest_rms);
@@ -151,8 +176,8 @@ constexpr int kProbeChannels = 6;
 std::vector<int> nearest_to_one(const double* coefs, int c0, int c1) {
     std::vector<int> order;
     for (int c = c0; c < c1; ++c) order.push_back(c);
-    auto cy_of = [&](int c) { return 1.0 + (coefs[(size_t)c * 10 + 7] + coefs[(size_t)c * 10 + 8]) / coefs[(size_t)c * 10 + 6]; };
-    std::sort(order.begin(), order.end(), [&](int a, int b) { return cy_of(a) < cy_of(b); });
+    std::sort(order.begin(), order.end(),
+              [&](int a, int b) { return chan_cy(coefs + (size_t)a * 10) < chan_cy(coefs + (size_t)b * 10); });
     order.resize((size_t)std::min(c1 - c0, kProbeChannels));
     return order;
 }
@@ -161,7 +186,6 @@ std::vector<int> nearest_to_one(const double* coefs, int c0, int c1) {
 double probe_float32_error(const double* coefs, int C, const std::vector<int>& order, int* worst_channel) {
     constexpr int kProbeLen = 8192;
     constexpr double kAmp = 8000.0;
-    auto cy_of = [&](int c) { return 1.0 + (coefs[(size_t)c * 10 + 7] + coefs[(size_t)c * 10 + 8]) / coefs[(size_t)c * 10 + 6]; };
     std::vector<float> x((size_t)kProbeLen);
     double worst = 0.0;
     if (worst_channel) *worst_channel = order.empty() ? 0 : order[0];
@@ -184,23 +208,11 @@ double probe_float32_error(const double* coefs, int C, const std::vector<int>& o
             loudest = 0.0;  // broadband: every channel is held to its own RMS
         }
         for (int c : order) {
-            const double* k = coefs + (size_t)c * 10;
-            ProbeChan p;
-            const double b1 = k[7] / k[6], b2 = k[8] / k[6], a0n = k[0] / k[6];
-            dither4(b2, p.cq);
-            dither4(-(1.0 + b1 + b2), p.ncy);
-            dither4(-b1, p.nb1);
-            for (int s = 0; s < 4; ++s) {
-                p.zd[s] = k[1 + s] / k[0];
-                p.z[s] = (float)p.zd[s];
-            }
-            p.b1 = b1, p.b2 = b2;
-            p.g4d = a0n * a0n * a0n * a0n / k[9];
-            p.g4 = (float)p.g4d;
-            double group_cy = 1e300;  // the kernel picks the section form per group of 32 channels
-            for (int cc = c / 32 * 32; cc < std::min(C, c / 32 * 32 + 32); ++cc) group_cy = std::min(group_cy, cy_of(cc));
-            p.direct = group_cy >= kDirectMinCyGfb;
-            const double e = probe_channel(p, x.data(), kProbeLen, loudest) / 1e-4;
+            float col[f2::kNumChanPar] = {};
+            const Sections d = chan_sections(coefs + (size_t)c * 10, col, 1);
+            const bool direct = group_min_cy(coefs, C, c / 32) >= kDirectMinCyGfb;
+            const double e = (direct ? probe_channel<1>(col, d, x.data(), kProbeLen, loudest)
+                                     : probe_channel<0>(col, d, x.data(), kProbeLen, loudest)) / 1e-4;
             if (e > worst) {
                 worst = e;
                 if (worst_channel) *worst_channel = c;
@@ -334,6 +346,7 @@ int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned 
     const int C = n_channels;
     const int c_pad = (int)align_up((size_t)C, 32);
     std::vector<float> par((size_t)f2::kNumChanPar * c_pad, 0.f);
+    std::vector<Sections> sec((size_t)C);
     double min_nlr = 1e300;
     for (int c = 0; c < C; ++c) {
         const double* k = coefs + (size_t)c * 10;
@@ -345,41 +358,23 @@ int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned 
         if (!(b2 > 0.0 && b2 < 1.0) || !(fabs(b1) < 1.0 + b2))
             return fail(F2_ERR_UNSUPPORTED, "channel %d: poles are not a stable complex pair", c);
         if (!(A0 != 0.0)) return fail(F2_ERR_INVALID, "channel %d: A0 == 0", c);
-        const double a0n = A0 / B0;
-        par[(size_t)f2::P_G4 * c_pad + c] = (float)(a0n * a0n * a0n * a0n / gain);
-        for (int s = 0; s < 4; ++s) par[(size_t)(f2::P_Z + s) * c_pad + c] = (float)(k[1 + s] / A0);
-        float cq[4], ncy[4], nb1[4];
-        dither4(b2, cq);
-        dither4(-(1.0 + b1 + b2), ncy);
-        dither4(-b1, nb1);
-        for (int s = 0; s < 4; ++s) {
-            par[(size_t)(f2::P_CQ + s) * c_pad + c] = cq[s];
-            par[(size_t)(f2::P_NCY + s) * c_pad + c] = ncy[s];
-            par[(size_t)(f2::P_NB1 + s) * c_pad + c] = nb1[s];
-        }
-        min_nlr = std::min(min_nlr, -0.5 * log(b2));  // -ln(pole radius)
+        sec[(size_t)c] = chan_sections(k, par.data() + c, (size_t)c_pad);
+        min_nlr = std::min(min_nlr, sec[(size_t)c].nlr);
     }
-    // Per group of 32 channels (one warp of the fused kernel): min of 1 + B1 + B2 = |1 - pole|^2.
-    // The fused kernel runs the direct form (3 FMAs per section) where this is large enough for its
-    // float32 round-off to match the delta form's, and the delta form nearer to z = 1.
     for (int g0 = 0; g0 < c_pad; g0 += 32) {
-        double cy = 1e300;
-        for (int c = g0; c < std::min(C, g0 + 32); ++c) {
-            const double* k = coefs + (size_t)c * 10;
-            cy = std::min(cy, 1.0 + (k[7] + k[8]) / k[6]);
-        }
-        for (int c = g0; c < g0 + 32; ++c) par[(size_t)f2::P_FORM * c_pad + c] = (float)cy;
-    }
-    // Per group: how much sooner than the bank's slowest channel the group's slowest channel forgets
-    // (ratio of -ln|pole|, rounded up a little so that float32 never shortens a length).
-    for (int g0 = 0; g0 < c_pad; g0 += 32) {
+        // Per group of 32 channels (one warp of the fused kernel): min of 1 + B1 + B2.  The fused kernel
+        // runs the direct form (3 FMAs per section) where this is large enough for its float32 round-off
+        // to match the delta form's, and the delta form nearer to z = 1.
+        const float cy = (float)group_min_cy(coefs, C, g0 / 32);
+        // How much sooner than the bank's slowest channel the group's slowest channel forgets
+        // (ratio of -ln|pole|, rounded up a little so that float32 never shortens a length).
         double nlr = 1e300;
-        for (int c = g0; c < std::min(C, g0 + 32); ++c) {
-            const double* k = coefs + (size_t)c * 10;
-            nlr = std::min(nlr, -0.5 * log(k[8] / k[6]));
-        }
+        for (int c = g0; c < std::min(C, g0 + 32); ++c) nlr = std::min(nlr, sec[(size_t)c].nlr);
         const float scale = (float)std::min(1.0, min_nlr / nlr * (1.0 + 1e-6));
-        for (int c = g0; c < g0 + 32; ++c) par[(size_t)f2::P_WSCALE * c_pad + c] = scale;
+        for (int c = g0; c < g0 + 32; ++c) {
+            par[(size_t)f2::P_FORM * c_pad + c] = cy;
+            par[(size_t)f2::P_WSCALE * c_pad + c] = scale;
+        }
     }
     // F2_PLAN_FLOAT64_SECTIONS: in a bank f2_bank_check refuses, the groups predicted to leave the tolerance in
     // float32 run FORM 2.  A bank it accepts keeps float32 everywhere, so that the flag never changes its
@@ -395,12 +390,11 @@ int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned 
         par64.assign((size_t)f2::kNumChanPar64 * c_pad, 0.0);
         for (int c = 0; c < C; ++c) {
             if (!f64_group[(size_t)(c / 32)]) continue;
-            const double* k = coefs + (size_t)c * 10;
-            const double a0n = k[0] / k[6];
-            par64[(size_t)f2::P64_G4 * c_pad + c] = a0n * a0n * a0n * a0n / k[9];
-            for (int s = 0; s < 4; ++s) par64[(size_t)(f2::P64_Z + s) * c_pad + c] = k[1 + s] / k[0];
-            par64[(size_t)f2::P64_B1 * c_pad + c] = k[7] / k[6];
-            par64[(size_t)f2::P64_B2 * c_pad + c] = k[8] / k[6];
+            const Sections& d = sec[(size_t)c];
+            par64[(size_t)f2::P64_G4 * c_pad + c] = d.g4;
+            for (int s = 0; s < 4; ++s) par64[(size_t)(f2::P64_Z + s) * c_pad + c] = d.z[s];
+            par64[(size_t)f2::P64_B1 * c_pad + c] = d.b1;
+            par64[(size_t)f2::P64_B2 * c_pad + c] = d.b2;
         }
         for (int c = 0; c < c_pad; ++c)
             if (f64_group[(size_t)(c / 32)]) par[(size_t)f2::P_FORM * c_pad + c] = f2::kForm2Marker;
@@ -414,8 +408,7 @@ int f2_plan_create_ex(const double* coefs, int n_channels, int device, unsigned 
             return fail(F2_ERR_UNSUPPORTED,
                         "filterbank too close to z = 1 for float32: channel %d (1+B1+B2 = %.3g) is predicted to miss "
                         "the 1e-4 x RMS tolerance by %.1fx (f2_bank_check); widen LOW_FREQ / lower `width`, or set "
-                        "F2CNN_B200_ALLOW_IMPRECISE=1 to run anyway", bad,
-                        1.0 + (coefs[(size_t)bad * 10 + 7] + coefs[(size_t)bad * 10 + 8]) / coefs[(size_t)bad * 10 + 6], predicted);
+                        "F2CNN_B200_ALLOW_IMPRECISE=1 to run anyway", bad, chan_cy(coefs + (size_t)bad * 10), predicted);
     }
     f2_plan* p = new (std::nothrow) f2_plan();
     if (!p) return fail(F2_ERR_INVALID, "out of host memory");
@@ -669,7 +662,7 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
     std::vector<f2::Item> items = build_items(seg_of, !equal_cost);
     std::vector<f2::Item> items_uniform;
     if (equal_cost) items_uniform = build_items(seg_same, true);
-    // the items of FORM 2 groups go last: the second launch (launch_fused64) runs them
+    // the items of FORM 2 groups go last: the second launch (launch_fused with float64) runs them
     auto split_form2 = [&](std::vector<f2::Item>& v) {
         if (plan->n_f64 == 0) return 0LL;
         auto mid = std::stable_partition(v.begin(), v.end(),
@@ -881,12 +874,12 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
             F2_CUDA(f2::launch_edge_scan(b->d_utts, b->n_utts, plan->d_chan, plan->d_scan_mats, plan->C, plan->c_pad, xz,
                                          edge, stream));
         else
-            F2_CUDA(f2::launch_edge(b->d_utts, b->n_utts, plan->d_chan, plan->C, plan->c_pad, xz, plan->w_edge, edge,
-                                    stream));
+            F2_CUDA(f2::launch_edge<0>(b->d_utts, b->n_utts, plan->d_chan, nullptr, plan->C, plan->c_pad, xz,
+                                       plan->w_edge, edge, stream));
         fp.edge = edge;
         if (plan->n_f64)
-            F2_CUDA(f2::launch_edge64(b->d_utts, b->n_utts, plan->d_chan, plan->d_chan64, plan->C, plan->c_pad, xz,
-                                      plan->w_edge, edge64, stream));
+            F2_CUDA(f2::launch_edge<2>(b->d_utts, b->n_utts, plan->d_chan, plan->d_chan64, plan->C, plan->c_pad, xz,
+                                       plan->w_edge, edge64, stream));
     }
     fp.C = plan->C;
     fp.c_pad = plan->c_pad;
@@ -907,12 +900,12 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     if (a->ev_fused_start) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_start, stream));
     const long long n_items = uniform_chunks ? b->n_items_uniform : b->n_items;
     const long long n_f64 = uniform_chunks ? b->n_items_uniform_f64 : b->n_items_f64;
-    F2_CUDA(f2::launch_fused(fp, (int)(n_items - n_f64), stream));
+    F2_CUDA(f2::launch_fused(fp, (int)(n_items - n_f64), false, stream));
     if (n_f64 > 0) {
         f2::FusedParams fp64 = fp;
         fp64.items = fp.items + (n_items - n_f64);
         fp64.edge64 = fp.edge ? edge64 : nullptr;
-        F2_CUDA(f2::launch_fused64(fp64, (int)n_f64, stream));
+        F2_CUDA(f2::launch_fused(fp64, (int)n_f64, true, stream));
     }
     if (a->ev_fused_stop) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_stop, stream));
 

@@ -1,13 +1,11 @@
 // f2_edge.cu -- edge residuals e_k of the zero-padded ring equation (DESIGN.md section 3, H1).
 //
-// For every (utterance, channel) the real cascade's state after the last sample n-1 gives
-//   e0_k = b1*y_k[n-1] + b2*y_k[n-2] - z_k*u_k[n-1] = (cy-1)*y - cq*q - z_k*u,   e1_k = cq*y
-// (a0-free stage variables).  All sections are strictly stable, so the state depends on the
-// last w_edge samples only (to float32 resolution).
+// For every (utterance, channel) the real cascade's state after the last sample n-1 gives the
+// residuals e0_k, e1_k (edge_residuals, f2_sections.cuh).  All sections are strictly stable, so
+// the state depends on the last w_edge samples only (to float32 resolution).
 //
-// Two kernels produce the same [utt][C][8] table (entries 0..3 multiply G at even t, 4..7 at
-// odd t):
-//  * edge_kernel      -- one thread per channel, sequential over the window.  Used when there
+// Two kernels produce the same float [utt][C][8] table (f2_sections.cuh: store_edge_entry):
+//  * edge_kernel<0>   -- one thread per channel, sequential over the window.  Used when there
 //                        are enough (utterance, channel) pairs to fill the GPU.
 //  * edge_scan_kernel -- chunked parallel linear-recurrence scan for small batches (a single
 //                        utterance would otherwise wait for 2048 sequential steps): one warp
@@ -17,143 +15,69 @@
 //                        __shfl_up_sync.  M = A^64 is the block transition of the four coupled
 //                        biquads (lower block-triangular, one 2x2 block per section on the
 //                        diagonal), its powers are precomputed per channel in float64.
+// edge_kernel<2> fills the float64 table of the FORM 2 groups with the fused kernel's FORM 2 sections.
 #include "f2_edge.cuh"
 
 #include <math.h>
 
 namespace f2 {
 
-__device__ __forceinline__ void real_step(const float (&z)[4], const float (&cq)[4], const float (&ncy)[4],
-                                          float (&y)[4], float (&q)[4], float u, float up) {
+// Residuals of channel c from the real cascade's state after sample n-1, into the table entry of utterance utt.
+// real_only (N2 <= 2): the analytic signal is real, nothing is injected.
+template <int FORM, class K, class S, class E>
+__device__ __forceinline__ void write_edge(const K& k, const S& s, int n, bool real_only, E* edge, size_t utt, int C,
+                                           int c) {
+    E e0[4], e1[4], ee[4], eo[4];
+    edge_residuals<FORM>(k, s, e0, e1);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-        const float in = fmaf(z[i], up, u);
-        const float yo = y[i];
-        float qn = fmaf(cq[i], q[i], in);
-        qn = fmaf(ncy[i], yo, qn);
-        const float yn = yo + qn;
-        q[i] = qn;
-        y[i] = yn;
-        up = yo;
-        u = yn;
+        e0[i] = real_only ? E(0) : e0[i];
+        e1[i] = real_only ? E(0) : e1[i];
     }
+    edge_parity(n, e0, e1, ee, eo);
+    store_edge_entry(edge, utt, C, c, ee, eo);
 }
 
-__device__ __forceinline__ void store_edge(const float (&z)[4], const float (&cq)[4], const float (&ncy)[4],
-                                           const float (&y)[4], const float (&q)[4], float x_last, int n, bool real_only,
-                                           float* __restrict__ dst) {
-    float e0[4], e1[4];
-    float uprev = x_last;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const float cy = -ncy[i];
-        e0[i] = real_only ? 0.f : fmaf(cy - 1.0f, y[i], -cq[i] * q[i]) - z[i] * uprev;
-        e1[i] = real_only ? 0.f : cq[i] * y[i];
-        uprev = y[i];
-    }
-    const bool n_odd = (n & 1) != 0;  // (t - n) odd -> e0 multiplies G[t]
-    float4* o = reinterpret_cast<float4*>(dst);
-    o[0] = n_odd ? make_float4(e0[0], e0[1], e0[2], e0[3]) : make_float4(e1[0], e1[1], e1[2], e1[3]);
-    o[1] = n_odd ? make_float4(e1[0], e1[1], e1[2], e1[3]) : make_float4(e0[0], e0[1], e0[2], e0[3]);
-}
-
-__global__ void __launch_bounds__(kEdgeChanPerBlock) edge_kernel(const UttDesc* utts, const float* __restrict__ chan,
-                                                             int C, int c_pad, const float2* __restrict__ xz,
-                                                             int w_edge, float* __restrict__ edge) {
+// Sequential pass, one thread per channel, from zero state w_edge samples before the end.  The float32 pass
+// runs the delta form (FORM 0) for every group, the form build_scan_matrices describes, so that it and the
+// scan give the same table.  FORM 2: one warp per group of 32 channels; groups that are not FORM 2 leave at
+// once, and their entries of the float64 table are not written.
+template <int FORM>
+__global__ void __launch_bounds__(FORM == 2 ? kChanPerBlock : kEdgeChanPerBlock)
+    edge_kernel(const UttDesc* utts, const float* __restrict__ chan, int C, int c_pad, const float2* __restrict__ xz,
+                int w_edge, typename SectionTypes<FORM>::E* __restrict__ edge, const double* __restrict__ chan64) {
+    constexpr int W = FORM == 2 ? kChanPerBlock : kEdgeChanPerBlock;
     const UttDesc ut = utts[blockIdx.x];
-    const int c = blockIdx.y * kEdgeChanPerBlock + threadIdx.x;
+    const int c = blockIdx.y * W + threadIdx.x;
+    if (FORM == 2 && chan[P_FORM * c_pad + blockIdx.y * W] != kForm2Marker) return;
     if (c >= C || ut.n <= 0) return;
-    float z[4], cq[4], ncy[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        z[i] = chan[(P_Z + i) * c_pad + c];
-        cq[i] = chan[(P_CQ + i) * c_pad + c];
-        ncy[i] = chan[(P_NCY + i) * c_pad + c];
-    }
-    float y[4] = {0.f, 0.f, 0.f, 0.f}, q[4] = {0.f, 0.f, 0.f, 0.f};
-    float up = 0.f;
+    typename SectionTypes<FORM>::K k;
+    load_coef<FORM>(chan, chan64, c_pad, c, true, k);
+    typename SectionTypes<FORM>::S s;
+    reset(s);
     const int n = ut.n;
     const int t0 = n - w_edge > 0 ? n - w_edge : 0;
     const float2* src = xz + ut.ring_off;
     if (ut.N2 > 2) {
 #pragma unroll 4
-        for (int t = t0; t < n; ++t) {
-            const float u = __ldg(&src[t].x);
-            real_step(z, cq, ncy, y, q, u, up);
-            up = u;
-        }
+        for (int t = t0; t < n; ++t) cascade_real<FORM>(k, s, __ldg(&src[t].x));
     }
-    store_edge(z, cq, ncy, y, q, up, n, ut.N2 <= 2, edge + ((size_t)blockIdx.x * C + c) * 8);
+    write_edge<FORM>(k, s, n, ut.N2 <= 2, edge, blockIdx.x, C, c);
 }
 
-cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, int C, int c_pad, const float2* xz,
-                        int w_edge, float* edge, cudaStream_t stream) {
+template <int FORM>
+cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
+                        const float2* xz, int w_edge, typename SectionTypes<FORM>::E* edge, cudaStream_t stream) {
     if (n_utts <= 0) return cudaSuccess;
-    dim3 grid(n_utts, (C + kEdgeChanPerBlock - 1) / kEdgeChanPerBlock);
-    edge_kernel<<<grid, kEdgeChanPerBlock, 0, stream>>>(utts, chan, C, c_pad, xz, w_edge, edge);
+    constexpr int W = FORM == 2 ? kChanPerBlock : kEdgeChanPerBlock;
+    dim3 grid(n_utts, (C + W - 1) / W);
+    edge_kernel<FORM><<<grid, W, 0, stream>>>(utts, chan, C, c_pad, xz, w_edge, edge, chan64);
     return cudaGetLastError();
 }
-
-// ---- FORM 2 groups: float64 direct-form residuals ---------------------------------------------
-// One CTA per (utterance, group of 32 channels); groups that are not FORM 2 leave at once.  The same
-// recurrence as cascade_real / edge_residuals of the fused kernel's FORM 2, from zero state w_edge
-// samples before the end.
-__global__ void __launch_bounds__(32) edge_kernel64(const UttDesc* utts, const float* __restrict__ chan,
-                                                    const double* __restrict__ chan64, int C, int c_pad,
-                                                    const float2* __restrict__ xz, int w_edge,
-                                                    double* __restrict__ edge) {
-    const UttDesc ut = utts[blockIdx.x];
-    const int c = blockIdx.y * 32 + threadIdx.x;
-    if (chan[P_FORM * c_pad + blockIdx.y * 32] != kForm2Marker || c >= C || ut.n <= 0) return;
-    double z[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) z[i] = chan64[(P64_Z + i) * c_pad + c];
-    const double b1 = chan64[P64_B1 * c_pad + c], b2 = chan64[P64_B2 * c_pad + c];
-    double y[4] = {0.0, 0.0, 0.0, 0.0}, y2[4] = {0.0, 0.0, 0.0, 0.0};
-    double up = 0.0;
-    const int n = ut.n;
-    const int t0 = n - w_edge > 0 ? n - w_edge : 0;
-    const float2* src = xz + ut.ring_off;
-    if (ut.N2 > 2) {
-#pragma unroll 4
-        for (int t = t0; t < n; ++t) {
-            double u = __ldg(&src[t].x), upi = up;
-            up = u;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const double yn = fma(-b1, y[i], fma(-b2, y2[i], fma(z[i], upi, u)));
-                upi = y[i];
-                y2[i] = y[i];
-                y[i] = yn;
-                u = yn;
-            }
-        }
-    }
-    double e0[4], e1[4];
-    double uprev = up;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const bool real_only = ut.N2 <= 2;
-        e0[i] = real_only ? 0.0 : fma(b1, y[i], b2 * y2[i]) - z[i] * uprev;
-        e1[i] = real_only ? 0.0 : b2 * y[i];
-        uprev = y[i];
-    }
-    const bool n_odd = (n & 1) != 0;  // (t - n) odd -> e0 multiplies G[t]
-    double* o = edge + ((size_t)blockIdx.x * C + c) * 8;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        o[i] = n_odd ? e0[i] : e1[i];
-        o[4 + i] = n_odd ? e1[i] : e0[i];
-    }
-}
-
-cudaError_t launch_edge64(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
-                          const float2* xz, int w_edge, double* edge, cudaStream_t stream) {
-    if (n_utts <= 0) return cudaSuccess;
-    dim3 grid(n_utts, (C + 31) / 32);
-    edge_kernel64<<<grid, 32, 0, stream>>>(utts, chan, chan64, C, c_pad, xz, w_edge, edge);
-    return cudaGetLastError();
-}
+template cudaError_t launch_edge<0>(const UttDesc*, int, const float*, const double*, int, int, const float2*, int,
+                                    float*, cudaStream_t);
+template cudaError_t launch_edge<2>(const UttDesc*, int, const float*, const double*, int, int, const float2*, int,
+                                    double*, cudaStream_t);
 
 // ---- scan version ----------------------------------------------------------------------------
 constexpr int kScanWarps = 4;                  // channels per CTA (they share the staged window)
@@ -180,48 +104,45 @@ __global__ void __launch_bounds__(kScanWarps * 32) edge_scan_kernel(const UttDes
     __syncthreads();
     const int c = blockIdx.y * kScanWarps + warp;
     if (c >= C) return;
-    float z[4], cq[4], ncy[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        z[i] = chan[(P_Z + i) * c_pad + c];
-        cq[i] = chan[(P_CQ + i) * c_pad + c];
-        ncy[i] = chan[(P_NCY + i) * c_pad + c];
-    }
+    Coef k;
+    load_coef<0>(chan, nullptr, c_pad, c, true, k);
     // 1. every lane: its block of 64 samples from zero state (the true previous input sample
     //    is part of the block's input response, not of the carried state)
-    float y[4] = {0.f, 0.f, 0.f, 0.f}, q[4] = {0.f, 0.f, 0.f, 0.f};
+    State s;
+    reset(s);
     const float* xb = s_x + 1 + lane * kScanPitch;
-    float up = lane == 0 ? s_x[0] : s_x[1 + (lane - 1) * kScanPitch + kScanBlock - 1];
+    s.up.x = lane == 0 ? s_x[0] : s_x[1 + (lane - 1) * kScanPitch + kScanBlock - 1];
 #pragma unroll 4
-    for (int i = 0; i < kScanBlock; ++i) {
-        const float u = xb[i];
-        real_step(z, cq, ncy, y, q, u, up);
-        up = u;
-    }
-    const float x_last = __shfl_sync(0xffffffffu, up, 31);
+    for (int i = 0; i < kScanBlock; ++i) cascade_real<0>(k, s, xb[i]);
+    const float x_last = __shfl_sync(0xffffffffu, s.up.x, 31);
     // 2. Kogge-Stone composition of the carries: S_j += M^(2^d) * S_(j - 2^d)
-    float S[8] = {y[0], q[0], y[1], q[1], y[2], q[2], y[3], q[3]};
+    float S[8] = {s.y[0].x, s.q[0].x, s.y[1].x, s.q[1].x, s.y[2].x, s.q[2].x, s.y[3].x, s.q[3].x};
     const float* M = mats + (size_t)c * kScanLevels * 64;
 #pragma unroll
     for (int d = 0; d < kScanLevels; ++d) {
         float P[8];
 #pragma unroll
-        for (int k = 0; k < 8; ++k) P[k] = __shfl_up_sync(0xffffffffu, S[k], 1 << d);
+        for (int j = 0; j < 8; ++j) P[j] = __shfl_up_sync(0xffffffffu, S[j], 1 << d);
         if (lane >= (1 << d)) {
             const float* Md = M + d * 64;
 #pragma unroll
             for (int r = 0; r < 8; ++r) {
                 float acc = S[r];
 #pragma unroll
-                for (int k = 0; k < 8; ++k) acc = fmaf(__ldg(Md + r * 8 + k), P[k], acc);
+                for (int j = 0; j < 8; ++j) acc = fmaf(__ldg(Md + r * 8 + j), P[j], acc);
                 S[r] = acc;
             }
         }
     }
     // 3. lane 31 holds the state after sample n-1
     if (lane == 31) {
-        const float yy[4] = {S[0], S[2], S[4], S[6]}, qq[4] = {S[1], S[3], S[5], S[7]};
-        store_edge(z, cq, ncy, yy, qq, x_last, n, ut.N2 <= 2, edge + ((size_t)blockIdx.x * C + c) * 8);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            s.y[i].x = S[2 * i];
+            s.q[i].x = S[2 * i + 1];
+        }
+        s.up.x = x_last;
+        write_edge<0>(k, s, n, ut.N2 <= 2, edge, blockIdx.x, C, c);
     }
 }
 

@@ -1,7 +1,7 @@
 // f2_edge.cuh -- edge residuals of the zero-padded ring equation, one pass per utterance
 // (f2_edge.cu): sequential kernel for full GPUs, chunked scan kernel for small batches.
 #pragma once
-#include "f2_common.cuh"
+#include "f2_sections.cuh"
 
 namespace f2 {
 
@@ -9,13 +9,12 @@ constexpr int kScanBlock = 64;    // samples per lane block of the edge scan
 constexpr int kScanLevels = 5;    // Kogge-Stone offsets 1, 2, 4, 8, 16 blocks
 constexpr int kScanWindow = 32 * kScanBlock;  // 2048 samples: the last w_edge samples
 
-// seq: one thread per channel runs the real cascade over the last w_edge samples.
-cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, int C, int c_pad, const float2* xz,
-                        int w_edge, float* edge, cudaStream_t stream);
-// FORM 2 groups (P_FORM == kForm2Marker): float64 sequential pass over the last w_edge samples into a
-// float64 table [utt][C][8] (same layout); the entries of other groups are not written.
-cudaError_t launch_edge64(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
-                          const float2* xz, int w_edge, double* edge, cudaStream_t stream);
+// seq: one thread per channel runs the real cascade over the last w_edge samples.  FORM 0: the float32
+// delta-form pass of every group into the float table.  FORM 2: the groups with P_FORM == kForm2Marker in
+// float64 into a float64 table of the same layout; the entries of other groups are not written.
+template <int FORM>
+cudaError_t launch_edge(const UttDesc* utts, int n_utts, const float* chan, const double* chan64, int C, int c_pad,
+                        const float2* xz, int w_edge, typename SectionTypes<FORM>::E* edge, cudaStream_t stream);
 // scan: one warp per (utterance, channel); lane = block of 64 samples run from zero state;
 // the 8-state cascade carries are composed across lanes with precomputed block transition
 // powers M^(2^d) (lower block-triangular, 2x2 blocks per biquad) and warp shuffles.

@@ -32,12 +32,11 @@ struct FusedParams {
     int w_casc;
     int w_lpf;
     float direct_min_cy; // groups of 32 channels with min(1+B1+B2) >= this run the direct-form sections
-    const double* chan64;  // [kNumChanPar64][c_pad] float64 block of the FORM 2 groups (launch_fused64 only)
+    const double* chan64;  // [kNumChanPar64][c_pad] float64 block of the FORM 2 groups (FORM 2 launch only)
     const double* edge64;  // float64 edge residuals [utt][C][8] of the FORM 2 groups (f2_edge.cu; null: in-kernel)
 };
 
-cudaError_t launch_fused(const FusedParams& p, int n_items, cudaStream_t stream);
-// The work items of FORM 2 groups (float64 sections): its own instantiation of the fused kernel.
-cudaError_t launch_fused64(const FusedParams& p, int n_items, cudaStream_t stream);
+// float64: p.items are work items of FORM 2 groups (float64 sections), run by their own instantiations.
+cudaError_t launch_fused(const FusedParams& p, int n_items, bool float64, cudaStream_t stream);
 
 }  // namespace f2

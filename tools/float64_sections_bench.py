@@ -89,10 +89,10 @@ def main():
         torch.cuda.synchronize()
     ktime = {}
     for e in prof.key_averages():
-        for tag in ("fused_kernel64", "fused_kernel<", "ring_cluster", "edge"):
+        for tag in ("fused_kernel<true", "fused_kernel<false", "ring_cluster", "edge"):   # <true: FORM 2 (float64)
             if tag in e.key:
                 ktime.setdefault(tag, []).append((e.key[:90], e.count, e.device_time_total / max(e.count, 1) / 1e3))
-    f64_ms = sum(t for k, c, t in ktime.get("fused_kernel64", []))
+    f64_ms = sum(t for k, c, t in ktime.get("fused_kernel<true", []))
     res["kernels_ms_per_call"] = {k: [(name, c, round(t, 3)) for name, c, t in v] for k, v in ktime.items()}
     res["form2_launch_ms"] = round(f64_ms, 3)
     res["form2_dfma_per_pass"] = dfma
