@@ -294,7 +294,6 @@ struct f2_batch {
     // the last n_items_f64 (n_items_uniform_f64) of each list belong to FORM 2 groups
     long long n_items_f64 = 0, n_items_uniform_f64 = 0;
     long long total_samples = 0, total_frames = 0, total_ring = 0;
-    int max_n = 0;
     int min_log2 = 0, max_log2 = 0;
     int private_g = 0;  // utterances without a shared injection table
 };
@@ -534,7 +533,6 @@ int f2_batch_create(f2_plan* plan, const int64_t* lengths, int n_utts, int step,
         if (n > 0) {
             b->min_log2 = std::min(b->min_log2, lg);
             b->max_log2 = std::max(b->max_log2, lg);
-            b->max_n = std::max(b->max_n, (int)n);
         }
     }
     if (b->min_log2 > b->max_log2) b->min_log2 = b->max_log2 = 0;
@@ -737,11 +735,8 @@ int f2_batch_frame_offsets(const f2_batch* b, int64_t* frame_offsets) {
     return F2_OK;
 }
 
-// workspace: [Z floats][xz float2][G floats][gfb_t][env_t], each section 256-byte aligned
+// workspace: [Z floats][xz float2][G floats][edge][edge64], each section 256-byte aligned
 static size_t ws_ring_bytes(long long total_ring) { return align_up((size_t)total_ring * 4, 256); }
-static size_t ws_full_bytes(const f2_batch* b) {
-    return align_up((size_t)b->total_samples * (size_t)b->plan->C * sizeof(float), 256);
-}
 
 static size_t ws_edge_bytes(const f2_batch* b) {
     return align_up((size_t)b->n_utts * (size_t)b->plan->C * 8 * sizeof(float), 256);
@@ -761,12 +756,9 @@ static int ws_ring_units(const f2_batch* b) {
     return compact ? 2 : 4;
 }
 
-size_t f2_batch_workspace_bytes(const f2_batch* b, int want_full_gfb, int want_full_env) {
+size_t f2_batch_workspace_bytes(const f2_batch* b, int, int) {
     if (!b) return 0;
-    size_t s = (size_t)ws_ring_units(b) * ws_ring_bytes(b->total_ring) + ws_edge_bytes(b) + ws_edge64_bytes(b);
-    if (want_full_gfb) s += ws_full_bytes(b);
-    if (want_full_env) s += ws_full_bytes(b);
-    return s + 256;
+    return (size_t)ws_ring_units(b) * ws_ring_bytes(b->total_ring) + ws_edge_bytes(b) + ws_edge64_bytes(b) + 256;
 }
 
 int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t workspace_bytes, void* stream_) {
@@ -787,14 +779,7 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
         if (!a->win_offsets || a->win_dots < 1)
             return fail(F2_ERR_INVALID, "f2_batch_run: `windows` needs win_offsets and win_dots >= 1");
     }
-    // (C, n) outputs: written by the fused kernel itself through a shared-memory transpose, unless the
-    // time-major envelope is wanted as well -- then the envelope is computed once into env_t and transposed
-    // (and the filterbank output takes the same route)
-    const bool direct_cn = (a->gfb != nullptr || a->env != nullptr) && a->env_t == nullptr &&
-                           (a->gfb == nullptr || a->env == nullptr || a->gfb_dtype == a->env_dtype);
-    const bool want_gfb = a->gfb != nullptr && !direct_cn;
-    const bool want_env_scratch = a->env != nullptr && a->env_t == nullptr && !direct_cn;
-    const size_t need = f2_batch_workspace_bytes(b, want_gfb, want_env_scratch);
+    const size_t need = f2_batch_workspace_bytes(b, 0, 0);
     if (!workspace || workspace_bytes < need)
         return fail(F2_ERR_WORKSPACE, "workspace %zu bytes, need %zu", workspace_bytes, need);
     double b0 = 0.0, a1 = 0.0;
@@ -816,18 +801,7 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     float* G = units == 4 ? (float*)(ws + 3 * rb) : nullptr;
     float* edge = (float*)(ws + (size_t)units * rb);
     double* edge64 = (double*)(ws + (size_t)units * rb + ws_edge_bytes(b));
-    char* cur = ws + (size_t)units * rb + ws_edge_bytes(b) + ws_edge64_bytes(b);
-    float* gfb_t = nullptr;
-    float* env_t = a->env_t;
-    if (want_gfb) {
-        gfb_t = (float*)cur;
-        cur += ws_full_bytes(b);
-    }
-    if (want_env_scratch) {
-        env_t = (float*)cur;
-        cur += ws_full_bytes(b);
-    }
-    const bool need_env = env_t != nullptr || a->dec != nullptr || a->windows != nullptr || (direct_cn && a->env != nullptr);
+    const bool need_env = a->env_t != nullptr || a->dec != nullptr || a->windows != nullptr || a->env != nullptr;
 
     f2::PrepParams pp;
     pp.utts = b->d_utts;
@@ -848,16 +822,17 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     f2::FusedParams fp;
     fp.utts = b->d_utts;
     // the filterbank output is store-bound and uses the direct form for fewer groups: equal-length chunks
-    const bool uniform_chunks = (gfb_t != nullptr || (direct_cn && a->gfb != nullptr)) && b->d_items_uniform != nullptr;
+    const bool uniform_chunks = a->gfb != nullptr && b->d_items_uniform != nullptr;
     fp.items = uniform_chunks ? b->d_items_uniform : b->d_items;
     fp.chan = plan->d_chan;
     fp.xz = xz;
     fp.G = G;
-    fp.gfb_t = gfb_t;
-    fp.env_t = env_t;
-    fp.gfb_cn = direct_cn ? a->gfb : nullptr;
-    fp.env_cn = direct_cn ? a->env : nullptr;
-    fp.cn_f64 = direct_cn && (a->gfb ? a->gfb_dtype : a->env_dtype) == F2_F64 ? 1 : 0;
+    fp.env_t = a->env_t;
+    // (C, n) outputs: written by the fused kernel itself through a shared-memory transpose, each in its own dtype
+    fp.gfb_cn = a->gfb;
+    fp.env_cn = a->env;
+    fp.gfb_cn_f64 = a->gfb && a->gfb_dtype == F2_F64 ? 1 : 0;
+    fp.env_cn_f64 = a->env && a->env_dtype == F2_F64 ? 1 : 0;
     fp.dec = a->dec;
     fp.win = a->windows;
     fp.win_off = reinterpret_cast<const long long*>(a->win_offsets);
@@ -908,13 +883,6 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
         F2_CUDA(f2::launch_fused(fp64, (int)n_f64, true, stream));
     }
     if (a->ev_fused_stop) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_stop, stream));
-
-    if (a->gfb && !direct_cn)
-        F2_CUDA(f2::launch_transpose_convert(b->d_utts, b->n_utts, b->max_n, gfb_t, a->gfb, a->gfb_dtype, plan->C,
-                                             stream));
-    if (a->env && !direct_cn)
-        F2_CUDA(f2::launch_transpose_convert(b->d_utts, b->n_utts, b->max_n, env_t, a->env, a->env_dtype, plan->C,
-                                             stream));
     return F2_OK;
 }
 

@@ -54,11 +54,11 @@ namespace f2 {
 
 // ENV: 0 = cascade only, 1 = magnitude, 2 = magnitude + low-pass.
 // OUT: 0 = nothing leaves the kernel (warm-up), 1 = decimated frames only, 2 = full-rate
-//      time-major stores (and decimated frames when asked), 3 = every decimated frame goes
-//      straight into the (up to win_dots) window rows that contain it.
+//      stores: (C, n) when CN, time-major envelope when asked (and decimated frames when
+//      asked), 3 = every decimated frame goes straight into the (up to win_dots) window rows
+//      that contain it.
 struct OutCtx {
-    float* gfb;     // points at sample t of this thread's channel (or null)
-    float* env;
+    float* env;     // time-major envelope: points at sample t of this thread's channel (or null)
     float* dec;     // OUT 1/2: the next decimated frame of this channel (or null).  OUT 3: slot 0 of the
                     // window that STARTS at the next decimated frame
     int next_dec;   // time index of the next decimated frame
@@ -69,15 +69,13 @@ struct OutCtx {
     int nwin;       // OUT 3: windows of this utterance
     // CN: (C, n) outputs in the reference's layout.  Each lane stages its channel's samples in a 32 x (kCnW+1)
     // shared-memory tile; every kCnW samples the warp writes the tile out row by row -- 32 consecutive samples
-    // of one channel per store instruction (128 / 256 contiguous bytes), kCnW per row instead of a time-major scratch
-    // matrix and a transposing second kernel.
+    // of one channel per store instruction (128 / 256 contiguous bytes), kCnW per row.
     float* tr_g;    // shared-memory tiles (or null)
     float* tr_e;
     char* cn_g;     // element (first channel of this CTA, sample 0) of the utterance's (C, n) block (or null)
     char* cn_e;
     int cn_n;       // samples per row
     int cn_rows;    // channels of this CTA that exist (<= 32)
-    int cn_f64;
 };
 
 // (C, n) staging tile: 32 channels x kCnW samples (+1 column of padding).  Longer runs per channel row make
@@ -85,11 +83,11 @@ struct OutCtx {
 constexpr int kCnW = 128;
 constexpr int kCnP = kCnW + 1;
 
-// rows of the staged tile -> global: samples [tb, tb + cnt) of every channel of this CTA
-__device__ __forceinline__ void flush_cn(const float* tr, char* base, const OutCtx& o, int tb, int cnt) {
+// rows of the staged tile -> global: samples [tb, tb + cnt) of every channel of this CTA, as float64 or float32
+__device__ __forceinline__ void flush_cn(const float* tr, char* base, int f64, const OutCtx& o, int tb, int cnt) {
     __syncwarp();
     const int lane = threadIdx.x;
-    if (o.cn_f64) {
+    if (f64) {
         double* row = reinterpret_cast<double*>(base) + tb + lane;
         for (int r = 0; r < o.cn_rows; ++r, row += o.cn_n)
 #pragma unroll
@@ -170,12 +168,9 @@ __device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s,
             const float2 u = make_float2(ZEROX ? 0.f : xv[2 * j], xv[2 * j + 1]);
             const float2 y = (j & 1) ? cascade<FORM>(k, s, u, gv[j], eo) : cascade<FORM>(k, s, u, gv[j], ee);
             if (ENV > 0) ev[j] = envelope<ENV>(p, s, y);
-            if (OUT == 2 && !CN) {
-                if (o.gfb && active) __stcs(o.gfb + (size_t)j * o.C, k.g4 * y.x);
-                if (ENV > 0 && o.env && active) {
-                    const float v = ENV == 2 ? ev[j] + (j > 0 ? ev[j > 0 ? j - 1 : 0] : wprev) : ev[j];
-                    __stcs(o.env + (size_t)j * o.C, o.env_scale * v);
-                }
+            if (OUT == 2 && ENV > 0 && o.env && active) {
+                const float v = ENV == 2 ? ev[j] + (j > 0 ? ev[j > 0 ? j - 1 : 0] : wprev) : ev[j];
+                __stcs(o.env + (size_t)j * o.C, o.env_scale * v);
             }
             if (OUT == 2 && CN) {
                 const int col = (t + i + j) & (kCnW - 1);
@@ -187,13 +182,10 @@ __device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s,
             }
         }
         if (ENV == 2) s.wprev = ev[U - 1];
-        if (OUT == 2 && !CN) {
-            if (o.gfb) o.gfb += U * o.C;
-            if (o.env) o.env += U * o.C;
-        }
+        if (OUT == 2 && o.env) o.env += U * o.C;
         if (OUT == 2 && CN && ((t + i + U) & (kCnW - 1)) == 0) {
-            if (o.cn_g) flush_cn(o.tr_g, o.cn_g, o, t + i + U - kCnW, kCnW);
-            if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, o, t + i + U - kCnW, kCnW);
+            if (o.cn_g) flush_cn(o.tr_g, o.cn_g, p.gfb_cn_f64, o, t + i + U - kCnW, kCnW);
+            if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, p.env_cn_f64, o, t + i + U - kCnW, kCnW);
         }
         if (OUT > 0 && ENV > 0 && o.dec) {
             while (o.next_dec < t + i + U) {
@@ -224,23 +216,17 @@ __device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s,
         if (ENV > 0) e = envelope<ENV>(p, s, y);
         const float out = ENV == 2 ? e + s.wprev : e;
         if (ENV == 2) s.wprev = e;
-        if (OUT == 2 && !CN) {
-            if (o.gfb) {
-                if (active) __stcs(o.gfb, k.g4 * y.x);
-                o.gfb += o.C;
-            }
-            if (ENV > 0 && o.env) {
-                if (active) __stcs(o.env, o.env_scale * out);
-                o.env += o.C;
-            }
+        if (OUT == 2 && ENV > 0 && o.env) {
+            if (active) __stcs(o.env, o.env_scale * out);
+            o.env += o.C;
         }
         if (OUT == 2 && CN) {
             const int col = (t + i) & (kCnW - 1);
             if (o.cn_g) o.tr_g[threadIdx.x * kCnP + col] = k.g4 * y.x;
             if (ENV > 0 && o.cn_e) o.tr_e[threadIdx.x * kCnP + col] = o.env_scale * out;
             if (col == kCnW - 1) {
-                if (o.cn_g) flush_cn(o.tr_g, o.cn_g, o, t + i - (kCnW - 1), kCnW);
-                if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, o, t + i - (kCnW - 1), kCnW);
+                if (o.cn_g) flush_cn(o.tr_g, o.cn_g, p.gfb_cn_f64, o, t + i - (kCnW - 1), kCnW);
+                if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, p.env_cn_f64, o, t + i - (kCnW - 1), kCnW);
             }
         }
         if (OUT > 0 && ENV > 0 && o.dec && o.next_dec == t + i) {
@@ -255,8 +241,8 @@ __device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s,
     }
     if (OUT == 2 && CN && ((t + cnt) & (kCnW - 1)) != 0) {   // the utterance ends inside a block of kCnW
         const int rest = (t + cnt) & (kCnW - 1);
-        if (o.cn_g) flush_cn(o.tr_g, o.cn_g, o, t + cnt - rest, rest);
-        if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, o, t + cnt - rest, rest);
+        if (o.cn_g) flush_cn(o.tr_g, o.cn_g, p.gfb_cn_f64, o, t + cnt - rest, rest);
+        if (ENV > 0 && o.cn_e) flush_cn(o.tr_e, o.cn_e, p.env_cn_f64, o, t + cnt - rest, rest);
     }
 }
 
@@ -297,7 +283,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
     const bool need_env = WIN || p.env_t != nullptr || p.dec != nullptr || (CN && p.env_cn != nullptr);
     const bool need_imag = need_env && N2 > 2;  // N2 <= 2: the analytic signal is real
     // WIN: the window-store instantiation (f2_run_args.windows; no full-rate outputs by contract)
-    const bool full_out = !WIN && (CN || p.gfb_t != nullptr || p.env_t != nullptr);
+    const bool full_out = !WIN && (CN || p.env_t != nullptr);
     const int nE = (need_imag && !EDGE) ? (n - tE0 + kTile - 1) / kTile : 0;
     const int w_lpf = (p.lpf && need_env) ? p.w_lpf : 0;
     int ts, tenv;
@@ -340,22 +326,19 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
     o.C = (size_t)p.C;
     o.step = p.step;
     o.env_scale = p.lpf ? k.g4 * p.lp_b0 : k.g4;
-    o.gfb = p.gfb_t ? p.gfb_t + (size_t)(ut.full_off + t0) * o.C + (active ? c : 0) : nullptr;
     o.env = p.env_t ? p.env_t + (size_t)(ut.full_off + t0) * o.C + (active ? c : 0) : nullptr;
     o.tr_g = o.tr_e = nullptr;
     o.cn_g = o.cn_e = nullptr;
     o.cn_n = n;
-    o.cn_f64 = p.cn_f64;
     o.cn_rows = 0;
     if (CN) {
         const int c0 = item.cblock * kChanPerBlock;
         o.cn_rows = min(kChanPerBlock, p.C - c0);
-        const size_t esize = p.cn_f64 ? 8 : 4;
-        const size_t block = ((size_t)ut.full_off * o.C + (size_t)c0 * (size_t)n) * esize;   // (C, n_u) blocks back to back
+        const size_t elems = (size_t)ut.full_off * o.C + (size_t)c0 * (size_t)n;   // (C, n_u) blocks back to back
         o.tr_g = sm.tr;
         o.tr_e = p.gfb_cn ? sm.tr + 32 * kCnP : sm.tr;   // envelope alone: the only tile
-        o.cn_g = p.gfb_cn ? reinterpret_cast<char*>(p.gfb_cn) + block : nullptr;
-        o.cn_e = p.env_cn ? reinterpret_cast<char*>(p.env_cn) + block : nullptr;
+        o.cn_g = p.gfb_cn ? reinterpret_cast<char*>(p.gfb_cn) + elems * (p.gfb_cn_f64 ? 8 : 4) : nullptr;
+        o.cn_e = p.env_cn ? reinterpret_cast<char*>(p.env_cn) + elems * (p.env_cn_f64 ? 8 : 4) : nullptr;
     }
     {
         // first decimated frame at or after t0: t = phase + j*step

@@ -10,11 +10,10 @@ struct FusedParams {
     const float* chan;   // [kNumChanPar][c_pad] per-channel parameter block
     const float2* xz;    // rings: (x[t], Im hilbert(x_padded)[t])
     const float* G;      // rings: circular Hilbert kernel aligned to each utterance's edge
-    float* gfb_t;        // full-rate filterbank output, time-major [t][C]   (nullable)
     float* env_t;        // full-rate envelope, time-major [t][C]            (nullable)
     void* gfb_cn;        // full-rate filterbank output in the REFERENCE layout: (C, n_u) blocks back to back,
-    void* env_cn;        //   float64 or float32 -- stored by the kernel through a shared-memory transpose (nullable)
-    int cn_f64;          // element type of gfb_cn / env_cn: 1 = float64, 0 = float32
+    void* env_cn;        //   float64 or float32 (gfb_cn_f64, env_cn_f64) -- stored by the kernel through a
+                         //   shared-memory transpose (nullable)
     float* dec;          // decimated envelope frames [frame][C]             (nullable)
     float* win;          // windows of win_dots consecutive frames [row][win_dots][C]   (nullable)
     const long long* win_off;  // [n_utts+1] first window row of each utterance
@@ -34,6 +33,8 @@ struct FusedParams {
     float direct_min_cy; // groups of 32 channels with min(1+B1+B2) >= this run the direct-form sections
     const double* chan64;  // [kNumChanPar64][c_pad] float64 block of the FORM 2 groups (FORM 2 launch only)
     const double* edge64;  // float64 edge residuals [utt][C][8] of the FORM 2 groups (f2_edge.cu; null: in-kernel)
+    int gfb_cn_f64;      // element type of gfb_cn: 1 = float64, 0 = float32
+    int env_cn_f64;      // element type of env_cn: 1 = float64, 0 = float32
 };
 
 // float64: p.items are work items of FORM 2 groups (float64 sections), run by their own instantiations.

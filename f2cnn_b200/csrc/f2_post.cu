@@ -1,8 +1,5 @@
 // f2_post.cu -- layout / windowing kernels either side of the fused kernel (all HBM-bound).
 //
-//   transpose_convert   time-major float [t][C]  ->  the reference's (C,n) float64/float32
-//                       matrices (.GFB.npy / .ENV1.npy layout, gammatone/filters.py:217,
-//                       scripts/processing/EnvelopeExtraction.py:53)
 //   gather_rows         window gather of InputGenerator.py:73-80 from decimated frames
 //   dense_frames        dense stride-1 framing of Evaluating.py:70-78 (+ normalizeInput,
 //                       scripts/CNN/Training.py:13-28)
@@ -12,49 +9,6 @@
 #include "f2_post.cuh"
 
 namespace f2 {
-
-// ------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void transpose_convert_kernel(const UttDesc* utts, const float* __restrict__ src, T* __restrict__ dst,
-                                         int C) {
-    __shared__ float tile[32][33];
-    const UttDesc ut = utts[blockIdx.x];
-    const int n = ut.n;
-    const float* s = src + (size_t)ut.full_off * C;
-    T* d = dst + (size_t)ut.full_off * C;  // (C,n) block of this utterance starts at C*full_off
-    const int tx = threadIdx.x, ty = threadIdx.y;  // 32 x 8
-    for (int tt = blockIdx.y * 32; tt < n; tt += gridDim.y * 32) {
-        for (int c0 = 0; c0 < C; c0 += 32) {
-#pragma unroll
-            for (int r = 0; r < 32; r += 8) {
-                const int t = tt + ty + r, c = c0 + tx;
-                tile[ty + r][tx] = (t < n && c < C) ? s[(size_t)t * C + c] : 0.f;
-            }
-            __syncthreads();
-#pragma unroll
-            for (int r = 0; r < 32; r += 8) {
-                const int c = c0 + ty + r, t = tt + tx;
-                if (t < n && c < C) d[(size_t)c * n + t] = (T)tile[tx][ty + r];
-            }
-            __syncthreads();
-        }
-    }
-}
-
-cudaError_t launch_transpose_convert(const UttDesc* utts, int n_utts, int max_n, const float* src, void* dst,
-                                     int dst_dtype, int C, cudaStream_t stream) {
-    if (n_utts <= 0 || max_n <= 0) return cudaSuccess;
-    int by = (max_n + 31) / 32;
-    if (by > 4096) by = 4096;
-    dim3 grid(n_utts, by), block(32, 8);
-    if (dst_dtype == F2_DT_F64)
-        transpose_convert_kernel<double><<<grid, block, 0, stream>>>(utts, src, (double*)dst, C);
-    else if (dst_dtype == F2_DT_F32)
-        transpose_convert_kernel<float><<<grid, block, 0, stream>>>(utts, src, (float*)dst, C);
-    else
-        return cudaErrorInvalidValue;
-    return cudaGetLastError();
-}
 
 // ------------------------------------------------------------------------------------------
 // out[(row*dots + j)*C + c] = src[(base[row] + j*stride)*C + c]

@@ -5,8 +5,6 @@
 
 namespace f2 {
 
-cudaError_t launch_transpose_convert(const UttDesc* utts, int n_utts, int max_n, const float* src, void* dst,
-                                     int dst_dtype, int C, cudaStream_t stream);
 cudaError_t launch_gather_rows(const float* src, const long long* base, long long n_rows, int dots,
                                long long stride, int C, float* out, cudaStream_t stream);
 cudaError_t launch_gather_index(const float* src, const long long* idx, long long n_idx, int C, float* out,

@@ -187,8 +187,8 @@ class Batch:
         except Exception:
             pass
 
-    def workspace_bytes(self, want_full_gfb=False, want_full_env=False):
-        return int(_native.lib().f2_batch_workspace_bytes(self._h, int(want_full_gfb), int(want_full_env)))
+    def workspace_bytes(self):
+        return int(_native.lib().f2_batch_workspace_bytes(self._h, 0, 0))
 
     def grid_windows(self, dots=11):
         """The label grid of LabelDataGenerator.py:38-50 on this batch's decimated frames: utterance
@@ -274,8 +274,7 @@ class Batch:
             a.windows, a.win_offsets, a.win_dots = w.data_ptr(), offs.data_ptr(), dots
         if fused_events is not None:  # (DeviceEvent, DeviceEvent) around the fused kernel
             a.ev_fused_start, a.ev_fused_stop = fused_events[0].handle, fused_events[1].handle
-        need = self.workspace_bytes(g is not None, e is not None and "env_t" not in res)
-        ws = plan.workspace(need, stream)
+        ws = plan.workspace(self.workspace_bytes(), stream)
         check(_native.lib().f2_batch_run(self._h, ctypes.byref(a), _ptr(ws), ws.numel(), _stream_ptr(stream)))
         return res
 

@@ -106,6 +106,8 @@ F2_API int64_t f2_batch_total_frames(const f2_batch* batch);
 F2_API int64_t f2_batch_num_items(const f2_batch* batch);
 /* frame_offsets: HOST array of n_utts+1: first decimated frame of each utterance. */
 F2_API int f2_batch_frame_offsets(const f2_batch* batch, int64_t* frame_offsets);
+/* Device workspace f2_batch_run needs for this batch, whatever outputs it is asked for: want_full_gfb and
+ * want_full_env are ignored (the fused kernel stores every full-rate output itself). */
 F2_API size_t f2_batch_workspace_bytes(const f2_batch* batch, int want_full_gfb, int want_full_env);
 
 typedef struct f2_run_args {

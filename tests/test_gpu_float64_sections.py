@@ -113,7 +113,7 @@ def test_refused_fuzz_banks_meet_the_bar(gpu, orc):
 
 def test_output_modes_of_a_refused_bank(gpu, orc, monkeypatch):
     """One refused 128-channel bank through every output mode: window store == decimated frames + gather bit for
-    bit; the (C, n) direct store == the transposed time-major output; gammatonegram; time chunks within the
+    bit; the (C, n) store == the transposed time-major output; gammatonegram; time chunks within the
     bound of test_time_chunking_is_transparent; batch == single runs bit for bit; two runs identical."""
     api, engine, filters, synth, torch = gpu
     co = refused_128(filters)
@@ -132,7 +132,7 @@ def test_output_modes_of_a_refused_bank(gpu, orc, monkeypatch):
     base = np.concatenate([batch.frame_offsets[u] + np.arange(nb[u]) for u in range(len(lens))]).astype(np.int64)
     assert not torch.isnan(win).any()
     assert torch.equal(win, engine.gather_windows(dec, torch.from_numpy(base).cuda(), dots, 1))
-    # (C, n) direct store vs time-major envelope + transpose
+    # (C, n) envelope alone, and next to the time-major envelope: the same bits, and env_t.T
     direct = batch.run(flat, lpf=True, cutoff=50, env=torch.float32)["env"]
     both = batch.run(flat, lpf=True, cutoff=50, env=torch.float32, env_t=True)
     assert torch.equal(direct, both["env"])

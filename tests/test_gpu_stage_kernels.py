@@ -2,7 +2,7 @@
 scipy) computation on the same float32 values -- not end to end, where the fused kernel's 1e-4 x RMS error
 budget would hide a defect of theirs.
 
-  (a) transpose_convert, the direct (C, n) store   bit for bit against env_t.T / its float64 widening
+  (a) the (C, n) store, each output in its dtype  bit for bit against env_t.T / its float64 widening
   (b) gather_rows (vector and scalar), gather_index,
       gather_cn                                    bit for bit against numpy indexing / numpy.astype(float32)
   (c) dense_frames                                 raw: bit for bit; normalised: NORM_TOL absolute against
@@ -25,7 +25,7 @@ Bounds, from the float32 (float64) operations involved; RMS is that of the float
 
 OBSERVED on one B200 (1000 W power limit), profiles/r03c_stage_kernels.log: normalised frames within 3.0e-8
 (the float32 output's rounding); rows within 0.15 (LOWPASS), 0.13 (HILBERT, ENVELOPE), 0.19 (ENVELOPE + LPF)
-of their bounds; label_fit p within 1.3e-3 of its bound; the direct (C, n) store bit-identical to the transposed."""
+of their bounds; label_fit p within 1.3e-3 of its bound; the (C, n) store bit-identical to env_t.T."""
 import math
 from fractions import Fraction
 
@@ -66,10 +66,9 @@ def _bits(t):
 # ---- (a) reference layouts ---------------------------------------------------------------------------------
 @pytest.mark.parametrize("C", [1, 31, 33, 128, 200])
 def test_reference_layouts_transposed_and_direct(gpu, C):
-    """(C, n) outputs next to env_t take transpose_convert: env must be env_t.T bit for bit in both dtypes, the
-    float64 filterbank the widening of the float32 one.  131 073 samples make grid.y = 4097 > 4096, so the
-    kernel loops.  Without env_t the fused kernel stores (C, n) itself (direct_cn): the same bits, since both
-    paths split the utterances into the same chunks."""
+    """The fused kernel stores (C, n) outputs itself, next to env_t or not: env must be env_t.T bit for bit in
+    both dtypes, the float64 filterbank the widening of the float32 one, and the runs without env_t the same bits
+    as those with it.  gfb and env in different dtypes each hold what the same-dtype runs hold."""
     torch, api, engine, synth, _ = gpu
     lens = [1, 31, 33, 131072, 131073, 4000, 2]
     waves = [synth.white_noise_i16(n, seed=70 + i) for i, n in enumerate(lens)]
@@ -78,6 +77,8 @@ def test_reference_layouts_transposed_and_direct(gpu, C):
     off = batch.sample_offsets
     t = {dt: batch.run(flat, lpf=True, cutoff=50, gfb=dt, env=dt, env_t=True) for dt in (torch.float32, torch.float64)}
     d = {dt: batch.run(flat, lpf=True, cutoff=50, gfb=dt, env=dt) for dt in (torch.float32, torch.float64)}
+    mixed = [(gd, ed, batch.run(flat, lpf=True, cutoff=50, gfb=gd, env=ed, env_t=with_t))
+             for gd, ed in ((torch.float64, torch.float32), (torch.float32, torch.float64)) for with_t in (False, True)]
     env_t = t[torch.float32]["env_t"]
     assert torch.equal(env_t, t[torch.float64]["env_t"])
     for u, n in enumerate(lens):
@@ -89,6 +90,12 @@ def test_reference_layouts_transposed_and_direct(gpu, C):
         for key in ("gfb", "env"):
             assert torch.equal(d[torch.float64][key][blk], d[torch.float32][key][blk].double()), (C, n, key)
             assert torch.equal(d[torch.float32][key][blk], t[torch.float32][key][blk]), (C, n, key)
+        for gd, ed, m in mixed:
+            assert torch.equal(m["gfb"][blk], d[gd]["gfb"][blk]), (C, n, gd, ed)
+            assert torch.equal(m["env"][blk], d[ed]["env"][blk]), (C, n, gd, ed)
+    for gd, ed, m in mixed:
+        if "env_t" in m:
+            assert torch.equal(m["env_t"], env_t), (C, gd, ed)
 
 
 # ---- (b) gathers -------------------------------------------------------------------------------------------

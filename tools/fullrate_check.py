@@ -1,5 +1,6 @@
-"""Full-rate (C, n) output modes: parity against the oracle on ragged shapes and the HBM roofline figure
-of SURVEY.md 8d (16.04 / 8.04 bytes per channel-sample) on 256 corpus utterances."""
+"""Full-rate output modes -- (C, n) in either dtype, alone, mixed or next to the time-major envelope: parity
+against the oracle and the HBM roofline figure of SURVEY.md 8d (16.04 / 12.04 / 8.04 bytes per channel-sample)
+on 256 corpus utterances."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -16,7 +17,9 @@ bq = plan.batch(lengths)
 cs = 128.0 * float(lengths.sum())
 for tag, kw, bpc in (("gfb+env f64 (reference layout)", dict(gfb=torch.float64, env=torch.float64), 16.04),
                      ("gfb+env f32", dict(gfb=torch.float32, env=torch.float32), 8.04),
-                     ("env f64 only", dict(env=torch.float64), 8.02), ("gfb f64 only", dict(gfb=torch.float64), 8.02)):
+                     ("env f64 only", dict(env=torch.float64), 8.02), ("gfb f64 only", dict(gfb=torch.float64), 8.02),
+                     ("env f64 + env_t f32", dict(env=torch.float64, env_t=True), 12.04),
+                     ("gfb f64 + env f32", dict(gfb=torch.float64, env=torch.float32), 12.04)):
     res = bq.run(fd, lpf=True, cutoff=50, **kw)
     torch.cuda.synchronize()
     a, z = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
