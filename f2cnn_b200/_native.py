@@ -84,7 +84,10 @@ SIGNATURES = {
     "f2_batch_workspace_bytes": (ctypes.c_size_t, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int]),
     "f2_batch_run": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(RunArgs), ctypes.c_void_p, ctypes.c_size_t,
                                     ctypes.c_void_p]),
-    "f2_envelope_rows_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64]),
+    "f2_batch_run_cutoffs": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                                            ctypes.POINTER(ctypes.c_double), ctypes.c_int, ctypes.c_void_p,
+                                            ctypes.c_int64, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
+    "f2_envelope_rows_workspace_bytes":(ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64]),
     "f2_envelope_rows": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
                                         ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_int,
                                         ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),

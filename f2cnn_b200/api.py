@@ -287,12 +287,14 @@ _pipelines_lock = threading.Lock()
 _MAX_PIPELINES = 2
 
 
-def _pipeline_for(plan, lengths, dots, step, phase, LPF, CUTOFF, src_offsets=None, share=1):
+def _pipeline_for(plan, lengths, dots, step, phase, LPF, CUTOFF, src_offsets=None, share=1, cutoffs=None):
     """The sub-batch layout, device buffers, pinned staging and worker pool of a corpus-sized request
     depend only on the utterance lengths and the grid: built once, reused by every later call with the
-    same corpus (a second `prepare input --cutoff K` run, the next epoch's noise draw, a benchmark)."""
+    same corpus (a second `prepare input --cutoff K` run, the next epoch's noise draw, a benchmark).
+    cutoffs: the settings of a cutoff sweep (their number is part of the layout)."""
     key = (id(plan), hashlib.sha1(lengths.tobytes()).hexdigest(), int(dots), int(step), int(phase), int(share),
-           None if src_offsets is None else hashlib.sha1(np.ascontiguousarray(src_offsets).tobytes()).hexdigest())
+           None if src_offsets is None else hashlib.sha1(np.ascontiguousarray(src_offsets).tobytes()).hexdigest(),
+           None if cutoffs is None else len(cutoffs))
     with _pipelines_lock:
         pipe = _pipelines.get(key)
         if pipe is None:
@@ -300,13 +302,15 @@ def _pipeline_for(plan, lengths, dots, step, phase, LPF, CUTOFF, src_offsets=Non
             # (one core stays free for the CUDA host-callback thread that hands frames to the pool)
             threads = max(1, engine.host_cores() // max(int(share), 1) - (1 if int(share) == 1 else 0))
             pipe = engine.WindowPipeline(plan, lengths, dots=dots, step=step, phase=phase, lpf=LPF, cutoff=CUTOFF,
-                                         src_offsets=src_offsets, placer=engine.Placer(threads))
+                                         src_offsets=src_offsets, placer=engine.Placer(threads), cutoffs=cutoffs)
             _pipelines[key] = pipe
             while len(_pipelines) > _MAX_PIPELINES:
                 _pipelines.popitem(last=False)
         else:
             _pipelines.move_to_end(key)
         pipe.lpf, pipe.cutoff = bool(LPF), CUTOFF
+        if cutoffs is not None:
+            pipe.cutoffs = tuple(cutoffs)
         return pipe
 
 
@@ -318,26 +322,9 @@ def release_cached_pipelines():
     engine.release_host_pool()
 
 
-def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=5, step=160, device_out=False,
-                        out=None, counts=None, shard=None):
-    """Fused path from waveforms to the (N, 2R+1, C) float32 input tensor.
-
-    waves: list of 1-D arrays (same dtype), or (flat, lengths) as returned by ingest.read_corpus
-    (one buffer of all samples, pinned for full speed); timepoints: list of int arrays (window
-    centres per utterance, in output order) -- or, with `counts`, ONE flat int array of all centres
-    and counts[u] of them per utterance.  Equivalent to
-    erb_filterbank -> ExtractEnvelopeFromMatrix(LPF, CUTOFF) -> the gather of
-    InputGenerator.py:73-80 per utterance, rows concatenated in list order.  `out`: an existing
-    C-contiguous (N, 2R+1, C) float32 numpy array to fill (a corpus-sized result is 7.5 GB: reusing
-    it saves its page faults); by default a fresh array is returned.
-    shard=(rank, world): one of `world` processes (one per GPU, e.g. under torchrun) that were all
-    handed the SAME corpus and the SAME `out` -- a shared mapping, hostmem.SharedArray.  This call
-    computes the utterances engine.shard_utterances deals to `rank` and writes their rows, and only
-    theirs, at their final offsets; there is nothing to exchange afterwards."""
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    C = plan.n_channels
-    dots = 2 * radius + 1
+def _corpus(waves, timepoints, counts):
+    """The (waves, timepoints, counts) arguments of features_to_windows -> (flat host tensor or None, list of
+    waves or None, lengths, flat centres, counts)."""
     flat_in = None
     if isinstance(waves, tuple) and len(waves) == 2:
         flat_in, lengths = waves
@@ -365,6 +352,56 @@ def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=
         counts = np.fromiter((len(t) for t in timepoints), dtype=np.int64, count=n_utts)
         centers = (np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in timepoints])
                    if n_utts else np.zeros(0, dtype=np.int64))
+    return flat_in, waves, lengths, centers, counts
+
+
+def _wave_to_device(flat_in, waves, device):
+    if flat_in is None:
+        flat_in = torch.from_numpy(np.concatenate(waves) if len(waves) > 1 else waves[0])
+    return (flat_in if flat_in.is_pinned() or flat_in.numel() * flat_in.element_size() < (1 << 16)
+            else flat_in.pin_memory()).to(device, non_blocking=True)
+
+
+def _gather_on_grid(dec, idx, phase, step, frame_offsets, dots):
+    """Windows (total, dots, C) from the decimated frames `dec` ([frames, C] on the device) of a batch whose
+    grid holds every index of `idx` (per utterance, from window_indices)."""
+    bases, strided = [], True
+    for u, i in enumerate(idx):
+        if not i.size:
+            continue
+        rows = (i - phase) // step + frame_offsets[u]
+        strided = strided and bool(np.all(np.diff(rows, axis=1) == 1))
+        bases.append(rows)
+    rows = np.concatenate(bases)
+    if strided:
+        base_dev = _to_device(np.ascontiguousarray(rows[:, 0]), dec.device)
+        return engine.gather_windows(dec, base_dev, dots, 1)
+    res_w = engine.gather_index(dec, _to_device(np.ascontiguousarray(rows.reshape(-1)), dec.device))
+    return res_w.view(rows.shape[0], dots, dec.shape[1])
+
+
+def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=5, step=160, device_out=False,
+                        out=None, counts=None, shard=None):
+    """Fused path from waveforms to the (N, 2R+1, C) float32 input tensor.
+
+    waves: list of 1-D arrays (same dtype), or (flat, lengths) as returned by ingest.read_corpus
+    (one buffer of all samples, pinned for full speed); timepoints: list of int arrays (window
+    centres per utterance, in output order) -- or, with `counts`, ONE flat int array of all centres
+    and counts[u] of them per utterance.  Equivalent to
+    erb_filterbank -> ExtractEnvelopeFromMatrix(LPF, CUTOFF) -> the gather of
+    InputGenerator.py:73-80 per utterance, rows concatenated in list order.  `out`: an existing
+    C-contiguous (N, 2R+1, C) float32 numpy array to fill (a corpus-sized result is 7.5 GB: reusing
+    it saves its page faults); by default a fresh array is returned.
+    shard=(rank, world): one of `world` processes (one per GPU, e.g. under torchrun) that were all
+    handed the SAME corpus and the SAME `out` -- a shared mapping, hostmem.SharedArray.  This call
+    computes the utterances engine.shard_utterances deals to `rank` and writes their rows, and only
+    theirs, at their final offsets; there is nothing to exchange afterwards."""
+    coefs = np.asarray(coefs, dtype=np.float64)
+    plan = engine.plan_for(coefs)
+    C = plan.n_channels
+    dots = 2 * radius + 1
+    flat_in, waves, lengths, centers, counts = _corpus(waves, timepoints, counts)
+    n_utts = int(lengths.shape[0])
     total = int(counts.sum())
     if out is not None:
         if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"] and
@@ -433,27 +470,11 @@ def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=
     allidx = np.concatenate([i.reshape(-1) for i in idx if i.size])
     phase = int(allidx[0] % step)
     on_grid = bool(np.all(allidx % step == phase))
-    if flat_in is None:
-        flat_in = torch.from_numpy(np.concatenate(waves) if len(waves) > 1 else waves[0])
-    wave_dev = (flat_in if flat_in.is_pinned() or flat_in.numel() * flat_in.element_size() < (1 << 16)
-                else flat_in.pin_memory()).to(plan.device, non_blocking=True)
+    wave_dev = _wave_to_device(flat_in, waves, plan.device)
     if on_grid:
         batch = plan.batch(lengths, step=step, phase=phase)
         res = batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, dec=True)
-        bases, strided = [], True
-        for u, i in enumerate(idx):
-            if not i.size:
-                continue
-            rows = (i - phase) // step + batch.frame_offsets[u]
-            strided = strided and bool(np.all(np.diff(rows, axis=1) == 1))
-            bases.append(rows)
-        rows = np.concatenate(bases)
-        if strided:
-            base_dev = _to_device(np.ascontiguousarray(rows[:, 0]), plan.device)
-            res_w = engine.gather_windows(res["dec"], base_dev, dots, 1)
-        else:
-            res_w = engine.gather_index(res["dec"], _to_device(np.ascontiguousarray(rows.reshape(-1)), plan.device))
-            res_w = res_w.view(total, dots, C)
+        res_w = _gather_on_grid(res["dec"], idx, phase, step, batch.frame_offsets, dots)
     else:
         batch = plan.batch(lengths, step=step, phase=0)
         res = batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, env_t=True)
@@ -467,6 +488,76 @@ def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=
         out[...] = host
         return out
     return host
+
+
+def features_to_windows_sweep(waves, coefs, timepoints, cutoffs, radius=5, step=160, counts=None, out=None):
+    """features_to_windows for several envelope settings at once: a list of K (N, 2R+1, C) float32 arrays, the
+    k-th equal to features_to_windows(..., LPF=cutoffs[k] is not None, CUTOFF=cutoffs[k]).  cutoffs: 1..4
+    entries, each a cutoff in (0, 8000) Hz or None for no low-pass.  The filterbank and the Hilbert transform
+    run once for all settings (engine.Batch.run_cutoffs).  waves, timepoints, counts and `out` (here a list of
+    K arrays) mean what they mean in features_to_windows.
+
+    Every window index must lie on one decimated grid (all indices equal mod `step`), as those of
+    LabelDataGenerator's CSV do; anything else raises ValueError (call features_to_windows per cutoff).
+    Corpus-sized requests go through engine.WindowPipeline (bit for bit what features_to_windows gives per
+    cutoff); smaller ones take one batch, whose time-chunked utterances all warm up for the lowest cutoff."""
+    settings = list(cutoffs)
+    engine.cutoff_settings(settings)
+    coefs = np.asarray(coefs, dtype=np.float64)
+    plan = engine.plan_for(coefs)
+    C = plan.n_channels
+    dots = 2 * radius + 1
+    flat_in, waves, lengths, centers, counts = _corpus(waves, timepoints, counts)
+    n_utts = int(lengths.shape[0])
+    total = int(counts.sum())
+    if out is not None:
+        out = list(out)
+        if len(out) != len(settings) or not all(
+                isinstance(o, np.ndarray) and o.dtype == np.float32 and o.flags["C_CONTIGUOUS"] and
+                o.shape == (total, dots, C) for o in out):
+            raise ValueError("out must be %d C-contiguous float32 arrays of shape %s" % (len(settings), (total, dots, C)))
+    if total == 0:
+        return [np.zeros((0, dots, C), dtype=np.float32) for _ in settings] if out is None else out
+
+    if total * dots * C * 4 >= _PIPELINE_BYTES and n_utts >= 8:
+        first = int(centers[0]) - radius * step
+        phase = first % step if first >= 0 else 0
+        head = int(min(8, n_utts))
+        n_dec_h = np.where(lengths[:head] > phase, (lengths[:head] - phase + step - 1) // step, 0)
+        probe, phase_h, _ = engine.window_runs(centers[:int(counts[:head].sum())], counts[:head], lengths[:head],
+                                               np.concatenate([[0], np.cumsum(n_dec_h)]), radius, step, phase)
+        if probe is not None and phase_h == phase:
+            pipe = _pipeline_for(plan, lengths, dots, step, phase, False, 100, cutoffs=settings)
+            results = [engine.host_empty((total, dots, C), np.float32) for _ in settings] if out is None else out
+            state = {}
+
+            def detect():
+                runs, phase2, _ = engine.window_runs(centers, counts, lengths, pipe.frame_offsets, radius, step, phase)
+                state["ok"] = runs is not None and phase2 == phase
+                return runs if state["ok"] else np.zeros((0, 3), dtype=np.int64)
+
+            pipe.run(flat_in if flat_in is not None else waves, detect, results)
+            if state["ok"]:
+                return results
+            del results
+
+    # one batch, windows gathered on the device from each plane
+    cpos = np.concatenate([[0], np.cumsum(counts)])
+    idx = [window_indices(int(n), centers[cpos[u]:cpos[u + 1]], radius, step) for u, n in enumerate(lengths)]
+    allidx = np.concatenate([i.reshape(-1) for i in idx if i.size])
+    phase = int(allidx[0] % step)
+    if not bool(np.all(allidx % step == phase)):
+        raise ValueError("features_to_windows_sweep needs every window index on one decimated grid (all equal mod "
+                         "step = %d); call features_to_windows once per cutoff for these timepoints" % step)
+    batch = plan.batch(lengths, step=step, phase=phase)
+    planes = batch.run_cutoffs(_wave_to_device(flat_in, waves, plan.device), settings)
+    results = [_to_host(_gather_on_grid(planes[j], idx, phase, step, batch.frame_offsets, dots))
+               for j in range(len(settings))]
+    if out is None:
+        return results
+    for o, r in zip(out, results):
+        o[...] = r
+    return out
 
 
 class FrameWindows:

@@ -761,6 +761,101 @@ size_t f2_batch_workspace_bytes(const f2_batch* b, int, int) {
     return (size_t)ws_ring_units(b) * ws_ring_bytes(b->total_ring) + ws_edge_bytes(b) + ws_edge64_bytes(b) + 256;
 }
 
+}  // extern "C"
+
+namespace {
+// The launch sequence f2_batch_run and f2_batch_run_cutoffs share: the Hilbert pre-pass, the edge residuals of a
+// time-chunked batch and the fused kernel (float32 groups, then FORM 2 groups).  The caller has checked its
+// arguments and the workspace, and filled fp's outputs and envelope settings; the rest of fp is filled here.
+int run_sequence(f2_batch* b, const void* wave, int wave_dtype, bool need_env, bool gfb, f2::FusedParams fp,
+                 void* workspace, void* ev_start, void* ev_stop, void* stream_) {
+    f2_plan* plan = b->plan;
+    DeviceGuard guard(plan->device);
+    if (!guard.ok) return fail(F2_ERR_CUDA, "cannot select device %d", plan->device);
+    cudaStream_t stream = (cudaStream_t)stream_;
+
+    char* ws = (char*)align_up((size_t)workspace, 256);
+    const size_t rb = ws_ring_bytes(b->total_ring);
+    const int units = ws_ring_units(b);   // 2: no FFT scratch, no private injection tables (see ws_ring_units)
+    float* Z = units == 4 ? (float*)ws : nullptr;
+    float2* xz = (float2*)(units == 4 ? ws + rb : ws);
+    float* G = units == 4 ? (float*)(ws + 3 * rb) : nullptr;
+    float* edge = (float*)(ws + (size_t)units * rb);
+    double* edge64 = (double*)(ws + (size_t)units * rb + ws_edge_bytes(b));
+
+    f2::PrepParams pp;
+    pp.utts = b->d_utts;
+    pp.wave = wave;
+    pp.wave_dtype = wave_dtype;
+    pp.bufA = G;   // the table ends up where the forward transform's first scratch was
+    pp.bufB = Z;
+    pp.xz = xz;
+    pp.G = G;
+    pp.hilbert = need_env ? 1 : 0;
+    f2::HostPrepInfo hp;
+    hp.n_utts = b->n_utts;
+    hp.min_log2N2 = b->min_log2;
+    hp.max_log2N2 = b->max_log2;
+    hp.private_g = b->private_g;
+    F2_CUDA(f2::launch_prep(pp, hp, stream));
+
+    fp.utts = b->d_utts;
+    // the filterbank output is store-bound and uses the direct form for fewer groups: equal-length chunks
+    const bool uniform_chunks = gfb && b->d_items_uniform != nullptr;
+    fp.items = uniform_chunks ? b->d_items_uniform : b->d_items;
+    fp.chan = plan->d_chan;
+    fp.xz = xz;
+    fp.G = G;
+    fp.edge = nullptr;
+    fp.chan64 = plan->d_chan64;
+    fp.edge64 = nullptr;
+    if (need_env && b->n_items > b->n_whole) {
+        // time-chunked batch: the edge residuals are per utterance, compute them once instead of
+        // in every chunk.  Few (utterance, channel) pairs -> chunked scan (low latency), many ->
+        // one sequential thread per channel.
+        const long long scan_ctas = (long long)b->n_utts * ((plan->C + 3) / 4);
+        if (plan->w_edge <= f2::kScanWindow && scan_ctas <= 148 * 16)
+            F2_CUDA(f2::launch_edge_scan(b->d_utts, b->n_utts, plan->d_chan, plan->d_scan_mats, plan->C, plan->c_pad, xz,
+                                         edge, stream));
+        else
+            F2_CUDA(f2::launch_edge<0>(b->d_utts, b->n_utts, plan->d_chan, nullptr, plan->C, plan->c_pad, xz,
+                                       plan->w_edge, edge, stream));
+        fp.edge = edge;
+        if (plan->n_f64)
+            F2_CUDA(f2::launch_edge<2>(b->d_utts, b->n_utts, plan->d_chan, plan->d_chan64, plan->C, plan->c_pad, xz,
+                                       plan->w_edge, edge64, stream));
+    }
+    fp.C = plan->C;
+    fp.c_pad = plan->c_pad;
+    // Direct-form threshold (measured against the float64 oracle, DESIGN.md section 3): round-off of
+    // the direct form grows like 1/(1+B1+B2).  The envelope stays at the delta form's error level
+    // (<= 1e-5 of the channel RMS) down to 0.035; the filterbank output itself only down to 0.25.
+    fp.direct_min_cy = gfb ? kDirectMinCyGfb : kDirectMinCyEnv;
+    fp.step = b->step;
+    fp.phase = b->phase;
+    fp.w_imag = plan->w_imag;
+    fp.w_edge = plan->w_edge;
+    fp.w_casc = plan->w_casc;
+    if (ev_start) F2_CUDA(cudaEventRecord((cudaEvent_t)ev_start, stream));
+    const long long n_items = uniform_chunks ? b->n_items_uniform : b->n_items;
+    const long long n_f64 = uniform_chunks ? b->n_items_uniform_f64 : b->n_items_f64;
+    F2_CUDA(f2::launch_fused(fp, (int)(n_items - n_f64), false, stream));
+    if (n_f64 > 0) {
+        f2::FusedParams fp64 = fp;
+        fp64.items = fp.items + (n_items - n_f64);
+        fp64.edge64 = fp.edge ? edge64 : nullptr;
+        F2_CUDA(f2::launch_fused(fp64, (int)n_f64, true, stream));
+    }
+    if (ev_stop) F2_CUDA(cudaEventRecord((cudaEvent_t)ev_stop, stream));
+    return F2_OK;
+}
+
+// low-pass warm-up of a mid-signal chunk: |a1|^W < 1e-7
+int lowpass_warmup(double a1) { return round_up_tile(log(1e-7) / log(-a1)); }
+}  // namespace
+
+extern "C" {
+
 int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t workspace_bytes, void* stream_) {
     if (!b || !a) return fail(F2_ERR_INVALID, "f2_batch_run: null batch/args");
     if (a->struct_size < sizeof(f2_run_args))
@@ -788,45 +883,9 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
             return fail(F2_ERR_INVALID, "cutoff must be in (0, 8000) Hz, got %g", a->cutoff_hz);
         butter1(a->cutoff_hz, &b0, &a1);
     }
-    f2_plan* plan = b->plan;
-    DeviceGuard guard(plan->device);
-    if (!guard.ok) return fail(F2_ERR_CUDA, "cannot select device %d", plan->device);
-    cudaStream_t stream = (cudaStream_t)stream_;
-
-    char* ws = (char*)align_up((size_t)workspace, 256);
-    const size_t rb = ws_ring_bytes(b->total_ring);
-    const int units = ws_ring_units(b);   // 2: no FFT scratch, no private injection tables (see ws_ring_units)
-    float* Z = units == 4 ? (float*)ws : nullptr;
-    float2* xz = (float2*)(units == 4 ? ws + rb : ws);
-    float* G = units == 4 ? (float*)(ws + 3 * rb) : nullptr;
-    float* edge = (float*)(ws + (size_t)units * rb);
-    double* edge64 = (double*)(ws + (size_t)units * rb + ws_edge_bytes(b));
     const bool need_env = a->env_t != nullptr || a->dec != nullptr || a->windows != nullptr || a->env != nullptr;
 
-    f2::PrepParams pp;
-    pp.utts = b->d_utts;
-    pp.wave = a->wave;
-    pp.wave_dtype = a->wave_dtype;
-    pp.bufA = G;   // the table ends up where the forward transform's first scratch was
-    pp.bufB = Z;
-    pp.xz = xz;
-    pp.G = G;
-    pp.hilbert = need_env ? 1 : 0;
-    f2::HostPrepInfo hp;
-    hp.n_utts = b->n_utts;
-    hp.min_log2N2 = b->min_log2;
-    hp.max_log2N2 = b->max_log2;
-    hp.private_g = b->private_g;
-    F2_CUDA(f2::launch_prep(pp, hp, stream));
-
-    f2::FusedParams fp;
-    fp.utts = b->d_utts;
-    // the filterbank output is store-bound and uses the direct form for fewer groups: equal-length chunks
-    const bool uniform_chunks = a->gfb != nullptr && b->d_items_uniform != nullptr;
-    fp.items = uniform_chunks ? b->d_items_uniform : b->d_items;
-    fp.chan = plan->d_chan;
-    fp.xz = xz;
-    fp.G = G;
+    f2::FusedParams fp{};
     fp.env_t = a->env_t;
     // (C, n) outputs: written by the fused kernel itself through a shared-memory transpose, each in its own dtype
     fp.gfb_cn = a->gfb;
@@ -837,53 +896,55 @@ int f2_batch_run(f2_batch* b, const f2_run_args* a, void* workspace, size_t work
     fp.win = a->windows;
     fp.win_off = reinterpret_cast<const long long*>(a->win_offsets);
     fp.win_dots = a->win_dots;
-    fp.edge = nullptr;
-    fp.chan64 = plan->d_chan64;
-    fp.edge64 = nullptr;
-    if (need_env && b->n_items > b->n_whole) {
-        // time-chunked batch: the edge residuals are per utterance, compute them once instead of
-        // in every chunk.  Few (utterance, channel) pairs -> chunked scan (low latency), many ->
-        // one sequential thread per channel.
-        const long long scan_ctas = (long long)b->n_utts * ((plan->C + 3) / 4);
-        if (plan->w_edge <= f2::kScanWindow && scan_ctas <= 148 * 16)
-            F2_CUDA(f2::launch_edge_scan(b->d_utts, b->n_utts, plan->d_chan, plan->d_scan_mats, plan->C, plan->c_pad, xz,
-                                         edge, stream));
-        else
-            F2_CUDA(f2::launch_edge<0>(b->d_utts, b->n_utts, plan->d_chan, nullptr, plan->C, plan->c_pad, xz,
-                                       plan->w_edge, edge, stream));
-        fp.edge = edge;
-        if (plan->n_f64)
-            F2_CUDA(f2::launch_edge<2>(b->d_utts, b->n_utts, plan->d_chan, plan->d_chan64, plan->C, plan->c_pad, xz,
-                                       plan->w_edge, edge64, stream));
-    }
-    fp.C = plan->C;
-    fp.c_pad = plan->c_pad;
-    // Direct-form threshold (measured against the float64 oracle, DESIGN.md section 3): round-off of
-    // the direct form grows like 1/(1+B1+B2).  The envelope stays at the delta form's error level
-    // (<= 1e-5 of the channel RMS) down to 0.035; the filterbank output itself only down to 0.25.
-    fp.direct_min_cy = a->gfb ? kDirectMinCyGfb : kDirectMinCyEnv;
-    fp.step = b->step;
-    fp.phase = b->phase;
     fp.lpf = a->lpf ? 1 : 0;
     fp.lp_k = (float)(-a1);
     fp.lp_b0 = (float)b0;
-    fp.w_imag = plan->w_imag;
-    fp.w_edge = plan->w_edge;
-    fp.w_casc = plan->w_casc;
-    // low-pass warm-up of a mid-signal chunk: |a1|^W < 1e-7
-    fp.w_lpf = a->lpf ? round_up_tile(log(1e-7) / log(-a1)) : 0;
-    if (a->ev_fused_start) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_start, stream));
-    const long long n_items = uniform_chunks ? b->n_items_uniform : b->n_items;
-    const long long n_f64 = uniform_chunks ? b->n_items_uniform_f64 : b->n_items_f64;
-    F2_CUDA(f2::launch_fused(fp, (int)(n_items - n_f64), false, stream));
-    if (n_f64 > 0) {
-        f2::FusedParams fp64 = fp;
-        fp64.items = fp.items + (n_items - n_f64);
-        fp64.edge64 = fp.edge ? edge64 : nullptr;
-        F2_CUDA(f2::launch_fused(fp64, (int)n_f64, true, stream));
+    fp.w_lpf = a->lpf ? lowpass_warmup(a1) : 0;
+    return run_sequence(b, a->wave, a->wave_dtype, need_env, a->gfb != nullptr, fp, workspace, a->ev_fused_start,
+                        a->ev_fused_stop, stream_);
+}
+
+int f2_batch_run_cutoffs(f2_batch* b, const void* wave, int wave_dtype, const double* cutoffs_hz, int n_settings,
+                         float* dec, int64_t plane_stride, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!b) return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: null batch");
+    if (n_settings < 1 || n_settings > f2::kMaxCutoffs)
+        return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: %d settings (1 .. %d)", n_settings, f2::kMaxCutoffs);
+    if (!cutoffs_hz) return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: null cutoffs");
+    f2::FusedParams fp{};
+    fp.sw_planes = n_settings;
+    double slowest = 0.0;   // a1 of the lowest cutoff: the longest warm-up
+    for (int j = 0; j < n_settings; ++j) {
+        const double f = cutoffs_hz[j];
+        fp.sw_state[j] = -1;
+        if (f == 0.0) continue;   // no low-pass
+        if (!(f > 0.0) || !(f < 8000.0))
+            return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: setting %d: cutoff must be 0 (no low-pass) or in (0, 8000) Hz, "
+                        "got %g", j, f);
+        double b0, a1;
+        butter1(f, &b0, &a1);
+        const int q = fp.sw_lp++;
+        fp.sw_state[j] = q;
+        fp.sw_k[q] = (float)(-a1);
+        fp.sw_b0[q] = (float)b0;
+        if (fp.sw_lp == 1 || -a1 > -slowest) slowest = a1;
     }
-    if (a->ev_fused_stop) F2_CUDA(cudaEventRecord((cudaEvent_t)a->ev_fused_stop, stream));
-    return F2_OK;
+    if (!dec) return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: null dec");
+    const int64_t plane = b->total_frames * (int64_t)b->plan->C;
+    if (plane_stride < plane)
+        return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: plane_stride %lld < total_frames x C = %lld",
+                    (long long)plane_stride, (long long)plane);
+    if (b->total_samples == 0) return F2_OK;
+    if (!wave || wave_dtype < F2_I16 || wave_dtype > F2_F64)
+        return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: wave pointer/dtype");
+    const size_t need = f2_batch_workspace_bytes(b, 0, 0);
+    if (!workspace || workspace_bytes < need)
+        return fail(F2_ERR_WORKSPACE, "workspace %zu bytes, need %zu", workspace_bytes, need);
+    fp.dec = dec;
+    fp.plane_stride = plane_stride;
+    // the chunk warm-up of the lowest cutoff serves every setting
+    fp.lpf = fp.sw_lp > 0 ? 1 : 0;
+    fp.w_lpf = fp.sw_lp > 0 ? lowpass_warmup(slowest) : 0;
+    return run_sequence(b, wave, wave_dtype, true, false, fp, workspace, nullptr, nullptr, stream);
 }
 
 // ---- stand-alone envelope rows ------------------------------------------------------------

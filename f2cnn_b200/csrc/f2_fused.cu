@@ -246,6 +246,102 @@ __device__ __forceinline__ void run_tile(const FusedParams& p, const K& k, S& s,
     }
 }
 
+// ---- cutoff sweep: one cascade, up to kMaxCutoffs envelope settings -------------------------------------
+// Every low-pass setting keeps its own one-pole state w (the operations of envelope<2>); |y| is formed once.
+// A plane's value is captured at the stored sample itself, from w[t] and w[t-1] = the state before this
+// sample's update, so no block of U envelope values per setting is held.  The stored values are the same
+// operations in the same order as run_tile's OUT 1 path: (w[t] + w[t-1]) * (g4 * b0), or g4 * |y|.
+template <int NL>
+__device__ __forceinline__ void store_planes(const FusedParams& p, float g4, OutCtx& o, float mag, const float (&w)[NL],
+                                             const float (&wp)[NL], bool active) {
+    if (active) {
+        float* d = o.dec;
+#pragma unroll
+        for (int j = 0; j < kMaxCutoffs; ++j) {
+            if (j < p.sw_planes) {
+                const int q = p.sw_state[j];
+                float v = mag, scale = g4;
+#pragma unroll
+                for (int r = 0; r < NL; ++r) {
+                    if (q == r) {
+                        v = w[r] + wp[r];
+                        scale = g4 * p.sw_b0[r];
+                    }
+                }
+                __stcs(d, scale * v);
+                d += p.plane_stride;
+            }
+        }
+    }
+    o.dec += o.C;
+    o.next_dec += o.step;
+}
+
+// One sample of the sweep.  CHECK: a decimated frame may fall on it.
+template <int FORM, int NL, bool CHECK, class K, class S, class E>
+__device__ __forceinline__ void sweep_sample(const FusedParams& p, const K& k, S& s, float (&w)[NL], float2 u, float g,
+                                             const E (&e)[4], int t, bool active, OutCtx& o) {
+    const float2 y = cascade<FORM>(k, s, u, g, e);
+    const float mag = fast_sqrt(fmaf(y.x, y.x, y.y * y.y));
+    float wp[NL];
+#pragma unroll
+    for (int r = 0; r < NL; ++r) {
+        wp[r] = w[r];
+        w[r] = fmaf(p.sw_k[r], w[r], mag);
+    }
+    if (CHECK && o.next_dec == t) store_planes<NL>(p, k.g4, o, mag, w, wp, active);
+}
+
+// STORE = false: the low-pass warm-up of a time chunk (run_tile<FORM, 2, 0> for every setting).
+template <int FORM, int NL, bool STORE, int U, class K, class S, class E>
+__device__ __forceinline__ void run_tile_sweep(const FusedParams& p, const K& k, S& s, float (&w)[NL], const E (&ee)[4],
+                                               const E (&eo)[4], const float2* __restrict__ sxz,
+                                               const float* __restrict__ sg, int t, int cnt, bool active, OutCtx& o) {
+    int i = 0;
+    for (; i + U <= cnt; i += U) {
+        float xv[2 * U];
+        float gv[U];
+#pragma unroll
+        for (int j = 0; j < U / 2; ++j) {
+            const float4 v = *reinterpret_cast<const float4*>(sxz + i + 2 * j);
+            xv[4 * j + 0] = v.x;
+            xv[4 * j + 1] = v.y;
+            xv[4 * j + 2] = v.z;
+            xv[4 * j + 3] = v.w;
+        }
+#pragma unroll
+        for (int j = 0; j < U / 4; ++j) {
+            const float4 v = *reinterpret_cast<const float4*>(sg + i + 4 * j);
+            gv[4 * j + 0] = v.x;
+            gv[4 * j + 1] = v.y;
+            gv[4 * j + 2] = v.z;
+            gv[4 * j + 3] = v.w;
+        }
+        // the frame test is uniform in the warp: trips without a frame (most of them at step 160) run
+        // without the per-sample compare
+        if (STORE && o.next_dec < t + i + U) {
+#pragma unroll
+            for (int j = 0; j < U; ++j) {
+                const float2 u = make_float2(xv[2 * j], xv[2 * j + 1]);
+                if (j & 1) sweep_sample<FORM, NL, true>(p, k, s, w, u, gv[j], eo, t + i + j, active, o);
+                else sweep_sample<FORM, NL, true>(p, k, s, w, u, gv[j], ee, t + i + j, active, o);
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < U; ++j) {
+                const float2 u = make_float2(xv[2 * j], xv[2 * j + 1]);
+                if (j & 1) sweep_sample<FORM, NL, false>(p, k, s, w, u, gv[j], eo, t + i + j, active, o);
+                else sweep_sample<FORM, NL, false>(p, k, s, w, u, gv[j], ee, t + i + j, active, o);
+            }
+        }
+    }
+    for (; i < cnt; ++i) {
+        const float2 xz = sxz[i];
+        if (i & 1) sweep_sample<FORM, NL, STORE>(p, k, s, w, xz, sg[i], eo, t + i, active, o);
+        else sweep_sample<FORM, NL, STORE>(p, k, s, w, xz, sg[i], ee, t + i, active, o);
+    }
+}
+
 struct Smem {
     float2 (*xz)[kTile];
     float (*g)[kTile];
@@ -255,8 +351,9 @@ struct Smem {
 
 // The whole CTA (= one warp = 32 adjacent channels) for one section form.
 // EDGE: the edge residuals come from the per-utterance table (time-chunked batches) instead of
-// the in-kernel pass.
-template <int FORM, int U, bool EDGE, bool WIN, bool CN>
+// the in-kernel pass.  SW > 0: the cutoff sweep (p.sw_planes planes of decimated frames) with SW one-pole
+// states.
+template <int FORM, int U, bool EDGE, bool WIN, bool CN, int SW = 0>
 __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& item, const Smem& sm, const int c) {
     const UttDesc ut = p.utts[item.utt];
     const int tid = threadIdx.x;
@@ -317,6 +414,9 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
 
     typename SectionTypes<FORM>::S s;
     reset(s);
+    float wsw[SW > 0 ? SW : 1];   // SW: the sweep's one-pole states
+#pragma unroll
+    for (int r = 0; r < (SW > 0 ? SW : 1); ++r) wsw[r] = 0.f;
     E ee[4] = {0, 0, 0, 0}, eo[4] = {0, 0, 0, 0};
     if (EDGE && need_imag && active) {
         if constexpr (FORM == 2) load_edge_entry(p.edge64, item.utt, p.C, c, ee, eo);
@@ -395,7 +495,10 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const Item& ite
             } else if (t < tenv) {
                 run_tile<FORM, 0, 0, false, U>(p, k, s, ee, eo, sxz, sg, t, cnt, active, o);
             } else if (t < t0) {
-                run_tile<FORM, 2, 0, false, U>(p, k, s, ee, eo, sxz, sg, t, cnt, active, o);
+                if constexpr (SW > 0) run_tile_sweep<FORM, SW, false, U>(p, k, s, wsw, ee, eo, sxz, sg, t, cnt, active, o);
+                else run_tile<FORM, 2, 0, false, U>(p, k, s, ee, eo, sxz, sg, t, cnt, active, o);
+            } else if constexpr (SW > 0) {
+                run_tile_sweep<FORM, SW, true, U>(p, k, s, wsw, ee, eo, sxz, sg, t, cnt, active, o);
             } else if (full_out) {
                 // full-rate stores: the 8-sample unroll is the faster one (3.9 vs 4.9 ms on 256 utterances)
                 constexpr int UF = U < 8 ? U : 8;
@@ -446,6 +549,37 @@ __global__ void __launch_bounds__(kChanPerBlock, MINB) fused_kernel(const FusedP
     }
 }
 
+// The cutoff sweep (FusedParams::sw_planes > 0): decimated frames only, NL one-pole states.
+template <bool F64, int MINB, int U, bool EDGE, int NL>
+__global__ void __launch_bounds__(kChanPerBlock, MINB) fused_sweep_kernel(const FusedParams p) {
+    __shared__ __align__(128) float2 s_xz[kStages][kTile];
+    __shared__ __align__(128) float s_g[kStages][kTile];
+    __shared__ __align__(8) uint64_t s_full[kStages];
+    if (threadIdx.x == 0) {
+        for (int b = 0; b < kStages; ++b) mbar_init(&s_full[b], 1);
+        mbar_fence_init();
+    }
+    __syncwarp();
+    const Item item = p.items[blockIdx.x];
+    const int c = item.cblock * kChanPerBlock + threadIdx.x;
+    const Smem sm{s_xz, s_g, s_full, nullptr};
+    if constexpr (F64) {
+        fused_body<2, U, EDGE, false, false, NL>(p, item, sm, c);
+    } else {
+        const float group_cy = p.chan[P_FORM * p.c_pad + c];
+        if (group_cy >= p.direct_min_cy) fused_body<1, U, EDGE, false, false, NL>(p, item, sm, c);
+        else fused_body<0, U, EDGE, false, false, NL>(p, item, sm, c);
+    }
+}
+
+template <bool F64, int MINB, int U, int NL>
+static void launch_sweep_nl(const FusedParams& p, int n_items, cudaStream_t stream) {
+    if (F64 ? p.edge64 != nullptr : p.edge != nullptr)
+        fused_sweep_kernel<F64, MINB, U, true, NL><<<n_items, kChanPerBlock, 0, stream>>>(p);
+    else
+        fused_sweep_kernel<F64, MINB, U, false, NL><<<n_items, kChanPerBlock, 0, stream>>>(p);
+}
+
 template <bool F64, int MINB, int U>
 static void launch_variant(const FusedParams& p, int n_items, cudaStream_t stream) {
     const bool edge = F64 ? p.edge64 != nullptr : p.edge != nullptr;
@@ -465,6 +599,18 @@ static void launch_variant(const FusedParams& p, int n_items, cudaStream_t strea
 
 cudaError_t launch_fused(const FusedParams& p, int n_items, bool float64, cudaStream_t stream) {
     if (n_items <= 0) return cudaSuccess;
+    if (p.sw_planes > 0) {
+        // float32: one instantiation per number of one-pole states, so that a setting without low-pass
+        // costs no FMA per sample.  Four states do not fit 128 registers (16 CTAs per SM) with 16 samples per
+        // loop trip without spilling: that instantiation loads 8 per trip.  FORM 2 (float64 sections dominate
+        // its time): four states always.
+        if (float64) launch_sweep_nl<true, 12, 8, 4>(p, n_items, stream);
+        else if (p.sw_lp <= 1) launch_sweep_nl<false, 16, 16, 1>(p, n_items, stream);
+        else if (p.sw_lp == 2) launch_sweep_nl<false, 16, 16, 2>(p, n_items, stream);
+        else if (p.sw_lp == 3) launch_sweep_nl<false, 16, 16, 3>(p, n_items, stream);
+        else launch_sweep_nl<false, 16, 8, 4>(p, n_items, stream);
+        return cudaGetLastError();
+    }
     // float32: 16 one-warp CTAs per SM, 16 samples per loop trip (profiles/r01j_tune_*.log, r01m); the
     // window-store mode is its own instantiation so that the other modes keep their code.  FORM 2: 12 and 8.
     if (float64) launch_variant<true, 12, 8>(p, n_items, stream);

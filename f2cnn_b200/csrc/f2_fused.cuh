@@ -35,7 +35,18 @@ struct FusedParams {
     const double* edge64;  // float64 edge residuals [utt][C][8] of the FORM 2 groups (f2_edge.cu; null: in-kernel)
     int gfb_cn_f64;      // element type of gfb_cn: 1 = float64, 0 = float32
     int env_cn_f64;      // element type of env_cn: 1 = float64, 0 = float32
+    // Cutoff sweep (f2_batch_run_cutoffs; 0 = off): plane j of the decimated frames is stored at
+    // dec + j * plane_stride.  Plane j reads one-pole state sw_state[j] (-1: no low-pass); states
+    // 0 .. sw_lp-1 have their own lp_k and b0.  lpf and w_lpf then describe the slowest of them.
+    int sw_planes;
+    int sw_lp;
+    int sw_state[4];
+    float sw_k[4];
+    float sw_b0[4];
+    long long plane_stride;
 };
+
+constexpr int kMaxCutoffs = 4;
 
 // float64: p.items are work items of FORM 2 groups (float64 sections), run by their own instantiations.
 cudaError_t launch_fused(const FusedParams& p, int n_items, bool float64, cudaStream_t stream);

@@ -278,6 +278,57 @@ class Batch:
         check(_native.lib().f2_batch_run(self._h, ctypes.byref(a), _ptr(ws), ws.numel(), _stream_ptr(stream)))
         return res
 
+    def run_cutoffs(self, wave_dev, cutoffs, out=None, stream=None):
+        """Decimated frames of several envelope settings from one filterbank and Hilbert pass
+        (f2_batch_run_cutoffs): (K, total_frames, C) float32, plane j equal to
+        run(dec=True, lpf=cutoffs[j] is not None, cutoff=cutoffs[j])["dec"].  cutoffs: 1..4 entries, each a
+        cutoff in (0, 8000) Hz or None for no low-pass.  `out`: a (K, total_frames, C) float32 tensor on the
+        plan's device or in pinned host memory whose planes may lie further apart than total_frames * C (a
+        slice of a larger array)."""
+        plan = self.plan
+        C = plan.n_channels
+        hz = cutoff_settings(cutoffs)
+        K = len(hz)
+        if wave_dev.numel() != self.total_samples:
+            raise ValueError("wave has %d samples, batch expects %d" % (wave_dev.numel(), self.total_samples))
+        if wave_dev.device != plan.device:
+            raise ValueError("wave is on %s, plan on %s" % (wave_dev.device, plan.device))
+        if not wave_dev.is_contiguous() or wave_dev.dtype not in _T2F2:
+            raise ValueError("wave must be a contiguous int16 / float32 / float64 tensor")
+        if out is None:
+            out = torch.empty((K, self.total_frames, C), dtype=torch.float32, device=plan.device)
+        mapped = out.device.type == "cpu" and out.is_pinned()
+        if (out.dtype != torch.float32 or tuple(out.shape) != (K, self.total_frames, C) or
+                (K > 1 and out.stride(0) < self.total_frames * C) or
+                (self.total_frames > 0 and out[0].stride() != (C, 1)) or (out.device != plan.device and not mapped)):
+            raise ValueError("out: need a (%d, %d, %d) float32 tensor on %s with contiguous planes" %
+                             (K, self.total_frames, C, plan.device))
+        stride = out.stride(0) if K > 1 else self.total_frames * C
+        ws = plan.workspace(self.workspace_bytes(), stream)
+        arr = (ctypes.c_double * K)(*hz)
+        check(_native.lib().f2_batch_run_cutoffs(self._h, _ptr(wave_dev), _T2F2[wave_dev.dtype], arr, K, _ptr(out),
+                                                 stride, _ptr(ws), ws.numel(), _stream_ptr(stream)))
+        return out
+
+
+def cutoff_settings(cutoffs):
+    """Envelope settings of a cutoff sweep -> the Hz values f2_batch_run_cutoffs takes (0 = no low-pass).
+    None is how a caller says "no low-pass" (LPF = CUTOFF is not None in the reference's f2cnn.py); 0 Hz is
+    refused like any other cutoff outside (0, 8000), as butter refuses it."""
+    cutoffs = list(cutoffs)
+    if not 1 <= len(cutoffs) <= 4:
+        raise ValueError("a cutoff sweep takes 1 to 4 settings, got %d" % len(cutoffs))
+    hz = []
+    for c in cutoffs:
+        if c is None:
+            hz.append(0.0)
+            continue
+        f = float(c)
+        if not 0.0 < f < 8000.0:
+            raise ValueError("cutoff must be None (no low-pass) or in (0, 8000) Hz, got %r" % (c,))
+        hz.append(f)
+    return hz
+
 
 class DeviceEvent:
     """cudaEvent_t owned through the C ABI (recorded on the stream the kernels run on)."""
@@ -444,11 +495,17 @@ class WindowPipeline:
     lengths[u]: samples of utterance u; src_offsets[u]: where it starts in the host buffer passed
     to run() (default: back to back), so a shard can read its utterances out of the buffer that
     holds the whole corpus.  Frames are numbered over the pipeline's utterances in order
-    (`frame_offsets`), which is what engine.window_runs wants."""
+    (`frame_offsets`), which is what engine.window_runs wants.
+
+    cutoffs: a sequence of 1..4 envelope settings (None = no low-pass) instead of lpf / cutoff: every
+    sub-batch then stores the frames of all of them from one filterbank pass (Batch.run_cutoffs), one
+    pinned plane per setting, and run() takes one output per setting (the number of settings is fixed
+    here; which cutoffs, `self.cutoffs`, may change between runs)."""
 
     def __init__(self, plan, lengths, dots=11, step=160, phase=0, lpf=True, cutoff=50, n_sub=None, src_offsets=None,
-                 placer=None):
+                 placer=None, cutoffs=None):
         self.plan, self.dots, self.lpf, self.cutoff = plan, int(dots), bool(lpf), cutoff
+        self.cutoffs = None if cutoffs is None else tuple(cutoffs)
         self.step, self.phase = int(step), int(phase)
         lengths = np.ascontiguousarray(lengths, dtype=np.int64).reshape(-1)
         self.lengths = lengths
@@ -506,7 +563,9 @@ class WindowPipeline:
         self._wave_dev = None
         self._stage = None      # pinned staging for pageable input
         with torch.cuda.device(dev):
-            self._dec_host = _pinned_empty(max(self.total_frames, 1) * C, torch.float32).view(-1, C)
+            n_planes = 1 if self.cutoffs is None else len(self.cutoffs)
+            self._dec_host = _pinned_empty(max(self.total_frames, 1) * C * n_planes, torch.float32).view(-1, C)
+            self._planes = self._dec_host.view(n_planes, -1, C)
             self._s_in, self._s_out = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
             # consecutive sub-batches alternate between two compute streams: a launch ends with a tail
             # of its longest utterances on half-empty SMs, and the next launch's CTAs fill them
@@ -545,7 +604,8 @@ class WindowPipeline:
         """wave_host: flat host tensor (int16 / float32 / float64; pinned for full speed -- pageable
         input is staged through a pinned buffer sub-batch by sub-batch) or a list of per-utterance
         numpy arrays; runs: (n, 3) int64 from engine.window_runs on this pipeline's frame_offsets;
-        out_host: the (N, dots, C) float32 host array or tensor the rows go to (any host memory).
+        out_host: the (N, dots, C) float32 host array or tensor the rows go to (any host memory); with
+        `cutoffs`, a list of one such array per setting.
         Returns when every row has been placed."""
         # no garbage-collector pause while the launch sequence is being queued: a generation-0/1 sweep of a
         # torch process takes ~5 ms, and when it hit between the kernel launches and the placement submits one
@@ -611,9 +671,13 @@ class WindowPipeline:
                     self._ev_in[i].record(self._s_in)
             comp = self._s_comp[i & 1]
             comp.wait_event(self._ev_in[i])
-            dec = self._dec_host[sub["f0"]:sub["f1"]]
-            sub["batch"].run(self._wave_dev[sub["s0"]:sub["s1"]], lpf=self.lpf, cutoff=self.cutoff, out={"dec": dec},
-                             stream=comp)
+            if self.cutoffs is None:
+                dec = self._dec_host[sub["f0"]:sub["f1"]]
+                sub["batch"].run(self._wave_dev[sub["s0"]:sub["s1"]], lpf=self.lpf, cutoff=self.cutoff, out={"dec": dec},
+                                 stream=comp)
+            else:
+                sub["batch"].run_cutoffs(self._wave_dev[sub["s0"]:sub["s1"]], self.cutoffs,
+                                         out=self._planes[:, sub["f0"]:sub["f1"]], stream=comp)
             self._ev_done[i].record(comp)
         # Uploads and kernels of every sub-batch are queued; only now is the placement plan needed.  `runs`
         # may be a callable: the run detection of a corpus (a few ms on the host) then happens while the
@@ -624,8 +688,11 @@ class WindowPipeline:
         with torch.cuda.stream(self._s_out):
             for i, sub in enumerate(self.subs):
                 self._s_out.wait_event(self._ev_done[i])
-                if per_sub[i].shape[0]:
+                if per_sub[i].shape[0] and self.cutoffs is None:
                     self.placer.submit(self._dec_host, per_sub[i], out_flat, dots=self.dots, stream=self._s_out)
+                elif per_sub[i].shape[0]:
+                    for plane, out_j in zip(self._planes, out_host):
+                        self.placer.submit(plane, per_sub[i], out_j, dots=self.dots, stream=self._s_out)
             self._ev_end.record(self._s_out)
         for s_ in (self._s_out, self._s_comp[0], self._s_comp[1]):
             caller.wait_stream(s_)

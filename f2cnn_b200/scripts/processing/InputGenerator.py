@@ -12,6 +12,8 @@ The window gather runs on the GPU (float64 -> float32 on the device rounds to ne
 numpy.astype).  Extension: an utterance whose .ENV1.npy is missing but whose .WAV is present is
 computed by the fused filterbank+envelope kernel, all such utterances in ONE batched launch
 sequence (the reference would stop with FileNotFoundError).
+Extension: GenerateInputDataSweep writes the input_data_LPF<k>.npy / input_data_NOLPF.npy of
+several cutoffs from one filterbank pass over the .WAV files.
 """
 import csv
 import os
@@ -50,20 +52,26 @@ def _say_lpf(LPF, CUTOFF):
     print("Using Low Pass Filtering with a cutoff at {}Hz".format(CUTOFF) if LPF else "Not using Low Pass Filtering")
 
 
-def _fill_from_waveforms(pending, out, cfg, rate, channels, radius, step, LPF, CUTOFF):
-    """pending: [(first row, wav path, timepoints)].  One batch for all of them."""
+def _bank_and_waves(paths, cfg, rate, channels):
+    """The configured filterbank and the waveforms of `paths` (features_to_windows' `waves` argument)."""
     from concurrent.futures import ThreadPoolExecutor
-    from ... import api, ingest
+    from ... import ingest
     from ...gammatone import filters
     from .GammatoneFiltering import GetArrayFromWAV
     low = cfg.getint('FILTERBANK', 'LOW_FREQ')
     coefs = filters.make_erb_filters(rate, filters.centre_freqs(rate, channels, low))
     try:  # mono 16-bit PCM (TIMIT): straight into one pinned buffer
-        flat, lengths, _ = ingest.read_corpus([p[1] for p in pending])
-        waves = (flat, lengths)
+        flat, lengths, _ = ingest.read_corpus(paths)
+        return coefs, (flat, lengths)
     except ValueError:  # anything else (e.g. the float64 WAVs of `cnn evalnoise`): decode file by file
         with ThreadPoolExecutor(max_workers=8) as readers:
-            waves = [samples for _, samples in readers.map(GetArrayFromWAV, [p[1] for p in pending])]
+            return coefs, [samples for _, samples in readers.map(GetArrayFromWAV, paths)]
+
+
+def _fill_from_waveforms(pending, out, cfg, rate, channels, radius, step, LPF, CUTOFF):
+    """pending: [(first row, wav path, timepoints)].  One batch for all of them."""
+    from ... import api
+    coefs, waves = _bank_and_waves([p[1] for p in pending], cfg, rate, channels)
     rows = api.features_to_windows(waves, coefs, [p[2] for p in pending], LPF, CUTOFF, radius, step)
     cursor = 0
     for first, _, points in pending:
@@ -123,3 +131,54 @@ def GenerateInputData(labelFile=None, inputFile=None, LPF=False, CUTOFF=100):
     numpy.save(os.path.join(_OUT_DIR, 'last_input_data.npy'), data)  # the reference's "just in case" copy
     print('                Total time:', time.time() - started)
     print('')
+
+
+def GenerateInputDataSweep(labelFile=None, CUTOFFS=(20, 50, 100)):
+    """GenerateInputData for several cutoffs at once: trainingData/input_data_LPF<k>.npy for every k of
+    CUTOFFS, input_data_NOLPF.npy for an entry None, rows ordered as GenerateInputData orders them.  The
+    filterbank and the Hilbert transform run once for all cutoffs (api.features_to_windows_sweep), so the
+    envelopes always come from the .WAV files: an .ENV1.npy on disk holds one cutoff and cannot serve a
+    sweep.  A missing .WAV raises FileNotFoundError.  Unlike GenerateInputData, no
+    trainingData/last_input_data.npy is written: there is no single last input."""
+    from ... import api
+    started = time.time()
+    if not os.path.isdir(_OUT_DIR):
+        print("LABEL GENERATION SHOULD BE DONE PRIOR TO INPUT...")
+        exit(-1)
+    cutoffs = list(CUTOFFS)
+    labels = labelFile or os.path.join(_OUT_DIR, "label_data.csv")
+    per_file = GetListOfEnvelopeFilesAndTimepoints(labels)
+    print("\n###############################\nGenerating Input Data from files with '{}'.".format(labels))
+    for cutoff in cutoffs:
+        _say_lpf(cutoff is not None, cutoff)
+    if not per_file:
+        print("NO ENV1.npy FILES FOUND, PLEASE GENERATE ENVELOPES")
+        exit(-1)
+    order = sorted(per_file)
+    total = sum(len(v) for v in per_file.values())
+    print(len(order), "files found along with their", total, "entry timepoints.")
+
+    cfg, radius, step, rate, channels = _geometry()
+    print("Output shape:", (total, 2 * radius + 1, channels), "x", len(cutoffs))
+    pending = []
+    for done, key in enumerate(order, start=1):
+        saved = os.path.join(_ROOT, key)
+        wave_path = saved[:-len('.ENV1.npy')] + '.WAV'
+        print("Reading:\t{}".format(wave_path))
+        if not os.path.isfile(wave_path):
+            raise FileNotFoundError(2, 'No such file or directory', wave_path)
+        pending.append((wave_path, per_file[key]))
+        print("\t\t{:<50} done !  {}/{} Files".format(wave_path, done, len(order)))
+    coefs, waves = _bank_and_waves([p[0] for p in pending], cfg, rate, channels)
+    planes = api.features_to_windows_sweep(waves, coefs, [p[1] for p in pending], cutoffs, radius, step)
+
+    os.makedirs(_OUT_DIR, exist_ok=True)
+    for cutoff, data in zip(cutoffs, planes):
+        print('Generated Input Matrix of shape {}.'.format(data.shape))
+        name = 'input_data_LPF{}.npy'.format(cutoff) if cutoff is not None else 'input_data_NOLPF.npy'
+        target = os.path.join(_OUT_DIR, name)
+        print("Saving as {}...".format(target))
+        numpy.save(target, data)
+    print('                Total time:', time.time() - started)
+    print('')
+

@@ -145,6 +145,21 @@ typedef struct f2_run_args {
  * GenerateInputData (InputGenerator.py:73-80). */
 F2_API int f2_batch_run(f2_batch* batch, const f2_run_args* args, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Decimated envelope frames of 1..4 envelope settings from ONE filterbank and Hilbert pass (the reference's
+ * `prepare input --cutoff K` for several K: input_data_LPF<K>.npy, input_data_NOLPF.npy).  cutoffs_hz: HOST
+ * array of n_settings entries, each a cutoff in (0, 8000) Hz or 0 for no low-pass.  Setting j's frames go to
+ * dec + j * plane_stride, [total_frames][C] float32 on the batch's grid, exactly as f2_run_args.dec of an
+ * f2_batch_run with that setting; plane_stride >= total_frames * C lets a sub-batch write its slice of a
+ * larger [K][frames][C] array.  dec is device memory or memory pinned with f2_host_pin.  Workspace:
+ * f2_batch_workspace_bytes.  Whole-utterance batches give every plane bit for bit what f2_batch_run gives;
+ * in a time-chunked batch every chunk warms up for the lowest cutoff, so that cutoff's plane is bit-identical
+ * and the others differ from their own runs only by the longer warm-up (below float32 resolution).
+ * F2_ERR_INVALID: n_settings outside 1..4, a cutoff that is NaN or outside {0} u (0, 8000), a null dec or a
+ * short plane_stride; F2_ERR_WORKSPACE: a short workspace. */
+F2_API int f2_batch_run_cutoffs(f2_batch* batch, const void* wave, int wave_dtype, const double* cutoffs_hz,
+                                int n_settings, float* dec, int64_t plane_stride, void* workspace,
+                                size_t workspace_bytes, void* stream);
+
 /* ---- stand-alone envelope of arbitrary matrix rows ---------------------------------------
  * ExtractEnvelopeFromMatrix(matrix, LPF, CUTOFF) for a matrix that did not come from this
  * library (e.g. loaded from .GFB.npy, EnvelopeExtraction.py:70-83): rows x n, row-major. */
