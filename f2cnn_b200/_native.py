@@ -128,6 +128,9 @@ SIGNATURES = {
     "f2_cnn_forward": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int64,
                                       ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
                                       ctypes.c_void_p]),
+    "f2_cnn_forward_segments": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
+                                               ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                                               ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
     "f2_cnn_workspace_layout": (ctypes.c_int, [ctypes.c_int64, ctypes.POINTER(ctypes.c_int64),
                                                ctypes.POINTER(ctypes.c_size_t)]),
     "f2_umma_selftest": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,

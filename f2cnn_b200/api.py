@@ -322,9 +322,9 @@ def release_cached_pipelines():
     engine.release_host_pool()
 
 
-def _corpus(waves, timepoints, counts):
-    """The (waves, timepoints, counts) arguments of features_to_windows -> (flat host tensor or None, list of
-    waves or None, lengths, flat centres, counts)."""
+def _waves_lengths(waves):
+    """waves as a list of 1-D arrays or as (flat, lengths) -> (flat host tensor or None, list of waves or None,
+    lengths).  Listed waves of different dtypes are promoted to float64."""
     flat_in = None
     if isinstance(waves, tuple) and len(waves) == 2:
         flat_in, lengths = waves
@@ -333,14 +333,19 @@ def _corpus(waves, timepoints, counts):
             flat_in = torch.from_numpy(_as_wave(flat_in))
         if flat_in.dim() != 1 or flat_in.numel() != int(lengths.sum()):
             raise ValueError("flat buffer holds %d samples, lengths add up to %d" % (flat_in.numel(), int(lengths.sum())))
-        n_utts = int(lengths.shape[0])
     else:
         waves = [_as_wave(w) for w in waves]
-        dts = {w.dtype for w in waves}
-        if len(dts) > 1:
+        if len({w.dtype for w in waves}) > 1:
             waves = [w.astype(np.float64) for w in waves]
         lengths = np.asarray([w.shape[0] for w in waves], dtype=np.int64)
-        n_utts = len(waves)
+    return flat_in, waves, lengths
+
+
+def _corpus(waves, timepoints, counts):
+    """The (waves, timepoints, counts) arguments of features_to_windows -> (flat host tensor or None, list of
+    waves or None, lengths, flat centres, counts)."""
+    flat_in, waves, lengths = _waves_lengths(waves)
+    n_utts = int(lengths.shape[0])
     if counts is not None:
         centers = np.ascontiguousarray(timepoints, dtype=np.int64).reshape(-1)
         counts = np.ascontiguousarray(counts, dtype=np.int64).reshape(-1)
@@ -625,19 +630,7 @@ def features_to_frames(waves, coefs, LPF=False, CUTOFF=100, radius=5, step=160, 
     coefs = np.asarray(coefs, dtype=np.float64)
     plan = engine.plan_for(coefs)
     dots = 2 * radius + 1
-    flat_in = None
-    if isinstance(waves, tuple) and len(waves) == 2:
-        flat_in, lengths = waves
-        lengths = np.ascontiguousarray(lengths, dtype=np.int64)
-        if not torch.is_tensor(flat_in):
-            flat_in = torch.from_numpy(_as_wave(flat_in))
-        if flat_in.dim() != 1 or flat_in.numel() != int(lengths.sum()):
-            raise ValueError("flat buffer holds %d samples, lengths add up to %d" % (flat_in.numel(), int(lengths.sum())))
-    else:
-        waves = [_as_wave(w) for w in waves]
-        if len({w.dtype for w in waves}) > 1:
-            waves = [w.astype(np.float64) for w in waves]
-        lengths = np.asarray([w.shape[0] for w in waves], dtype=np.int64)
+    flat_in, waves, lengths = _waves_lengths(waves)
     n_frames = (lengths + step - 1) // step
     grid = np.maximum((lengths / step - dots - 1).astype(np.int64), 0)
     if counts is None:
@@ -756,6 +749,90 @@ def cnn_evaluate(wave, coefs, weights, LPF=False, CUTOFF=100, radius=5, step=160
                                                              env_t=True)["env_t"]
     scores = net.predict_envelope(env_t, step)
     return _to_host(scores), envelopes
+
+
+_CNN_ENV_BYTES = 2 << 30   # time-major envelope of one sub-batch of cnn_evaluate_corpus (512 bytes per sample)
+
+
+def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, step=160, out=None, shard=None):
+    """cnn_evaluate for a whole corpus: the scores of every stride-1 frame of every utterance, e.g. a test set
+    scored by a trained model.  waves: list of 1-D arrays, or (flat, lengths) as returned by ingest.read_corpus.
+    Returns (scores, offsets): scores is the float32 (sum(nb_u), 2) host array with nb_u = max(n_u - (2R+1)*step,
+    0) (Evaluating.py:70-78), and utterance u's scores are scores[offsets[u]:offsets[u+1]].
+
+    Utterances go through the front end in sub-batches of whole utterances (never split into time chunks, so an
+    utterance's envelope and scores do not depend on the sub-batch or shard it lands in), and each sub-batch
+    through the network in one pass whose chunks run across utterance boundaries
+    (TensorCoreCNN.predict_segments).  Scores equal cnn_evaluate's where cnn_evaluate computes the same envelope
+    (it may split a lone long utterance into time chunks, whose envelope differs in the last float32 bits).
+    Raises ValueError naming the first utterance with a frame value <= 0 (Training.normalizeInput).
+    out: an existing C-contiguous float32 (sum(nb_u), 2) array to fill.  shard=(rank, world): one of `world`
+    processes (one per GPU) handed the same corpus and the same `out` -- a shared mapping,
+    hostmem.SharedArray -- scores the utterances engine.shard_utterances deals to `rank` and writes them, and
+    only them, at their final offsets.  Only the configured geometry (RADIUS = 5, 128 channels)."""
+    from . import cnn
+    coefs = np.asarray(coefs, dtype=np.float64)
+    if radius != 5 or coefs.shape[0] != 128:
+        raise ValueError("the tensor-core network is built for RADIUS = 5 and 128 channels")
+    flat_in, waves, lengths = _waves_lengths(waves)
+    if flat_in is not None and flat_in.device.type != "cpu":
+        raise ValueError("cnn_evaluate_corpus takes the flat wave buffer in host memory (it is on %s)" % flat_in.device)
+    step = int(step)
+    nb = np.maximum(lengths - (2 * radius + 1) * step, 0)
+    offsets = np.concatenate([[0], np.cumsum(nb)]).astype(np.int64)
+    total = int(offsets[-1])
+    if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"]
+                                and out.shape == (total, 2)):
+        raise ValueError("out must be a C-contiguous float32 array of shape %s" % ((total, 2),))
+    sel = np.arange(lengths.shape[0])
+    if shard is not None:
+        rank, world = int(shard[0]), int(shard[1])
+        if out is None or not 0 <= rank < world:
+            raise ValueError("shard=(rank, world) needs 0 <= rank < world and the shared `out` array")
+        sel = engine.shard_utterances(lengths, world)[rank]
+    scores = np.empty((total, 2), dtype=np.float32) if out is None else out
+    sel = sel[nb[sel] > 0]          # an utterance without frames has nothing to score
+    if sel.size == 0:
+        return scores, offsets
+    plan = engine.plan_for(coefs)
+    net = _network_for(weights)
+    # consecutive utterances (in `sel` order) whose envelopes fit _CNN_ENV_BYTES; a larger one goes alone
+    env_bytes = lengths[sel] * plan.n_channels * 4
+    subs, start, used = [], 0, 0
+    for i, b in enumerate(env_bytes):
+        if used + b > _CNN_ENV_BYTES and i > start:
+            subs.append(sel[start:i])
+            start, used = i, 0
+        used += int(b)
+    subs.append(sel[start:])
+    src = np.concatenate([[0], np.cumsum(lengths)]).astype(np.int64)
+    host = flat_in.numpy() if flat_in is not None else None
+    wdt = flat_in.dtype if flat_in is not None else torch.from_numpy(waves[0][:0]).dtype
+    max_samples = max(int(lengths[sub].sum()) for sub in subs)
+    max_frames = max(int(nb[sub].sum()) for sub in subs)
+    stage = torch.empty(max_samples, dtype=wdt, pin_memory=True)
+    wave_dev = torch.empty(max_samples, dtype=wdt, device=plan.device)
+    env_buf = torch.empty((max_samples, plan.n_channels), dtype=torch.float32, device=plan.device)
+    scores_host = torch.empty((max_frames, 2), dtype=torch.float32, pin_memory=True)
+    for sub in subs:
+        lens = lengths[sub]
+        n = int(lens.sum())
+        np.concatenate([host[src[u]:src[u + 1]] if host is not None else waves[u] for u in sub], out=stage.numpy()[:n])
+        wave_dev[:n].copy_(stage[:n], non_blocking=True)
+        batch = plan.batch(lens, step=step, target_items=1)
+        env_t = batch.run(wave_dev[:n], lpf=LPF, cutoff=CUTOFF, out={"env_t": env_buf[:n]})["env_t"]
+        try:
+            sc = net.predict_segments(env_t, step, batch.sample_offsets[:-1], nb[sub])
+        except cnn.NonPositiveInput as e:
+            raise ValueError("values must all be positive (utterance %d)" % int(sub[e.segment])) from None
+        k = int(sc.shape[0])
+        scores_host[:k].copy_(sc)
+        got = scores_host.numpy()
+        at = 0
+        for u in sub:
+            scores[offsets[u]:offsets[u + 1]] = got[at:at + nb[u]]
+            at += int(nb[u])
+    return scores, offsets
 
 
 def label_fit(tracks, firsts, centers, radius=5, step=160):

@@ -130,9 +130,7 @@ class TensorCoreCNN:
         frame i = rows i + k*step, k < 11, normalised per frame like Training.normalizeInput
         (Evaluating.py:70-87).  Returns an (n_frames, 2) float32 device tensor; raises ValueError where
         normalizeInput would (a value <= 0)."""
-        if env_t.dtype != torch.float32 or not env_t.is_contiguous() or env_t.dim() != 2 or env_t.shape[1] != 128 \
-                or env_t.device != self.device:
-            raise ValueError("env_t: contiguous float32 [n, 128] tensor on %s" % self.device)
+        self._check_env_t(env_t)
         n = int(env_t.shape[0])
         nb = max(n - 11 * int(step), 0)
         i0, i1 = (0, nb) if frames is None else (int(frames[0]), int(frames[1]))
@@ -142,10 +140,7 @@ class TensorCoreCNN:
         if i1 == i0:
             return scores
         L = _native.lib()
-        need = int(L.f2_cnn_workspace_bytes(self._h, i1 - i0))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        self._workspace(i1 - i0)
         flags = torch.zeros(2, dtype=torch.int32, device=self.device)
         s = stream if stream is not None else torch.cuda.current_stream(self.device)
         check(L.f2_cnn_forward(self._h, ctypes.c_void_p(env_t.data_ptr()), n, int(step), i0, i1,
@@ -158,6 +153,56 @@ class TensorCoreCNN:
             raise ValueError("values must all be positive")  # Training.py:18-20
         return scores
 
+    def predict_segments(self, env_t, step, rows, counts, stream=None):
+        """Scores of several utterances whose envelopes lie in ONE time-major env_t ([n, 128] float32 on the
+        device), in one pass: segment s is counts[s] stride-1 frames starting at row rows[s] (frame i of it =
+        rows rows[s] + i + k*step, k < 11), e.g. every frame of utterance s (counts[s] = max(n_s - 11*step, 0)).
+        Returns the (sum(counts), 2) float32 device tensor of the segments' scores back to back; each frame's
+        scores are bit for bit those predict_envelope gives for it.  Raises NonPositiveInput (a ValueError)
+        naming the first segment that has a frame holding a value <= 0 (Training.normalizeInput raises there)."""
+        self._check_env_t(env_t)
+        rows = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+        counts = np.ascontiguousarray(counts, dtype=np.int64).reshape(-1)
+        if rows.shape != counts.shape:
+            raise ValueError("rows and counts: one entry per segment")
+        n, step = int(env_t.shape[0]), int(step)
+        live = counts > 0
+        if np.any(rows < 0) or np.any(counts < 0) or np.any(rows[live] + counts[live] + 10 * step > n):
+            raise IndexError("a segment's frames leave the %d rows of this envelope" % n)
+        total = int(counts.sum())
+        scores = torch.empty((total, 2), dtype=torch.float32, device=self.device)
+        if total == 0:
+            return scores
+        L = _native.lib()
+        self._workspace(total)
+        n_segs = int(rows.shape[0])
+        flags = torch.zeros(n_segs + 1, dtype=torch.int32, device=self.device)
+        s = stream if stream is not None else torch.cuda.current_stream(self.device)
+        check(L.f2_cnn_forward_segments(self._h, ctypes.c_void_p(env_t.data_ptr()), n, step,
+                                        rows.ctypes.data_as(ctypes.c_void_p), counts.ctypes.data_as(ctypes.c_void_p),
+                                        n_segs, ctypes.c_void_p(scores.data_ptr()), ctypes.c_void_p(flags.data_ptr()),
+                                        ctypes.c_void_p(self._ws.data_ptr()), self._ws.numel(),
+                                        ctypes.c_void_p(s.cuda_stream)))
+        s.synchronize()
+        flags = flags.cpu().numpy()
+        if flags[-1]:
+            raise RuntimeError("tensor-core pipeline did not complete (stage %d)" % flags[-1])
+        bad = np.flatnonzero(flags[:-1])
+        if bad.size:
+            raise NonPositiveInput(int(bad[0]))
+        return scores
+
+    def _check_env_t(self, env_t):
+        if env_t.dtype != torch.float32 or not env_t.is_contiguous() or env_t.dim() != 2 or env_t.shape[1] != 128 \
+                or env_t.device != self.device:
+            raise ValueError("env_t: contiguous float32 [n, 128] tensor on %s" % self.device)
+
+    def _workspace(self, n_frames):
+        need = int(_native.lib().f2_cnn_workspace_bytes(self._h, int(n_frames)))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+
     def intermediates(self, n_frames):
         """(pooled conv2 output (n, 32, 4, 63), features (n, 1920)) of the last chunk, as float32 -- for
         the layer-by-layer tests (n_frames <= 32768 so that the chunk is the whole call)."""
@@ -168,6 +213,15 @@ class TensorCoreCNN:
         pooled = raw.permute(0, 1, 3, 2).reshape(n_frames, 32, 4, 63).float()
         feat = self._ws[base + off.value:base + off.value + n_frames * 1920 * 2].view(torch.bfloat16).view(n_frames, 1920)
         return pooled, feat.float()
+
+
+class NonPositiveInput(ValueError):
+    """A frame of segment `segment` of TensorCoreCNN.predict_segments held a value <= 0: the ValueError
+    Training.normalizeInput raises (Training.py:18-20)."""
+
+    def __init__(self, segment):
+        super().__init__("values must all be positive (segment %d)" % segment)
+        self.segment = segment
 
 
 def keras_arrays(model):

@@ -1181,20 +1181,60 @@ int f2_cnn_workspace_layout(int64_t n_frames, int64_t* chunk_frames, size_t* fea
     return F2_OK;
 }
 
+namespace {
+int cnn_launch(f2_cnn* c, const float* env_t, int step, const int64_t* seg_rows, const int64_t* seg_frames, int n_segs,
+               int64_t total, float* scores, int* flags, void* workspace, size_t workspace_bytes, void* stream) {
+    const size_t need = f2_cnn_workspace_bytes(c, total);
+    if (!workspace || workspace_bytes < need) return fail(F2_ERR_WORKSPACE, "workspace %zu bytes, need %zu", workspace_bytes, need);
+    DeviceGuard guard(c->device);
+    if (!guard.ok) return fail(F2_ERR_CUDA, "cannot select device %d", c->device);
+    static_assert(sizeof(long long) == sizeof(int64_t), "int64_t layout");
+    F2_CUDA(f2::launch_cnn_forward(c->w, env_t, step, reinterpret_cast<const long long*>(seg_rows),
+                                   reinterpret_cast<const long long*>(seg_frames), n_segs,
+                                   std::min<long long>(total, kCnnChunkFrames), scores, flags, workspace, c->sm_count,
+                                   (cudaStream_t)stream));
+    return F2_OK;
+}
+}  // namespace
+
 int f2_cnn_forward(f2_cnn* c, const float* env_t, int64_t n_rows, int step, int64_t i0, int64_t i1, float* scores,
                    int* flags, void* workspace, size_t workspace_bytes, void* stream) {
     if (!c) return fail(F2_ERR_INVALID, "f2_cnn_forward: null network");
     if (i1 <= i0) return F2_OK;
-    if (!env_t || !scores || !flags || step <= 0 || i0 < 0 || i1 + (int64_t)10 * step > n_rows)
+    // i1 + 10*step > n_rows, written so that no caller value can overflow it
+    if (!env_t || !scores || !flags || step <= 0 || i0 < 0 || n_rows < 0 || i1 > n_rows - (int64_t)10 * step)
         return fail(F2_ERR_INVALID, "f2_cnn_forward: frames [%lld, %lld) x 11 dots of step %d leave the %lld envelope rows",
                     (long long)i0, (long long)i1, step, (long long)n_rows);
-    const size_t need = f2_cnn_workspace_bytes(c, i1 - i0);
-    if (!workspace || workspace_bytes < need) return fail(F2_ERR_WORKSPACE, "workspace %zu bytes, need %zu", workspace_bytes, need);
-    DeviceGuard guard(c->device);
-    if (!guard.ok) return fail(F2_ERR_CUDA, "cannot select device %d", c->device);
-    F2_CUDA(f2::launch_cnn_forward(c->w, env_t, step, i0, i1 - i0, std::min<long long>(i1 - i0, kCnnChunkFrames), scores, flags,
-                                   flags + 1, workspace, c->sm_count, (cudaStream_t)stream));
-    return F2_OK;
+    const int64_t frames = i1 - i0;
+    return cnn_launch(c, env_t, step, &i0, &frames, 1, frames, scores, flags, workspace, workspace_bytes, stream);
+}
+
+int f2_cnn_forward_segments(f2_cnn* c, const float* env_t, int64_t n_rows, int step, const int64_t* seg_rows,
+                            const int64_t* seg_frames, int n_segs, float* scores, int* flags, void* workspace,
+                            size_t workspace_bytes, void* stream) {
+    if (!c) return fail(F2_ERR_INVALID, "f2_cnn_forward_segments: null network");
+    if (n_segs < 0 || (n_segs > 0 && (!seg_rows || !seg_frames)))
+        return fail(F2_ERR_INVALID, "f2_cnn_forward_segments: %d segments, null segment arrays", n_segs);
+    int64_t total = 0;
+    for (int s = 0; s < n_segs; ++s) {
+        if (seg_rows[s] < 0 || seg_frames[s] < 0 || seg_frames[s] > INT64_MAX - total)
+            return fail(F2_ERR_INVALID, "f2_cnn_forward_segments: segment %d has row %lld, %lld frames", s,
+                        (long long)seg_rows[s], (long long)seg_frames[s]);
+        total += seg_frames[s];
+    }
+    if (total == 0) return F2_OK;
+    if (!env_t || !scores || !flags || step <= 0 || n_rows < 0)
+        return fail(F2_ERR_INVALID, "f2_cnn_forward_segments: null pointer, step %d or %lld envelope rows", step,
+                    (long long)n_rows);
+    // frame f of segment s reads rows up to seg_rows[s] + f + 10*step: seg_rows + seg_frames + 10*step <= n_rows,
+    // compared without a sum that caller values could overflow
+    const int64_t last_row = n_rows - (int64_t)10 * step;   // rows a frame may start before
+    for (int s = 0; s < n_segs; ++s)
+        if (seg_frames[s] > 0 && (seg_frames[s] > last_row || seg_rows[s] > last_row - seg_frames[s]))
+            return fail(F2_ERR_INVALID, "f2_cnn_forward_segments: segment %d, %lld frames from row %lld x 11 dots of step %d "
+                        "leave the %lld envelope rows", s, (long long)seg_frames[s], (long long)seg_rows[s], step,
+                        (long long)n_rows);
+    return cnn_launch(c, env_t, step, seg_rows, seg_frames, n_segs, total, scores, flags, workspace, workspace_bytes, stream);
 }
 
 int f2_umma_selftest(const void* a, int a_rows, const void* b, int n, int k, int shift, int variant, float* d, int* status,

@@ -8,6 +8,7 @@
 #include <cuda_bf16.h>
 
 #include <algorithm>
+#include <vector>
 
 #include "f2_umma.cuh"
 
@@ -27,6 +28,9 @@ namespace f2 {
 //   cnn_front_kernel   normalizeInput + conv1 + conv2 + pool   (frames straight from the envelope)
 //   cnn_mid_kernel     conv3 + conv4 + pool -> 1920 features per frame
 //   cnn_dense_kernel   dense 516 + relu + dense 2 + softmax
+// A launch scores a list of segments (frame ranges of one envelope, e.g. the utterances of a batch) whose scores
+// lie back to back; frames run in chunks that cross segment boundaries.  Only cnn_front_kernel knows where a frame
+// comes from (a per-chunk run table, CnnRuns); mid and dense index chunk-local frames.
 // =====================================================================================================
 namespace cnn {
 
@@ -80,9 +84,10 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 }
 
 __global__ void __launch_bounds__(kThreads, 1)
-cnn_front_kernel(const float* __restrict__ env_t, int step, long long frame0, int n_frames, const uint8_t* __restrict__ w1p,
-                 const uint8_t* __restrict__ w2p, const float* __restrict__ b1, const float* __restrict__ b2,
-                 uint8_t* __restrict__ pooled2, int* __restrict__ bad_flag, int* __restrict__ status) {
+cnn_front_kernel(const float* __restrict__ env_t, int step, const CnnRuns runs, int n_frames,
+                 const uint8_t* __restrict__ w1p, const uint8_t* __restrict__ w2p, const float* __restrict__ b1,
+                 const float* __restrict__ b2, uint8_t* __restrict__ pooled2, int* __restrict__ bad_flags,
+                 int* __restrict__ status) {
     extern __shared__ __align__(1024) uint8_t smem[];
     __shared__ __align__(8) uint64_t bar[2];   // issuer -> workers: conv1 / conv2 of the current frame have completed
     __shared__ __align__(8) uint64_t rdy[2];   // workers -> issuer: patch matrix staged + TMEM drained / conv1 output written
@@ -164,11 +169,30 @@ cnn_front_kernel(const float* __restrict__ env_t, int step, long long frame0, in
         const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
         // The envelope samples of a frame are fetched one whole iteration before they are needed (global
         // latency is far longer than anything four warps per scheduler can hide): this thread holds channel
-        // c, dots k0, k0 + 4, k0 + 8 of the NEXT frame to be staged.
+        // c, dots k0, k0 + 4, k0 + 8 of the NEXT frame to be staged, and v_seg the segment that frame belongs to.
         const int c = tid & 127, k0 = tid >> 7;
         float v[3] = {1.f, 1.f, 1.f};
+        int v_seg = 0;
         auto fetch_input = [&](int f) {
-            const float* src = env_t + (size_t)(frame0 + f) * kChan + c;
+            // the last run that starts at or before chunk frame f (every thread looks at the same entries): a
+            // short table is read from the launch parameters at fixed indices (constant bank, no dependent
+            // global load ahead of the envelope reads), a long one is binary-searched in the workspace
+            CnnRun r = runs.inline_runs[0];
+            if (runs.n <= CnnRuns::kInline) {
+#pragma unroll
+                for (int i = 1; i < CnnRuns::kInline; ++i)
+                    if (i < runs.n && runs.inline_runs[i].first <= f) r = runs.inline_runs[i];
+            } else {
+                int a = 0, b = runs.n - 1;
+                while (a < b) {
+                    const int m = (a + b + 1) >> 1;
+                    if (__ldg(&runs.table[m].first) <= f) a = m;
+                    else b = m - 1;
+                }
+                r = runs.table[a];
+            }
+            v_seg = r.seg;
+            const float* src = env_t + (size_t)(r.row + (f - r.first)) * kChan + c;
 #pragma unroll
             for (int j = 0; j < 3; ++j) {
                 const int k = k0 + 4 * j;
@@ -203,7 +227,7 @@ cnn_front_kernel(const float* __restrict__ env_t, int step, long long frame0, in
                 lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
                 hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
             }
-            if (!(lo > 0.f) && tid == 0) atomicOr(bad_flag, 1);   // the reference raises ValueError
+            if (!(lo > 0.f) && tid == 0) atomicOr(bad_flags + v_seg, 1);   // the reference raises ValueError
             // Within a factor 2 of lo, v - lo and hi - lo are exact and log1pf keeps the digits that
             // logf(v) - logf(lo) would cancel (a frame spanning a few ulps gave NaN or several times its span);
             // beyond it (hi - lo) / lo may overflow and the log difference has no cancellation to speak of.
@@ -667,7 +691,8 @@ cnn_dense_kernel(const __nv_bfloat16* __restrict__ feat, int n_frames, const uin
 size_t cnn_workspace_bytes(long long chunk_frames) {
     const size_t pooled = (size_t)chunk_frames * 4 * cnn::kPool2 * 16;
     const size_t feat = (size_t)chunk_frames * cnn::kFeat * 2;
-    return ((pooled + 255) / 256 + (feat + 255) / 256) * 256 + 256;
+    const size_t runs = (size_t)chunk_frames * sizeof(CnnRun);   // a chunk holds at most one run per frame
+    return ((pooled + 255) / 256 + (feat + 255) / 256 + (runs + 255) / 256) * 256 + 256;
 }
 
 cudaError_t configure_cnn_kernels() {
@@ -678,22 +703,47 @@ cudaError_t configure_cnn_kernels() {
     return e;
 }
 
-cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, long long frame0, long long n_frames,
-                               long long chunk_frames, float* scores, int* bad_flag, int* status, void* workspace,
-                               int sm_count, cudaStream_t stream) {
+cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, const long long* seg_rows,
+                               const long long* seg_frames, int n_segs, long long chunk_frames, float* scores, int* flags,
+                               void* workspace, int sm_count, cudaStream_t stream) {
     using namespace cnn;
     uint8_t* pooled2 = (uint8_t*)(((size_t)workspace + 255) / 256 * 256);
     const size_t pooled_bytes = ((size_t)chunk_frames * 4 * kPool2 * 16 + 255) / 256 * 256;
     __nv_bfloat16* feat = (__nv_bfloat16*)(pooled2 + pooled_bytes);
-    for (long long f0 = 0; f0 < n_frames; f0 += chunk_frames) {
-        const int nf = (int)std::min<long long>(chunk_frames, n_frames - f0);
+    const size_t feat_bytes = ((size_t)chunk_frames * kFeat * 2 + 255) / 256 * 256;
+    CnnRun* runs_dev = (CnnRun*)((uint8_t*)feat + feat_bytes);
+    long long total = 0;
+    for (int s = 0; s < n_segs; ++s) total += seg_frames[s];
+    std::vector<CnnRun> runs;
+    CnnRuns param{};
+    param.table = runs_dev;
+    int s0 = 0;            // first segment that still has frames at or after f0
+    long long g0 = 0;      // its first frame in the scores
+    for (long long f0 = 0; f0 < total; f0 += chunk_frames) {
+        const int nf = (int)std::min<long long>(chunk_frames, total - f0);
+        while (s0 < n_segs && g0 + seg_frames[s0] <= f0) g0 += seg_frames[s0++];
+        runs.clear();
+        for (long long s = s0, g = g0; s < n_segs && g < f0 + nf; g += seg_frames[s++]) {
+            if (seg_frames[s] == 0) continue;
+            const long long skip = std::max<long long>(f0 - g, 0);   // frames of the segment in earlier chunks
+            runs.push_back(CnnRun{(int)(g + skip - f0), (int)s, seg_rows[s] + skip});
+        }
+        param.n = (int)runs.size();
+        if (param.n <= CnnRuns::kInline) {
+            std::copy(runs.begin(), runs.end(), param.inline_runs);
+        } else {
+            // pageable source: the copy is staged before the call returns, so `runs` may be refilled right away;
+            // stream order keeps the table of the previous chunk until its front kernel has read it
+            cudaError_t e = cudaMemcpyAsync(runs_dev, runs.data(), runs.size() * sizeof(CnnRun), cudaMemcpyHostToDevice, stream);
+            if (e != cudaSuccess) return e;
+        }
         const int grid = std::min(nf, sm_count);
-        cnn_front_kernel<<<grid, kThreads, FrontSmem::total, stream>>>(env_t, step, frame0 + f0, nf, w.w1, w.w2, w.b1, w.b2, pooled2,
-                                                                  bad_flag, status);
-        cnn_mid_kernel<<<grid, kThreads, MidSmem::total, stream>>>(pooled2, nf, w.w3, w.w4, w.b3, w.b4, feat, status);
+        cnn_front_kernel<<<grid, kThreads, FrontSmem::total, stream>>>(env_t, step, param, nf, w.w1, w.w2, w.b1, w.b2, pooled2,
+                                                                  flags, flags + n_segs);
+        cnn_mid_kernel<<<grid, kThreads, MidSmem::total, stream>>>(pooled2, nf, w.w3, w.w4, w.b3, w.b4, feat, flags + n_segs);
         cnn_dense_kernel<<<(nf + 127) / 128, 128, DenseSmem::total, stream>>>(feat, nf, w.w5, w.b5, w.w6, w.b6, scores + (size_t)f0 * 2,
-                                                                              status);
-        cudaError_t e = cudaGetLastError();
+                                                                              flags + n_segs);
+        const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;

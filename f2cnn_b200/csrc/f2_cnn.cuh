@@ -22,16 +22,39 @@ struct CnnWeights {
     const float* b6;    // [2]
 };
 
+// Frames of one chunk that come from one segment, back to back: chunk frames first .. (the next run's first) - 1
+// belong to segment `seg` and read env_t from row `row` on.  cnn_front_kernel looks a frame's run up
+// in the chunk's table, ordered by `first`.
+struct alignas(16) CnnRun {
+    int first;
+    int seg;
+    long long row;
+};
+// The run table of one chunk as a kernel parameter: up to kInline runs travel with the launch, so that no copy
+// precedes the kernel in the stream (a chunk of utterances of 0.7 s or more has at most four runs; the parameter
+// is kept small because every launch uploads it); a longer table is uploaded to the workspace and `table` points
+// to it.
+struct CnnRuns {
+    static constexpr int kInline = 4;
+    CnnRun inline_runs[kInline];
+    const CnnRun* table;
+    int n;
+};
+
+// Pooled conv2 output, features and the run table of one chunk of chunk_frames frames.
 size_t cnn_workspace_bytes(long long chunk_frames);
 // Raises the dynamic shared-memory limit of the three CNN kernels on the CURRENT device.  A function
 // attribute belongs to one device's copy of the kernel, so every device that runs the network needs this
 // once (f2_cnn_create calls it under its device guard).
 cudaError_t configure_cnn_kernels();
-// Frames frame0 .. frame0 + n_frames - 1 of the time-major envelope env_t ([rows][128] float32): frame i =
-// rows i + k*step, k < 11 (Evaluating.py:70-78).  scores: [n_frames][2] float32 softmax.
-cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, long long frame0, long long n_frames,
-                               long long chunk_frames, float* scores, int* bad_flag, int* status, void* workspace,
-                               int sm_count, cudaStream_t stream);
+// Segment s = seg_frames[s] frames of the time-major envelope env_t ([rows][128] float32) starting at row
+// seg_rows[s]: frame i of it = rows seg_rows[s] + i + k*step, k < 11 (Evaluating.py:70-78).  The segments' frames
+// lie back to back in scores ([sum seg_frames][2] float32 softmax) and are run in chunks of chunk_frames, a chunk
+// crossing segment boundaries.  flags[s] != 0 when a frame of segment s held a value <= 0, flags[n_segs] != 0
+// when the tensor-core pipeline did not complete.  seg_rows / seg_frames are host arrays.
+cudaError_t launch_cnn_forward(const CnnWeights& w, const float* env_t, int step, const long long* seg_rows,
+                               const long long* seg_frames, int n_segs, long long chunk_frames, float* scores, int* flags,
+                               void* workspace, int sm_count, cudaStream_t stream);
 
 cudaError_t launch_umma_selftest(const void* A, int a_rows, const void* B, int N, int K, int shift, int variant, float* D,
                                  int* status, cudaStream_t stream);

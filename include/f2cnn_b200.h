@@ -277,6 +277,9 @@ F2_API int f2_label_fit(const double* formant, const int64_t* first, const int32
 typedef struct f2_cnn f2_cnn;
 F2_API int f2_cnn_create(int device, const float* const* arrays, int dots, int channels, f2_cnn** out);
 F2_API int f2_cnn_destroy(f2_cnn* cnn);
+/* Device workspace of f2_cnn_forward / f2_cnn_forward_segments for n_frames frames: the intermediate tensors of
+ * one chunk of min(n_frames, 32768) frames and room for that chunk's run table (16 bytes per frame, used when a
+ * chunk crosses more segment boundaries than travel with the launch). */
 F2_API size_t f2_cnn_workspace_bytes(const f2_cnn* cnn, int64_t n_frames);
 /* Frames i0 <= i < i1 of env_t ([n_rows][128] float32, device); scores: [i1 - i0][2] float32 softmax
  * (falling, rising), device.  flags: two device ints the caller zeroes: flags[0] != 0 afterwards when a
@@ -284,6 +287,18 @@ F2_API size_t f2_cnn_workspace_bytes(const f2_cnn* cnn, int64_t n_frames);
  * tensor-core pipeline did not complete.  Frames are processed in chunks through `workspace`. */
 F2_API int f2_cnn_forward(f2_cnn* cnn, const float* env_t, int64_t n_rows, int step, int64_t i0, int64_t i1, float* scores,
                           int* flags, void* workspace, size_t workspace_bytes, void* stream);
+/* Many utterances in one pass: segment s is seg_frames[s] frames of env_t starting at row seg_rows[s] (frame i of
+ * it = rows seg_rows[s] + i + k*step, k < 11), e.g. every frame of utterance s of a batch whose env_t holds
+ * several.  seg_rows and seg_frames are HOST arrays of n_segs entries; zero-frame segments are legal.  The
+ * segments' scores lie back to back in `scores` ([sum seg_frames][2] float32, device), and a chunk of frames
+ * crosses segment boundaries, so a corpus of short utterances runs in full chunks.  flags: n_segs + 1 device
+ * ints the caller zeroes: flags[s] != 0 afterwards when a frame of segment s held a value <= 0, flags[n_segs] != 0
+ * when the tensor-core pipeline did not complete.  Workspace: f2_cnn_workspace_bytes(cnn, sum seg_frames).
+ * F2_ERR_INVALID: a negative row or frame count, or a segment whose frames would read past n_rows;
+ * F2_ERR_WORKSPACE: a short workspace.  f2_cnn_forward(i0, i1) is the one segment (i0, i1 - i0). */
+F2_API int f2_cnn_forward_segments(f2_cnn* cnn, const float* env_t, int64_t n_rows, int step, const int64_t* seg_rows,
+                                   const int64_t* seg_frames, int n_segs, float* scores, int* flags, void* workspace,
+                                   size_t workspace_bytes, void* stream);
 /* Where the intermediate tensors of the LAST chunk sit in the workspace (tests compare them layer by layer):
  * pooled conv2 output at the aligned start, [frame][4 planes][4*63 pixels][8 channels] bf16; the 1920
  * features per frame (Keras flatten order) as bf16 at *features_offset. */
