@@ -505,7 +505,8 @@ def features_to_windows_sweep(waves, coefs, timepoints, cutoffs, radius=5, step=
     Every window index must lie on one decimated grid (all indices equal mod `step`), as those of
     LabelDataGenerator's CSV do; anything else raises ValueError (call features_to_windows per cutoff).
     Corpus-sized requests go through engine.WindowPipeline (bit for bit what features_to_windows gives per
-    cutoff); smaller ones take one batch, whose time-chunked utterances all warm up for the lowest cutoff."""
+    cutoff); smaller ones take one batch, whose time-chunked utterances all warm up for the slowest setting (the
+    low-pass pole nearest the unit circle)."""
     settings = list(cutoffs)
     engine.cutoff_settings(settings)
     coefs = np.asarray(coefs, dtype=np.float64)

@@ -850,8 +850,17 @@ int run_sequence(f2_batch* b, const void* wave, int wave_dtype, bool need_env, b
     return F2_OK;
 }
 
-// low-pass warm-up of a mid-signal chunk: |a1|^W < 1e-7
-int lowpass_warmup(double a1) { return round_up_tile(log(1e-7) / log(-a1)); }
+// Low-pass warm-up of a mid-signal chunk: |a1|^W < 1e-7, for either sign of the pole (a1 > 0 above 4 kHz).
+// At least one tile: the output at t0 reads the one-pole state at t0 - 1 even when a1 = 0.  At most
+// kMaxLowpassWarmup, past the longest utterance (2^25 samples): a warm-up that reaches t = 0 starts there, and
+// t0 - w_lpf - w_casc in the fused kernel cannot overflow (cutoffs near 0 or 8000 Hz put |a1| within 1e-9 of 1).
+constexpr int kMaxLowpassWarmup = 1 << 26;
+int lowpass_warmup(double a1) {
+    const double k = fabs(a1);
+    if (!(k < 1.0)) return kMaxLowpassWarmup;
+    const double w = k > 0.0 ? log(1e-7) / log(k) : 0.0;
+    return w < kMaxLowpassWarmup ? std::max(round_up_tile(w), f2::kTile) : kMaxLowpassWarmup;
+}
 }  // namespace
 
 extern "C" {
@@ -912,7 +921,7 @@ int f2_batch_run_cutoffs(f2_batch* b, const void* wave, int wave_dtype, const do
     if (!cutoffs_hz) return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: null cutoffs");
     f2::FusedParams fp{};
     fp.sw_planes = n_settings;
-    double slowest = 0.0;   // a1 of the lowest cutoff: the longest warm-up
+    double slowest = 0.0;   // a1 of the largest |a1| (the lowest cutoff or the highest): the longest warm-up
     for (int j = 0; j < n_settings; ++j) {
         const double f = cutoffs_hz[j];
         fp.sw_state[j] = -1;
@@ -926,7 +935,7 @@ int f2_batch_run_cutoffs(f2_batch* b, const void* wave, int wave_dtype, const do
         fp.sw_state[j] = q;
         fp.sw_k[q] = (float)(-a1);
         fp.sw_b0[q] = (float)b0;
-        if (fp.sw_lp == 1 || -a1 > -slowest) slowest = a1;
+        if (fp.sw_lp == 1 || fabs(a1) > fabs(slowest)) slowest = a1;
     }
     if (!dec) return fail(F2_ERR_INVALID, "f2_batch_run_cutoffs: null dec");
     const int64_t plane = b->total_frames * (int64_t)b->plan->C;
@@ -941,7 +950,7 @@ int f2_batch_run_cutoffs(f2_batch* b, const void* wave, int wave_dtype, const do
         return fail(F2_ERR_WORKSPACE, "workspace %zu bytes, need %zu", workspace_bytes, need);
     fp.dec = dec;
     fp.plane_stride = plane_stride;
-    // the chunk warm-up of the lowest cutoff serves every setting
+    // the chunk warm-up of the slowest setting serves every setting
     fp.lpf = fp.sw_lp > 0 ? 1 : 0;
     fp.w_lpf = fp.sw_lp > 0 ? lowpass_warmup(slowest) : 0;
     return run_sequence(b, wave, wave_dtype, true, false, fp, workspace, nullptr, nullptr, stream);

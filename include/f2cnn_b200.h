@@ -152,8 +152,10 @@ F2_API int f2_batch_run(f2_batch* batch, const f2_run_args* args, void* workspac
  * f2_batch_run with that setting; plane_stride >= total_frames * C lets a sub-batch write its slice of a
  * larger [K][frames][C] array.  dec is device memory or memory pinned with f2_host_pin.  Workspace:
  * f2_batch_workspace_bytes.  Whole-utterance batches give every plane bit for bit what f2_batch_run gives;
- * in a time-chunked batch every chunk warms up for the lowest cutoff, so that cutoff's plane is bit-identical
- * and the others differ from their own runs only by the longer warm-up (below float32 resolution).
+ * in a time-chunked batch every chunk warms up for the slowest setting, the low-pass pole of largest |a1| (the
+ * lowest cutoff, or the highest when it lies nearer 8000 Hz than the lowest lies to 0), so that setting's plane
+ * is bit-identical and the others differ from their own runs only by the longer warm-up (below float32
+ * resolution).  The warm-up bound |a1|^W < 1e-7 holds for either sign of the pole.
  * F2_ERR_INVALID: n_settings outside 1..4, a cutoff that is NaN or outside {0} u (0, 8000), a null dec or a
  * short plane_stride; F2_ERR_WORKSPACE: a short workspace. */
 F2_API int f2_batch_run_cutoffs(f2_batch* batch, const void* wave, int wave_dtype, const double* cutoffs_hz,
