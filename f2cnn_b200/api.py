@@ -771,30 +771,48 @@ def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, 
     processes (one per GPU) handed the same corpus and the same `out` -- a shared mapping,
     hostmem.SharedArray -- scores the utterances engine.shard_utterances deals to `rank` and writes them, and
     only them, at their final offsets.  Only the configured geometry (RADIUS = 5, 128 channels)."""
-    from . import cnn
+    coefs, flat_in, waves, lengths, nb, offsets, sel = _scoring_corpus(waves, coefs, radius, step, shard, out is not None,
+                                                                       "cnn_evaluate_corpus")
+    total = int(offsets[-1])
+    if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"]
+                                and out.shape == (total, 2)):
+        raise ValueError("out must be a C-contiguous float32 array of shape %s" % ((total, 2),))
+    scores = np.empty((total, 2), dtype=np.float32) if out is None else out
+    for _ in _scored_sub_batches(flat_in, waves, lengths, nb, sel, coefs, weights, LPF, CUTOFF, int(step),
+                                 scores, offsets):
+        pass
+    return scores, offsets
+
+
+def _scoring_corpus(waves, coefs, radius, step, shard, shared_out, caller):
+    """The arguments common to the corpus scoring calls, checked -> (coefs, flat host tensor or None, list of waves
+    or None, lengths, frames per utterance nb, score offsets, the utterances this call scores)."""
     coefs = np.asarray(coefs, dtype=np.float64)
     if radius != 5 or coefs.shape[0] != 128:
         raise ValueError("the tensor-core network is built for RADIUS = 5 and 128 channels")
     flat_in, waves, lengths = _waves_lengths(waves)
     if flat_in is not None and flat_in.device.type != "cpu":
-        raise ValueError("cnn_evaluate_corpus takes the flat wave buffer in host memory (it is on %s)" % flat_in.device)
-    step = int(step)
-    nb = np.maximum(lengths - (2 * radius + 1) * step, 0)
+        raise ValueError("%s takes the flat wave buffer in host memory (it is on %s)" % (caller, flat_in.device))
+    nb = np.maximum(lengths - (2 * radius + 1) * int(step), 0)
     offsets = np.concatenate([[0], np.cumsum(nb)]).astype(np.int64)
-    total = int(offsets[-1])
-    if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"]
-                                and out.shape == (total, 2)):
-        raise ValueError("out must be a C-contiguous float32 array of shape %s" % ((total, 2),))
     sel = np.arange(lengths.shape[0])
     if shard is not None:
         rank, world = int(shard[0]), int(shard[1])
-        if out is None or not 0 <= rank < world:
+        if not shared_out or not 0 <= rank < world:
             raise ValueError("shard=(rank, world) needs 0 <= rank < world and the shared `out` array")
         sel = engine.shard_utterances(lengths, world)[rank]
-    scores = np.empty((total, 2), dtype=np.float32) if out is None else out
+    return coefs, flat_in, waves, lengths, nb, offsets, sel
+
+
+def _scored_sub_batches(flat_in, waves, lengths, nb, sel, coefs, weights, LPF, CUTOFF, step, scores=None,
+                        offsets=None):
+    """The utterances `sel` (ascending) through the front end and the network in sub-batches of whole utterances:
+    yields (sub, device scores of sub's frames back to back) per sub-batch; the scores are valid until the next
+    step.  With `scores`, utterance u's rows are also copied to scores[offsets[u]:offsets[u+1]] on the host."""
+    from . import cnn
     sel = sel[nb[sel] > 0]          # an utterance without frames has nothing to score
     if sel.size == 0:
-        return scores, offsets
+        return
     plan = engine.plan_for(coefs)
     net = _network_for(weights)
     # consecutive utterances (in `sel` order) whose envelopes fit _CNN_ENV_BYTES; a larger one goes alone
@@ -814,7 +832,7 @@ def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, 
     stage = torch.empty(max_samples, dtype=wdt, pin_memory=True)
     wave_dev = torch.empty(max_samples, dtype=wdt, device=plan.device)
     env_buf = torch.empty((max_samples, plan.n_channels), dtype=torch.float32, device=plan.device)
-    scores_host = torch.empty((max_frames, 2), dtype=torch.float32, pin_memory=True)
+    scores_host = torch.empty((max_frames, 2), dtype=torch.float32, pin_memory=True) if scores is not None else None
     for sub in subs:
         lens = lengths[sub]
         n = int(lens.sum())
@@ -823,17 +841,130 @@ def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, 
         batch = plan.batch(lens, step=step, target_items=1)
         env_t = batch.run(wave_dev[:n], lpf=LPF, cutoff=CUTOFF, out={"env_t": env_buf[:n]})["env_t"]
         try:
+            # returns after a device synchronise: the staging buffer is free for the next sub-batch
             sc = net.predict_segments(env_t, step, batch.sample_offsets[:-1], nb[sub])
         except cnn.NonPositiveInput as e:
             raise ValueError("values must all be positive (utterance %d)" % int(sub[e.segment])) from None
-        k = int(sc.shape[0])
-        scores_host[:k].copy_(sc)
-        got = scores_host.numpy()
-        at = 0
-        for u in sub:
-            scores[offsets[u]:offsets[u + 1]] = got[at:at + nb[u]]
-            at += int(nb[u])
-    return scores, offsets
+        if scores is not None:
+            k = int(sc.shape[0])
+            scores_host[:k].copy_(sc)
+            got = scores_host.numpy()
+            at = 0
+            for u in sub:
+                scores[offsets[u]:offsets[u + 1]] = got[at:at + nb[u]]
+                at += int(nb[u])
+        yield sub, sc
+
+
+def _label_ints(a, dtype, what):
+    """A 1-D array of integers (integral floats included) that `dtype` holds, as `dtype`; else ValueError."""
+    a = np.asarray(a).reshape(-1)
+    lo, hi = np.iinfo(dtype).min, np.iinfo(dtype).max
+    if a.size:
+        if a.dtype.kind == "f":
+            ok = bool(np.all(np.isfinite(a))) and np.array_equal(np.trunc(a), a) and a.min() >= lo and a.max() < -float(lo)
+        else:
+            ok = a.dtype.kind in "iub" and int(a.min()) >= lo and int(a.max()) <= hi
+        if not ok:
+            raise ValueError("label %s must be integers that %s holds" % (what, np.dtype(dtype).name))
+    return np.ascontiguousarray(a, dtype=dtype)
+
+
+def _label_arrays(times, classes, counts, n_utts):
+    """Flattened labels, checked: (int64 times, int32 classes, int64 label offsets (n_utts + 1)).  ValueError for
+    times and classes of different lengths, non-integer values, counts that do not add up to the number of labels
+    and times that decrease within an utterance."""
+    times, classes = _label_ints(times, np.int64, "times"), _label_ints(classes, np.int32, "classes")
+    counts = _label_ints(counts, np.int64, "counts")
+    if times.shape != classes.shape:
+        raise ValueError("%d label times, %d classes" % (times.shape[0], classes.shape[0]))
+    if counts.shape[0] != n_utts or np.any(counts < 0) or int(counts.sum()) != times.shape[0]:
+        raise ValueError("label counts: one entry per utterance (%d), adding up to the %d labels"
+                         % (n_utts, times.shape[0]))
+    loff = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    falls = np.flatnonzero(np.diff(times) < 0) + 1      # label k is below label k - 1 ...
+    falls = falls[~np.isin(falls, loff)]                 # ... of the same utterance
+    if falls.size:
+        u = int(np.searchsorted(loff, falls[0], side="right")) - 1
+        raise ValueError("label times of utterance %d decrease (label %d)" % (u, int(falls[0] - loff[u])))
+    return times, classes, loff
+
+
+def label_accuracy(scores, labels, step=160):
+    """The reference's label accuracy of one utterance (Evaluating.py:87-110) as two exact integers (hits,
+    counted): accuracy = hits / counted.  scores: the (F, 2) scores of the utterance's stride-1 frames, a host
+    array or a CUDA tensor (float32 on the device; a host array of another dtype is reduced to its decisions
+    s[1] > s[0] first, which rounding it to float32 could change); labels: [(time in samples, class), ...],
+    times non-decreasing, as ExtractLabel gives them.  Frame i counts when it lies strictly between two
+    consecutive label times and closer than `step` to one of them, and hits when its decision equals the class of
+    the nearer label (the earlier one on a tie).  Computed on the GPU (f2_label_accuracy)."""
+    labels = [tuple(l) for l in labels]
+    times, classes, loff = _label_arrays([l[0] for l in labels], [l[1] for l in labels], [len(labels)], 1)
+    if torch.is_tensor(scores) and scores.is_cuda:
+        if scores.dtype != torch.float32 or scores.dim() != 2 or scores.shape[1] != 2:
+            raise ValueError("device scores must be a (F, 2) float32 tensor")
+        sc = scores.contiguous()
+    else:
+        host = scores.numpy() if torch.is_tensor(scores) else np.asarray(scores)
+        if host.ndim != 2 or host.shape[1] != 2:
+            raise ValueError("scores must have shape (F, 2), got %s" % (host.shape,))
+        if host.dtype != np.float32:
+            rising = host[:, 1] > host[:, 0]
+            host = np.zeros(host.shape, dtype=np.float32)
+            host[:, 1] = rising
+        sc = _to_device(np.ascontiguousarray(host), torch.device("cuda", torch.cuda.current_device()))
+    dev = sc.device
+    counts = engine.label_accuracy(sc, _to_device(np.asarray([0, sc.shape[0]], dtype=np.int64), dev),
+                                   _to_device(times, dev), _to_device(classes, dev), _to_device(loff, dev), int(step))
+    hits, counted = _to_host(counts)[:, 0]
+    return int(hits), int(counted)
+
+
+def cnn_label_accuracy_corpus(waves, coefs, weights, labels, LPF=False, CUTOFF=100, radius=5, step=160,
+                              with_scores=False, out=None, shard=None):
+    """The reference's label accuracy (Evaluating.py:87-110) of every utterance of a labelled corpus under one
+    network: cnn_evaluate_corpus, with each sub-batch's scores counted on the device (f2_label_accuracy) before
+    they leave it.  labels = (times, classes, counts): all label times (samples, non-decreasing within an
+    utterance) and classes back to back, counts[u] of them for utterance u -- flattened like the (centres, counts)
+    of features_to_windows.  Returns int64 arrays (hits, counted) of one entry per utterance, utterance u's
+    accuracy being hits[u] / counted[u]; with_scores=True returns (hits, counted, scores, offsets) with the scores
+    and offsets cnn_evaluate_corpus returns.  out=(hits, counted): existing C-contiguous int64 arrays to fill.
+    shard=(rank, world): as in cnn_evaluate_corpus, with `out` the shared pair of arrays; it does not combine with
+    with_scores (cnn_evaluate_corpus scores a shard into a shared array).  Raises ValueError before any launch on
+    malformed labels or another geometry than RADIUS = 5, 128 channels."""
+    if shard is not None and with_scores:
+        raise ValueError("shard= does not combine with with_scores")
+    coefs, flat_in, waves, lengths, nb, offsets, sel = _scoring_corpus(
+        waves, coefs, radius, step, shard, out is not None, "cnn_label_accuracy_corpus")
+    n_utts = int(lengths.shape[0])
+    if len(labels) != 3:
+        raise ValueError("labels = (times, classes, counts)")
+    times, classes, loff = _label_arrays(*labels, n_utts)
+    if out is not None and not (len(out) == 2 and all(
+            isinstance(a, np.ndarray) and a.dtype == np.int64 and a.flags["C_CONTIGUOUS"] and a.shape == (n_utts,)
+            for a in out)):
+        raise ValueError("out must be two C-contiguous int64 arrays of shape (%d,)" % n_utts)
+    hits, counted = (np.zeros(n_utts, np.int64), np.zeros(n_utts, np.int64)) if out is None else out
+    hits[sel] = 0
+    counted[sel] = 0
+    scores = np.empty((int(offsets[-1]), 2), dtype=np.float32) if with_scores else None
+    owner = np.repeat(np.arange(n_utts), np.diff(loff))
+    mine = np.zeros(n_utts, dtype=bool)
+    step = int(step)
+    for sub, sc in _scored_sub_batches(flat_in, waves, lengths, nb, sel, coefs, weights, LPF, CUTOFF, step,
+                                       scores, offsets):
+        dev = sc.device
+        mine[:] = False
+        mine[sub] = True
+        pick = mine[owner]        # sub's labels, in utterance order (sub is ascending)
+        sub_loff = np.concatenate([[0], np.cumsum(np.diff(loff)[sub])]).astype(np.int64)
+        sub_off = np.concatenate([[0], np.cumsum(nb[sub])]).astype(np.int64)
+        got = _to_host(engine.label_accuracy(sc, _to_device(sub_off, dev), _to_device(times[pick], dev),
+                                             _to_device(classes[pick], dev), _to_device(sub_loff, dev), step))
+        hits[sub], counted[sub] = got[0], got[1]
+    if with_scores:
+        return hits, counted, scores, offsets
+    return hits, counted
 
 
 def label_fit(tracks, firsts, centers, radius=5, step=160):

@@ -1350,4 +1350,21 @@ int f2_label_fit(const double* formant, const int64_t* first, const int32_t* cen
     return F2_OK;
 }
 
+int f2_label_accuracy(const float* scores, const int64_t* score_offsets, const int64_t* label_times,
+                      const int32_t* label_classes, const int64_t* label_offsets, int n_utts, int step, int64_t* hits,
+                      int64_t* counted, void* stream) {
+    if (n_utts == 0) return F2_OK;
+    if (n_utts < 0 || step <= 0 || !scores || !score_offsets || !label_times || !label_classes || !label_offsets ||
+        !hits || !counted || ((uintptr_t)scores & 7) != 0)
+        return fail(F2_ERR_INVALID, "f2_label_accuracy: bad arguments (%d utterances, step %d; every pointer non-null, "
+                    "scores 8-byte aligned)", n_utts, step);
+    static_assert(sizeof(long long) == sizeof(int64_t), "int64_t layout");
+    F2_CUDA(f2::launch_label_accuracy(scores, reinterpret_cast<const long long*>(score_offsets),
+                                      reinterpret_cast<const long long*>(label_times), label_classes,
+                                      reinterpret_cast<const long long*>(label_offsets), n_utts, step,
+                                      reinterpret_cast<long long*>(hits), reinterpret_cast<long long*>(counted),
+                                      (cudaStream_t)stream));
+    return F2_OK;
+}
+
 }  // extern "C"

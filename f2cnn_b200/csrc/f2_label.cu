@@ -123,4 +123,83 @@ cudaError_t launch_label_fit(const double* formant, const long long* first, cons
     return cudaGetLastError();
 }
 
+// Label accuracy of `cnn eval*` (scripts/CNN/Evaluating.py:87-110, Evaluating._label_accuracy) for every frame of
+// many utterances.  Frame i of utterance u (utterance-local, compared with the label times in samples as the
+// reference does) decides 1 when s[1] > s[0] (equal scores and NaN decide 0).  The reference scores it against the
+// label pair t_j < i < t_{j+1} whose nearer end is closer than `step`, ties going to the earlier label.  With times
+// non-decreasing the open intervals are disjoint, so the one pair the reference's loop can find is j = (number of
+// times < i) - 1, found by binary search; duplicate times give an empty interval there as well.
+//
+// The frame count lives on the device (score_offsets[n_utts]), so the grid strides over it.  A warp's lanes hold
+// consecutive frames: lanes of one utterance (__match_any_sync) add their ballots with one 64-bit atomic each, and
+// integer sums in any order are exact.
+__global__ void __launch_bounds__(256) label_accuracy_kernel(const float2* __restrict__ scores,
+                                                             const long long* __restrict__ score_offsets,
+                                                             const long long* __restrict__ times,
+                                                             const int* __restrict__ classes,
+                                                             const long long* __restrict__ label_offsets, int n_utts,
+                                                             int step, unsigned long long* __restrict__ hits,
+                                                             unsigned long long* __restrict__ counted) {
+    const int lane = threadIdx.x & 31;
+    const long long first = score_offsets[0], end = score_offsets[n_utts];
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    // the loop test is on the warp's first frame, so whole warps run every iteration (the shuffles need all lanes)
+    for (long long f = first + (long long)blockIdx.x * blockDim.x + threadIdx.x; f - lane < end; f += stride) {
+        int u = -1;
+        bool count = false, hit = false;
+        if (f < end) {
+            // utterance: the last u < n_utts with score_offsets[u] <= f (zero-frame utterances are passed over)
+            int lo = 0, hi = n_utts - 1;
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (score_offsets[mid] <= f) lo = mid; else hi = mid - 1;
+            }
+            u = lo;
+            const long long i = f - score_offsets[u];
+            const long long l0 = label_offsets[u], l1 = label_offsets[u + 1];
+            // first label at or after i: [l0, a) holds the times < i
+            long long a = l0, b = l1;
+            while (a < b) {
+                const long long mid = a + ((b - a) >> 1);
+                if (times[mid] < i) a = mid + 1; else b = mid;
+            }
+            if (a > l0 && a < l1 && times[a] > i) {
+                // the distances are positive and below 2^64 for any int64 times: exact in unsigned arithmetic
+                const unsigned long long d_lo = (unsigned long long)i - (unsigned long long)times[a - 1];
+                const unsigned long long d_hi = (unsigned long long)times[a] - (unsigned long long)i;
+                if (d_lo < (unsigned long long)step || d_hi < (unsigned long long)step) {
+                    const int target = d_lo <= d_hi ? classes[a - 1] : classes[a];
+                    const float2 s = scores[f];
+                    count = true;
+                    hit = (s.y > s.x ? 1 : 0) == target;
+                }
+            }
+        }
+        const unsigned same = __match_any_sync(0xffffffffu, u);
+        const unsigned n_count = __popc(__ballot_sync(0xffffffffu, count) & same);
+        const unsigned n_hit = __popc(__ballot_sync(0xffffffffu, hit) & same);
+        if (u >= 0 && n_count != 0 && lane == __ffs(same) - 1) {
+            atomicAdd(counted + u, (unsigned long long)n_count);
+            if (n_hit != 0) atomicAdd(hits + u, (unsigned long long)n_hit);
+        }
+    }
+}
+
+cudaError_t launch_label_accuracy(const float* scores, const long long* score_offsets, const long long* times,
+                                  const int* classes, const long long* label_offsets, int n_utts, int step,
+                                  long long* hits, long long* counted, cudaStream_t stream) {
+    if (n_utts <= 0) return cudaSuccess;
+    cudaError_t e = cudaMemsetAsync(hits, 0, sizeof(long long) * (size_t)n_utts, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(counted, 0, sizeof(long long) * (size_t)n_utts, stream);
+    if (e != cudaSuccess) return e;
+    int device = 0, sms = 0;
+    if ((e = cudaGetDevice(&device)) != cudaSuccess) return e;
+    if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) return e;
+    // eight 256-thread CTAs fill an SM; the grid strides over frame counts it does not know on the host
+    label_accuracy_kernel<<<(unsigned)sms * 8, 256, 0, stream>>>(
+        reinterpret_cast<const float2*>(scores), score_offsets, times, classes, label_offsets, n_utts, step,
+        reinterpret_cast<unsigned long long*>(hits), reinterpret_cast<unsigned long long*>(counted));
+    return cudaGetLastError();
+}
+
 }  // namespace f2

@@ -414,6 +414,30 @@ def label_fit(formant_dev, first_dev, center_dev, dots, step, stream=None):
     return out
 
 
+def label_accuracy(scores_dev, score_offsets_dev, times_dev, classes_dev, label_offsets_dev, step, stream=None):
+    """Label accuracy counts of Evaluating.py:87-110 for every utterance at once (f2_label_accuracy).
+    scores_dev: contiguous (F, 2) float32; score_offsets_dev, label_offsets_dev: int64 (U+1); times_dev int64 and
+    classes_dev int32, utterance u's labels at label_offsets[u] .. label_offsets[u+1], times non-decreasing.
+    Returns a (2, U) int64 device tensor: hits, counted."""
+    if scores_dev.dtype != torch.float32 or scores_dev.dim() != 2 or scores_dev.shape[1] != 2 \
+            or not scores_dev.is_contiguous():
+        raise TypeError("label_accuracy wants contiguous (F, 2) float32 scores")
+    if score_offsets_dev.dtype != torch.int64 or label_offsets_dev.dtype != torch.int64 \
+            or times_dev.dtype != torch.int64 or classes_dev.dtype != torch.int32:
+        raise TypeError("label_accuracy wants int64 offsets and times, int32 classes")
+    n_utts = int(score_offsets_dev.shape[0]) - 1
+    if n_utts < 0 or int(label_offsets_dev.shape[0]) != n_utts + 1 or times_dev.shape != classes_dev.shape:
+        raise ValueError("label_accuracy: n_utts + 1 offsets of each kind, one class per label time")
+    out = torch.empty((2, n_utts), dtype=torch.int64, device=scores_dev.device)
+    # an empty tensor has no address; the kernel reads none of its entries
+    scores_dev, times_dev, classes_dev = (t if t.numel() else torch.zeros(2, dtype=t.dtype, device=t.device)
+                                          for t in (scores_dev, times_dev, classes_dev))
+    check(_native.lib().f2_label_accuracy(_ptr(scores_dev), _ptr(score_offsets_dev), _ptr(times_dev),
+                                          _ptr(classes_dev), _ptr(label_offsets_dev), n_utts, int(step), _ptr(out[0]),
+                                          _ptr(out[1]), _stream_ptr(stream)))
+    return out
+
+
 def shard_utterances(lengths, world):
     """Length-sorted round-robin deal of utterances over `world` devices (SURVEY.md section 8e; the
     reference's unit of parallelism is the file, GammatoneFiltering.py:121-125): sort by length,

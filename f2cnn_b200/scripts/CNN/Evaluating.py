@@ -8,7 +8,9 @@ reference network on the tensor cores (api.cnn_evaluate -> csrc/f2_cnn.cu, 3.4 m
 46 240 frames of a 3 s utterance) and, transposed, is the matrix the figure shows.  `model` may
 be an .npz of the 12 arrays of model.get_weights() (cnn.save_weights) -- no Keras needed -- or
 a Keras model, whose weights are then read with get_weights(); a geometry other than the
-configured RADIUS = 5 / 128 channels keeps Keras' own predict on the GPU-made frames.  The figure
+configured RADIUS = 5 / 128 channels keeps Keras' own predict on the GPU-made frames.  The
+accuracy heuristic is counted on the GPU as well (api.label_accuracy; _label_accuracy stays as its
+host restatement).  The figure
 still belongs to the reference tree (matplotlib) and is imported where the reference needs it.
 
 Public names, signatures, defaults and side effects (files written under OutputWavFiles/,
@@ -170,7 +172,11 @@ def EvaluateOneWavArray(wavArray, framerate, wavFileName, model='last_trained_mo
         keras.backend.clear_session()
         del network
 
-    accuracy = _label_accuracy(labels, _decisions(scores), step) if labels is not None else None
+    accuracy = None
+    if labels is not None:
+        # the reference's heuristic (:87-110) on the GPU; hits / counted raises ZeroDivisionError as it does there
+        hits, counted = api.label_accuracy(scores, labels, step)
+        accuracy = hits / counted
     print("Plotting...")
     PlotEnvelopesAndCNNResultsWithPhonemes(envelopes, scores, accuracy, centre, phonemes, formants, wavFileName)
 

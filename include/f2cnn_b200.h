@@ -265,6 +265,19 @@ F2_API int f2_host_unpin(void* ptr);
  * arithmetic throughout (the CSV keeps round(a, 5), round(p, 5)). */
 F2_API int f2_label_fit(const double* formant, const int64_t* first, const int32_t* center, int64_t n_items, int dots,
                         int step, double* out, void* stream);
+/* Label accuracy of `cnn eval*` (Evaluating.py:87-110) for many utterances in one launch.  scores: [F][2]
+ * float32 (falling, rising), 8-byte aligned, utterance u's frames at rows score_offsets[u] .. score_offsets[u+1]
+ * (n_utts + 1 non-decreasing entries), as f2_cnn_forward_segments lays them out.  Utterance u's labels are
+ * entries label_offsets[u] .. label_offsets[u+1] of label_times (samples, non-decreasing within the utterance,
+ * as ExtractLabel writes them) and label_classes.  Frame i of an utterance (its own frame number, compared with
+ * the times as the reference does) decides 1 when scores[1] > scores[0] (equal or NaN: 0) and counts when
+ * t_j < i < t_{j+1} for consecutive labels and i - t_j < step or t_{j+1} - i < step; its target is class j when
+ * i - t_j <= t_{j+1} - i, else class j+1.  hits[u] / counted[u] (n_utts int64 each, overwritten) are then the
+ * reference's accuracy.  Every array is device memory; decreasing times or offsets give counts of no meaning.
+ * F2_ERR_INVALID: n_utts < 0, step <= 0, a null pointer or misaligned scores. */
+F2_API int f2_label_accuracy(const float* scores, const int64_t* score_offsets, const int64_t* label_times,
+                             const int32_t* label_classes, const int64_t* label_offsets, int n_utts, int step,
+                             int64_t* hits, int64_t* counted, void* stream);
 
 /* ---- CNN forward of `cnn eval*` on the tensor cores (SURVEY.md section 8f rank 1) ---------------------
  * The reference network (scripts/CNN/Training.py:93-114): Conv32 3x3 same, Conv32 3x3, MaxPool2, Conv64 3x3
