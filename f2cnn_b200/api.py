@@ -30,9 +30,24 @@ def _as_wave(wave):
     return np.ascontiguousarray(w)
 
 
-def _to_device(arr, device):
-    t = torch.from_numpy(arr)
-    if arr.nbytes >= (1 << 16):
+def _as_matrix(matrix):
+    """A (rows, n) matrix as the C ABI takes it: int16, float32 or float64, C-contiguous; anything else is
+    promoted to float64."""
+    m = np.asarray(matrix)
+    if m.dtype not in (np.dtype(np.float32), np.dtype(np.float64), np.dtype(np.int16)):
+        m = m.astype(np.float64)
+    return np.ascontiguousarray(m)
+
+
+def _torch_dtype(dtype):
+    """The output dtype a call was asked for: float64, or float32 for anything else."""
+    return torch.float64 if np.dtype(dtype) == np.float64 else torch.float32
+
+
+def _to_device(a, device):
+    """A host numpy array or tensor on `device`; 64 KiB and more go through pinned memory."""
+    t = torch.from_numpy(a) if isinstance(a, np.ndarray) else a
+    if t.numel() * t.element_size() >= (1 << 16) and not t.is_pinned():
         t = t.pin_memory()
     return t.to(device, non_blocking=True)
 
@@ -44,32 +59,57 @@ def _to_host(t):
     return host.numpy()
 
 
+def _check_out(out, shape, dtype=np.float32, count=None, message=None):
+    """An existing array for a call to fill: a C-contiguous numpy array of `dtype` and `shape` -- with `count`, a
+    sequence of that many, returned as a list.  Anything else raises ValueError(message)."""
+    outs = [out] if count is None else list(out)
+    if (count is not None and len(outs) != count) or not all(
+            isinstance(o, np.ndarray) and o.dtype == dtype and o.flags["C_CONTIGUOUS"] and o.shape == shape
+            for o in outs):
+        raise ValueError(message or "out must be a C-contiguous %s array of shape %s" % (np.dtype(dtype).name, shape))
+    return out if count is None else outs
+
+
+def _utterance(wave, coefs):
+    """One waveform's (host wave, plan, n) for the single-utterance calls."""
+    w = _as_wave(wave)
+    plan = engine.plan_for(np.asarray(coefs, dtype=np.float64))
+    return w, plan, int(w.shape[0])
+
+
+def _run_utterance(plan, w, step=160, phase=0, **outputs):
+    """The fused pass over one host waveform: Batch.run's result dict for the requested `outputs`."""
+    return plan.batch([int(w.shape[0])], step=step, phase=phase).run(_to_device(w, plan.device), **outputs)
+
+
+def _normalised_frames(env_t, dots, step, i0, i1, normalize, dtype):
+    """Dense stride-1 frames i0..i1 of a time-major envelope on the host (Evaluating.py:70-78), normalised per frame
+    (Training.normalizeInput) when `normalize`."""
+    out, flag = engine.dense_frames(env_t, dots, step, i0, i1, normalize=normalize, out_dtype=_torch_dtype(dtype))
+    host = _to_host(out)
+    if normalize and int(flag.item()) != 0:
+        raise ValueError("values must all be positive")  # Training.py:18-20
+    return host
+
+
 def erb_filterbank(wave, coefs, dtype=np.float64):
     """gammatone/filters.py:195-239 -> (C, n) float64 (the reference's dtype; float32 on request)."""
-    w = _as_wave(wave)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    n = int(w.shape[0])
+    w, plan, n = _utterance(wave, coefs)
     if n == 0:
         return np.zeros((plan.n_channels, 0), dtype=dtype)
-    batch = plan.batch([n])
-    res = batch.run(_to_device(w, plan.device), gfb=torch.float64 if np.dtype(dtype) == np.float64 else torch.float32)
+    res = _run_utterance(plan, w, gfb=_torch_dtype(dtype))
     return _to_host(res["gfb"]).reshape(plan.n_channels, n)
 
 
 def filterbank_envelope(wave, coefs, LPF=False, CUTOFF=100, with_gfb=False, dtype=np.float64):
     """Fused erb_filterbank + ExtractEnvelopeFromMatrix on one waveform: the (C,n) envelope
     (and optionally the filterbank output) without the intermediate host round trip."""
-    w = _as_wave(wave)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    n = int(w.shape[0])
-    tdt = torch.float64 if np.dtype(dtype) == np.float64 else torch.float32
+    w, plan, n = _utterance(wave, coefs)
+    tdt = _torch_dtype(dtype)
     if n == 0:
         z = np.zeros((plan.n_channels, 0), dtype=dtype)
         return (z, z.copy()) if with_gfb else z
-    batch = plan.batch([n])
-    res = batch.run(_to_device(w, plan.device), lpf=LPF, cutoff=CUTOFF, env=tdt, gfb=tdt if with_gfb else None)
+    res = _run_utterance(plan, w, lpf=LPF, cutoff=CUTOFF, env=tdt, gfb=tdt if with_gfb else None)
     env = _to_host(res["env"]).reshape(plan.n_channels, n)
     if with_gfb:
         return _to_host(res["gfb"]).reshape(plan.n_channels, n), env
@@ -80,16 +120,13 @@ def gammatonegram(wave, coefs, hop, LPF=False, CUTOFF=100, dtype=np.float64):
     """Every `hop`-th sample of the envelope of `filterbank_envelope` -- (C, ceil(n / hop)), the samples at
     t = 0, hop, 2*hop, ... -- stored by the fused kernel itself: what a plot of a whole file needs
     (scripts/plotting/PlottingProcessing.py:101-109 takes the full-rate matrix for it)."""
-    w = _as_wave(wave)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    n, hop = int(w.shape[0]), int(hop)
+    w, plan, n = _utterance(wave, coefs)
+    hop = int(hop)
     if hop < 1:
         raise ValueError("hop must be >= 1")
     if n == 0:
         return np.zeros((plan.n_channels, 0), dtype=dtype)
-    batch = plan.batch([n], step=hop, phase=0)
-    dec = batch.run(_to_device(w, plan.device), lpf=LPF, cutoff=CUTOFF, dec=True)["dec"]
+    dec = _run_utterance(plan, w, step=hop, lpf=LPF, cutoff=CUTOFF, dec=True)["dec"]
     return np.ascontiguousarray(_to_host(dec).T.astype(dtype, copy=False))
 
 
@@ -97,12 +134,9 @@ def extract_envelope_from_matrix(matrix, LPF=False, CUTOFF=100, dtype=np.float64
     """scripts/processing/EnvelopeExtraction.py:51-67 on an arbitrary (rows, n) matrix:
     abs(paddedHilbert(row)) then lowPassFilter(row, CUTOFF) iff LPF -> float64 (float32 on request),
     same shape."""
-    m = np.asarray(matrix)
-    if m.ndim != 2:
+    if np.ndim(matrix) != 2:
         raise ValueError("matrix must be two-dimensional (channels x samples)")
-    if m.dtype not in (np.dtype(np.float32), np.dtype(np.float64), np.dtype(np.int16)):
-        m = m.astype(np.float64)
-    m = np.ascontiguousarray(m)
+    m = _as_matrix(matrix)
     rows, n = m.shape
     if rows == 0:
         return np.zeros(m.shape, dtype=dtype)
@@ -110,9 +144,7 @@ def extract_envelope_from_matrix(matrix, LPF=False, CUTOFF=100, dtype=np.float64
         # paddedHilbert(empty) -> scipy.signal.hilbert raises "N must be positive."
         raise ValueError("N must be positive.")
     plan = engine.any_plan()
-    out = plan.envelope_rows(_to_device(m, plan.device), LPF, CUTOFF,
-                             out_dtype=torch.float64 if np.dtype(dtype) == np.float64 else torch.float32)
-    return _to_host(out)
+    return _to_host(plan.envelope_rows(_to_device(m, plan.device), LPF, CUTOFF, out_dtype=_torch_dtype(dtype)))
 
 
 class MatrixStream:
@@ -123,23 +155,22 @@ class MatrixStream:
     without another copy while the next batch is computed into the other slot.  A slot is recycled when
     the futures registered with retire() for it have finished.
 
-    mode "filterbank": waves -> erb_filterbank (+ envelope with with_env): process(list of waves).
+    mode "filterbank": waves -> erb_filterbank: process(list of waves).
     mode "envelope":   loaded .GFB matrices -> ExtractEnvelopeFromMatrix: process(list of (C, n) arrays)."""
 
-    def __init__(self, coefs, mode="filterbank", LPF=False, CUTOFF=100, with_env=False, dtype=np.float64,
-                 slot_bytes=768 << 20):
+    def __init__(self, coefs, mode="filterbank", LPF=False, CUTOFF=100, dtype=np.float64, slot_bytes=768 << 20):
         # the envelope of a loaded matrix does not depend on a filterbank: any plan of the device will do
         self.plan = engine.any_plan() if coefs is None else engine.plan_for(np.asarray(coefs, dtype=np.float64))
-        self.mode, self.lpf, self.cutoff, self.with_env = mode, bool(LPF), CUTOFF, bool(with_env)
+        self.mode, self.lpf, self.cutoff = mode, bool(LPF), CUTOFF
         self.dtype = np.dtype(dtype)
-        self.tdt = torch.float64 if self.dtype == np.float64 else torch.float32
+        self.tdt = _torch_dtype(self.dtype)
         self.slot_bytes = int(slot_bytes)
         self._slots = [torch.empty(self.slot_bytes, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
         self._guards = [[], []]
         self._dev = torch.empty(self.slot_bytes, dtype=torch.uint8, device=self.plan.device)
         self._stage = None
         self._k = 0
-        self.per_value = self.dtype.itemsize * (2 if (mode == "filterbank" and with_env) else 1)
+        self.per_value = self.dtype.itemsize   # bytes of one matrix element in a slot
 
     def batches(self, sizes):
         """Split a list of matrix sizes (elements: C * n per utterance) into runs that fit a slot."""
@@ -176,47 +207,32 @@ class MatrixStream:
         stream = torch.cuda.current_stream(self.plan.device)
         views = []
         if self.mode == "filterbank":
-            waves = [_as_wave(w) for w in items]
-            if len({w.dtype for w in waves}) > 1:
-                waves = [w.astype(np.float64) for w in waves]
-            lengths = np.asarray([w.shape[0] for w in waves], dtype=np.int64)
+            _, waves, lengths = _waves_lengths(list(items))
             total = int(lengths.sum())
             if total == 0:
-                z = np.zeros((C, 0), dtype=self.dtype)
-                return [(z, z.copy()) if self.with_env else z for _ in waves]
+                return [np.zeros((C, 0), dtype=self.dtype) for _ in waves]
             wdt = torch.from_numpy(waves[0][:0]).dtype
             stage = self._pinned_stage(total * waves[0].dtype.itemsize).view(wdt)[:total]
             np.concatenate(waves, out=stage.numpy())
             wave_dev = stage.to(self.plan.device, non_blocking=True)
-            nval = C * total
-            out = {"gfb": dev[:nval * self.dtype.itemsize].view(self.tdt)}
-            if self.with_env:
-                out["env"] = dev[nval * self.dtype.itemsize:2 * nval * self.dtype.itemsize].view(self.tdt)
-            self.plan.batch(lengths).run(wave_dev, lpf=self.lpf, cutoff=self.cutoff, out=out, gfb=self.tdt,
-                                         env=self.tdt if self.with_env else None)
-            nbytes = nval * self.per_value
+            nbytes = C * total * self.per_value
+            self.plan.batch(lengths).run(wave_dev, lpf=self.lpf, cutoff=self.cutoff,
+                                         out={"gfb": dev[:nbytes].view(self.tdt)}, gfb=self.tdt)
             slot[:nbytes].copy_(dev[:nbytes], non_blocking=True)
             stream.synchronize()
             host = slot.numpy()
             off = 0
             for n in lengths:
-                sz = C * int(n) * self.dtype.itemsize
-                g = host[off:off + sz].view(self.dtype).reshape(C, int(n))
-                if self.with_env:
-                    e0 = nval * self.dtype.itemsize + off
-                    views.append((g, host[e0:e0 + sz].view(self.dtype).reshape(C, int(n))))
-                else:
-                    views.append(g)
+                sz = C * int(n) * self.per_value
+                views.append(host[off:off + sz].view(self.dtype).reshape(C, int(n)))
                 off += sz
         else:
             off = 0
             placed = []
             for m in items:
-                m = np.asarray(m)
-                if m.ndim != 2:
+                if np.ndim(m) != 2:
                     raise ValueError("matrix must be two-dimensional (channels x samples)")
-                if m.dtype not in (np.dtype(np.float32), np.dtype(np.float64), np.dtype(np.int16)):
-                    m = m.astype(np.float64)
+                m = _as_matrix(m)
                 rows, n = m.shape
                 if n == 0:
                     raise ValueError("N must be positive.")
@@ -236,10 +252,7 @@ class MatrixStream:
 
 
 def _rows_op(matrix, op, lpf, cutoff):
-    m = np.asarray(matrix)
-    if m.dtype not in (np.dtype(np.float32), np.dtype(np.float64), np.dtype(np.int16)):
-        m = m.astype(np.float64)
-    m = np.ascontiguousarray(m)
+    m = _as_matrix(matrix)
     if m.shape[1] == 0:
         raise ValueError("N must be positive.")
     plan = engine.any_plan()
@@ -360,11 +373,17 @@ def _corpus(waves, timepoints, counts):
     return flat_in, waves, lengths, centers, counts
 
 
-def _wave_to_device(flat_in, waves, device):
-    if flat_in is None:
-        flat_in = torch.from_numpy(np.concatenate(waves) if len(waves) > 1 else waves[0])
-    return (flat_in if flat_in.is_pinned() or flat_in.numel() * flat_in.element_size() < (1 << 16)
-            else flat_in.pin_memory()).to(device, non_blocking=True)
+def _shard(lengths, shard, shared_out=None):
+    """shard=(rank, world) -> (the utterances engine.shard_utterances deals to `rank`, world); every utterance and
+    1 without a shard.  shared_out: whether the call was given the `out` array all ranks fill (None: the call
+    writes none)."""
+    if shard is None:
+        return np.arange(lengths.shape[0]), 1
+    rank, world = int(shard[0]), int(shard[1])
+    if (shared_out is not None and not shared_out) or not 0 <= rank < world:
+        raise ValueError("shard=(rank, world) needs 0 <= rank < world" +
+                         ("" if shared_out is None else " and the shared `out` array"))
+    return engine.shard_utterances(lengths, world)[rank], world
 
 
 def _gather_on_grid(dec, idx, phase, step, frame_offsets, dots):
@@ -385,6 +404,107 @@ def _gather_on_grid(dec, idx, phase, step, frame_offsets, dots):
     return res_w.view(rows.shape[0], dots, dec.shape[1])
 
 
+def _windows(waves, coefs, timepoints, counts, radius, step, out, settings=None, LPF=False, CUTOFF=100, shard=None,
+             device_out=False):
+    """The windows of features_to_windows (settings None: the one envelope setting LPF / CUTOFF, Batch.run) and of
+    features_to_windows_sweep (settings: its list, Batch.run_cutoffs), as a list of one result per setting."""
+    sweep = settings is not None
+    K = len(settings) if sweep else 1
+    plan = engine.plan_for(np.asarray(coefs, dtype=np.float64))
+    C = plan.n_channels
+    dots = 2 * radius + 1
+    flat_in, waves, lengths, centers, counts = _corpus(waves, timepoints, counts)
+    n_utts = int(lengths.shape[0])
+    total = int(counts.sum())
+    shape = (total, dots, C)
+    outs = None
+    if out is not None:
+        if sweep:
+            outs = _check_out(out, shape, count=K, message="out must be %d C-contiguous float32 arrays of shape %s"
+                                                          % (K, shape))
+        else:
+            outs = [_check_out(out, shape)]
+            if device_out:
+                raise ValueError("out= is a host array; it cannot be combined with device_out")
+    sel, world = _shard(lengths, shard, shared_out=out is not None)
+    if total == 0:
+        return [np.zeros((0, dots, C), dtype=np.float32) for _ in range(K)] if outs is None else outs
+
+    on_one_grid = False
+    if shard is not None or (not device_out and total * dots * C * 4 >= _PIPELINE_BYTES and n_utts >= 8):
+        # corpus-sized request: decimated frames over PCIe, rows placed on the host (engine.WindowPipeline)
+        first = int(centers[0]) - radius * step
+        phase = first % step if first >= 0 else 0
+        cen, lens, cnts, src_offsets, row_offsets = centers, lengths, counts, None, None
+        if shard is not None:
+            mine = np.zeros(n_utts, dtype=bool)
+            mine[sel] = True
+            cen, lens, cnts = centers[np.repeat(mine, counts)], lengths[sel], counts[sel]
+            src_offsets = (np.cumsum(lengths) - lengths)[sel]
+            row_offsets = (np.cumsum(counts) - counts)[sel]
+        # cheap look at the first utterances before anything is built: a request that is not on one grid
+        # goes straight to the one-batch path
+        head = int(min(8, cnts.shape[0]))
+        n_dec_h = np.where(lens[:head] > phase, (lens[:head] - phase + step - 1) // step, 0)
+        probe, phase_h, _ = engine.window_runs(cen[:int(cnts[:head].sum())], cnts[:head], lens[:head],
+                                               np.concatenate([[0], np.cumsum(n_dec_h)]), radius, step, phase)
+        on_one_grid = probe is not None and phase_h == phase
+    if on_one_grid:
+        pipe = _pipeline_for(plan, lens, dots, step, phase, LPF, CUTOFF, src_offsets, world, cutoffs=settings)
+        results = [engine.host_empty(shape, np.float32) for _ in range(K)] if outs is None else outs
+        state = {}
+
+        def detect():
+            # runs on the host while the first sub-batch is already on the device
+            runs, phase2, _ = engine.window_runs(cen, cnts, lens, pipe.frame_offsets, radius, step, phase,
+                                                 row_offsets=row_offsets)
+            state["ok"] = runs is not None and phase2 == phase
+            return runs if state["ok"] else np.zeros((0, 3), dtype=np.int64)
+
+        pipe.run(flat_in if flat_in is not None else waves if shard is None else [waves[u] for u in sel], detect,
+                 results if sweep else results[0])
+        if state["ok"]:
+            return results
+        # legal timepoints that are not windows of consecutive frames of one grid (a wrapping index, mixed
+        # phases) further down the corpus: nothing was placed; the one-batch path below answers
+        del results
+    if shard is not None:
+        raise ValueError("shard= needs timepoints that are windows of consecutive frames of one decimated grid")
+
+    # one batch, windows gathered on the device
+    cpos = np.concatenate([[0], np.cumsum(counts)])
+    idx = [window_indices(int(n), centers[cpos[u]:cpos[u + 1]], radius, step) for u, n in enumerate(lengths)]
+    # one decimated grid serves every window when all indices share a residue mod step
+    allidx = np.concatenate([i.reshape(-1) for i in idx if i.size])
+    phase = int(allidx[0] % step)
+    on_grid = bool(np.all(allidx % step == phase))
+    if sweep and not on_grid:
+        raise ValueError("features_to_windows_sweep needs every window index on one decimated grid (all equal mod "
+                         "step = %d); call features_to_windows once per cutoff for these timepoints" % step)
+    wave_dev = _to_device(flat_in if flat_in is not None else np.concatenate(waves) if len(waves) > 1 else waves[0],
+                          plan.device)
+    if on_grid:
+        batch = plan.batch(lengths, step=step, phase=phase)
+        planes = (batch.run_cutoffs(wave_dev, settings) if sweep else
+                  [batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, dec=True)["dec"]])
+        res_w = [_gather_on_grid(p, idx, phase, step, batch.frame_offsets, dots) for p in planes]
+    else:
+        # an off-grid request (features_to_windows only): windows gathered from the full-rate envelope
+        batch = plan.batch(lengths, step=step, phase=0)
+        env_t = batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, env_t=True)["env_t"]
+        rows = np.concatenate([i + batch.sample_offsets[u] for u, i in enumerate(idx) if i.size])
+        res_w = [engine.gather_index(env_t, _to_device(np.ascontiguousarray(rows.reshape(-1)), plan.device))
+                 .view(shape)]
+    if device_out:
+        return res_w
+    host = [_to_host(r) for r in res_w]
+    if outs is None:
+        return host
+    for o, h in zip(outs, host):
+        o[...] = h
+    return outs
+
+
 def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=5, step=160, device_out=False,
                         out=None, counts=None, shard=None):
     """Fused path from waveforms to the (N, 2R+1, C) float32 input tensor.
@@ -401,98 +521,8 @@ def features_to_windows(waves, coefs, timepoints, LPF=False, CUTOFF=100, radius=
     handed the SAME corpus and the SAME `out` -- a shared mapping, hostmem.SharedArray.  This call
     computes the utterances engine.shard_utterances deals to `rank` and writes their rows, and only
     theirs, at their final offsets; there is nothing to exchange afterwards."""
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    C = plan.n_channels
-    dots = 2 * radius + 1
-    flat_in, waves, lengths, centers, counts = _corpus(waves, timepoints, counts)
-    n_utts = int(lengths.shape[0])
-    total = int(counts.sum())
-    if out is not None:
-        if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"] and
-                out.shape == (total, dots, C)):
-            raise ValueError("out must be a C-contiguous float32 array of shape %s" % ((total, dots, C),))
-        if device_out:
-            raise ValueError("out= is a host array; it cannot be combined with device_out")
-    if shard is not None:
-        rank, world = int(shard[0]), int(shard[1])
-        if out is None or device_out or not 0 <= rank < world:
-            raise ValueError("shard=(rank, world) needs 0 <= rank < world and the shared `out` array")
-    if total == 0:
-        return np.zeros((0, dots, C), dtype=np.float32) if out is None else out
-
-    if shard is not None or (not device_out and total * dots * C * 4 >= _PIPELINE_BYTES and n_utts >= 8):
-        # corpus-sized request: decimated frames over PCIe, rows placed on the host (engine.WindowPipeline)
-        first = int(centers[0]) - radius * step
-        phase = first % step if first >= 0 else 0
-        sel, src_offsets, row_offsets, share = slice(None), None, None, 1
-        cen, lens, cnts = centers, lengths, counts
-        if shard is not None:
-            sel = engine.shard_utterances(lengths, world)[rank]
-            mine = np.zeros(n_utts, dtype=bool)
-            mine[sel] = True
-            cen, lens, cnts = centers[np.repeat(mine, counts)], lengths[sel], counts[sel]
-            src_offsets = (np.cumsum(lengths) - lengths)[sel]
-            row_offsets = (np.cumsum(counts) - counts)[sel]
-            share = world
-        # cheap look at the first utterances before anything is built: a request that is not on one grid
-        # goes straight to the general path
-        head = int(min(8, cnts.shape[0]))
-        n_dec_h = np.where(lens[:head] > phase, (lens[:head] - phase + step - 1) // step, 0)
-        probe, phase_h, _ = engine.window_runs(cen[:int(cnts[:head].sum())], cnts[:head], lens[:head],
-                                               np.concatenate([[0], np.cumsum(n_dec_h)]), radius, step, phase)
-        on_one_grid = probe is not None and phase_h == phase
-    else:
-        on_one_grid = False
-    if on_one_grid:
-        pipe = _pipeline_for(plan, lens, dots, step, phase, LPF, CUTOFF, src_offsets, share)
-        result = engine.host_empty((total, dots, C), np.float32) if out is None else out
-        state = {}
-
-        def detect():
-            # runs on the host while the first sub-batch is already on the device
-            runs, phase2, _ = engine.window_runs(cen, cnts, lens, pipe.frame_offsets, radius, step, phase,
-                                                 row_offsets=row_offsets)
-            state["ok"] = runs is not None and phase2 == phase
-            return runs if state["ok"] else np.zeros((0, 3), dtype=np.int64)
-
-        if flat_in is not None:
-            pipe.run(flat_in, detect, result)
-        else:
-            pipe.run(waves if shard is None else [waves[u] for u in sel], detect, result)
-        if state["ok"]:
-            return result
-        # legal timepoints that are not windows of consecutive frames of one grid (a wrapping index, mixed
-        # phases) further down the corpus: nothing was placed; the general path below answers
-        del result
-    if shard is not None:
-        raise ValueError("shard= needs timepoints that are windows of consecutive frames of one decimated grid")
-
-    # general path: one batch, windows gathered on the device
-    cpos = np.concatenate([[0], np.cumsum(counts)])
-    idx = [window_indices(int(n), centers[cpos[u]:cpos[u + 1]], radius, step) for u, n in enumerate(lengths)]
-    # one decimated grid serves every window when all indices share a residue mod step
-    allidx = np.concatenate([i.reshape(-1) for i in idx if i.size])
-    phase = int(allidx[0] % step)
-    on_grid = bool(np.all(allidx % step == phase))
-    wave_dev = _wave_to_device(flat_in, waves, plan.device)
-    if on_grid:
-        batch = plan.batch(lengths, step=step, phase=phase)
-        res = batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, dec=True)
-        res_w = _gather_on_grid(res["dec"], idx, phase, step, batch.frame_offsets, dots)
-    else:
-        batch = plan.batch(lengths, step=step, phase=0)
-        res = batch.run(wave_dev, lpf=LPF, cutoff=CUTOFF, env_t=True)
-        rows = np.concatenate([i + batch.sample_offsets[u] for u, i in enumerate(idx) if i.size])
-        res_w = engine.gather_index(res["env_t"], _to_device(np.ascontiguousarray(rows.reshape(-1)), plan.device))
-        res_w = res_w.view(total, dots, C)
-    if device_out:
-        return res_w
-    host = _to_host(res_w)
-    if out is not None:
-        out[...] = host
-        return out
-    return host
+    return _windows(waves, coefs, timepoints, counts, radius, step, out, LPF=LPF, CUTOFF=CUTOFF, shard=shard,
+                    device_out=device_out)[0]
 
 
 def features_to_windows_sweep(waves, coefs, timepoints, cutoffs, radius=5, step=160, counts=None, out=None):
@@ -509,61 +539,7 @@ def features_to_windows_sweep(waves, coefs, timepoints, cutoffs, radius=5, step=
     low-pass pole nearest the unit circle)."""
     settings = list(cutoffs)
     engine.cutoff_settings(settings)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    C = plan.n_channels
-    dots = 2 * radius + 1
-    flat_in, waves, lengths, centers, counts = _corpus(waves, timepoints, counts)
-    n_utts = int(lengths.shape[0])
-    total = int(counts.sum())
-    if out is not None:
-        out = list(out)
-        if len(out) != len(settings) or not all(
-                isinstance(o, np.ndarray) and o.dtype == np.float32 and o.flags["C_CONTIGUOUS"] and
-                o.shape == (total, dots, C) for o in out):
-            raise ValueError("out must be %d C-contiguous float32 arrays of shape %s" % (len(settings), (total, dots, C)))
-    if total == 0:
-        return [np.zeros((0, dots, C), dtype=np.float32) for _ in settings] if out is None else out
-
-    if total * dots * C * 4 >= _PIPELINE_BYTES and n_utts >= 8:
-        first = int(centers[0]) - radius * step
-        phase = first % step if first >= 0 else 0
-        head = int(min(8, n_utts))
-        n_dec_h = np.where(lengths[:head] > phase, (lengths[:head] - phase + step - 1) // step, 0)
-        probe, phase_h, _ = engine.window_runs(centers[:int(counts[:head].sum())], counts[:head], lengths[:head],
-                                               np.concatenate([[0], np.cumsum(n_dec_h)]), radius, step, phase)
-        if probe is not None and phase_h == phase:
-            pipe = _pipeline_for(plan, lengths, dots, step, phase, False, 100, cutoffs=settings)
-            results = [engine.host_empty((total, dots, C), np.float32) for _ in settings] if out is None else out
-            state = {}
-
-            def detect():
-                runs, phase2, _ = engine.window_runs(centers, counts, lengths, pipe.frame_offsets, radius, step, phase)
-                state["ok"] = runs is not None and phase2 == phase
-                return runs if state["ok"] else np.zeros((0, 3), dtype=np.int64)
-
-            pipe.run(flat_in if flat_in is not None else waves, detect, results)
-            if state["ok"]:
-                return results
-            del results
-
-    # one batch, windows gathered on the device from each plane
-    cpos = np.concatenate([[0], np.cumsum(counts)])
-    idx = [window_indices(int(n), centers[cpos[u]:cpos[u + 1]], radius, step) for u, n in enumerate(lengths)]
-    allidx = np.concatenate([i.reshape(-1) for i in idx if i.size])
-    phase = int(allidx[0] % step)
-    if not bool(np.all(allidx % step == phase)):
-        raise ValueError("features_to_windows_sweep needs every window index on one decimated grid (all equal mod "
-                         "step = %d); call features_to_windows once per cutoff for these timepoints" % step)
-    batch = plan.batch(lengths, step=step, phase=phase)
-    planes = batch.run_cutoffs(_wave_to_device(flat_in, waves, plan.device), settings)
-    results = [_to_host(_gather_on_grid(planes[j], idx, phase, step, batch.frame_offsets, dots))
-               for j in range(len(settings))]
-    if out is None:
-        return results
-    for o, r in zip(out, results):
-        o[...] = r
-    return out
+    return _windows(waves, coefs, timepoints, counts, radius, step, out, settings=settings)
 
 
 class FrameWindows:
@@ -640,20 +616,11 @@ def features_to_frames(waves, coefs, LPF=False, CUTOFF=100, radius=5, step=160, 
         counts = np.ascontiguousarray(counts, dtype=np.int64).reshape(-1)
         if counts.shape[0] != lengths.shape[0] or np.any(counts < 0) or np.any(counts + dots - 1 > np.maximum(n_frames, dots - 1)):
             raise IndexError("counts: one entry per utterance, windows must lie inside the utterance's frames")
-    sel, src_offsets, share = np.arange(lengths.shape[0]), None, 1
-    if shard is not None:
-        rank, world = int(shard[0]), int(shard[1])
-        if not 0 <= rank < world:
-            raise ValueError("shard=(rank, world) needs 0 <= rank < world")
-        sel = engine.shard_utterances(lengths, world)[rank]
-        src_offsets = (np.cumsum(lengths) - lengths)[sel]
-        share = world
-    pipe = _pipeline_for(plan, lengths[sel], dots, step, 0, LPF, CUTOFF, src_offsets, share)
+    sel, world = _shard(lengths, shard)
+    pipe = _pipeline_for(plan, lengths[sel], dots, step, 0, LPF, CUTOFF,
+                         None if shard is None else (np.cumsum(lengths) - lengths)[sel], world)
     no_runs = np.zeros((0, 3), dtype=np.int64)
-    if flat_in is not None:
-        pipe.run(flat_in, no_runs, None)
-    else:
-        pipe.run([waves[u] for u in sel], no_runs, None)
+    pipe.run(flat_in if flat_in is not None else [waves[u] for u in sel], no_runs, None)
     return FrameWindows(pipe._dec_host.numpy(), pipe.frame_offsets, counts[sel], dots, sel, pipe.placer)
 
 
@@ -662,10 +629,7 @@ def dense_frames(wave, coefs, LPF=False, CUTOFF=100, radius=5, step=160, normali
     """In-memory front end of Evaluating.EvaluateOneWavArray (Evaluating.py:52-80):
     filterbank -> envelope -> dense stride-1 framing (-> normalizeInput per frame).
     Returns (nb, 2R+1, C); `frames=(i0, i1)` restricts the frame range."""
-    w = _as_wave(wave)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    n = int(w.shape[0])
+    w, plan, n = _utterance(wave, coefs)
     dots = 2 * radius + 1
     nb = int(n - dots * step)
     i0, i1 = (0, nb) if frames is None else (int(frames[0]), int(frames[1]))
@@ -673,44 +637,37 @@ def dense_frames(wave, coefs, LPF=False, CUTOFF=100, radius=5, step=160, normali
         raise IndexError("frames=(%d, %d) outside the %d frames of this utterance" % (i0, i1, max(nb, 0)))
     if nb <= 0 or i1 <= i0:
         return np.zeros((0, dots, plan.n_channels), dtype=dtype)
-    batch = plan.batch([n], step=step)
-    res = batch.run(_to_device(w, plan.device), lpf=LPF, cutoff=CUTOFF, env_t=True)
-    tdt = torch.float64 if np.dtype(dtype) == np.float64 else torch.float32
-    out, flag = engine.dense_frames(res["env_t"], dots, step, i0, i1, normalize=normalize, out_dtype=tdt)
-    host = _to_host(out)
-    if normalize and int(flag.item()) != 0:
-        raise ValueError("values must all be positive")  # Training.py:18-20
-    return host
+    env_t = _run_utterance(plan, w, step=step, lpf=LPF, cutoff=CUTOFF, env_t=True)["env_t"]
+    return _normalised_frames(env_t, dots, step, i0, i1, normalize, dtype)
 
 
 def evaluate_front_end(wave, coefs, LPF=False, CUTOFF=100, radius=5, step=160, frames=True, dtype=np.float64):
     """ONE filterbank pass for `cnn eval*` (Evaluating.py:52-80): the (C, n) envelopes the figure shows
     and the (nb, 2R+1, C) normalised frames model.predict takes, both from the same time-major envelope.
     frames=False returns (envelopes, device env_t) for a consumer on the device (api.cnn_evaluate)."""
-    w = _as_wave(wave)
-    coefs = np.asarray(coefs, dtype=np.float64)
-    plan = engine.plan_for(coefs)
-    n = int(w.shape[0])
+    w, plan, n = _utterance(wave, coefs)
     dots = 2 * radius + 1
     if n == 0:
         raise ValueError("N must be positive.")
-    batch = plan.batch([n], step=step)
-    res = batch.run(_to_device(w, plan.device), lpf=LPF, cutoff=CUTOFF, env=torch.float64, env_t=True)
+    res = _run_utterance(plan, w, step=step, lpf=LPF, cutoff=CUTOFF, env=torch.float64, env_t=True)
     envelopes = _to_host(res["env"]).reshape(plan.n_channels, n)
     if not frames:
         return envelopes, res["env_t"]
     nb = int(n - dots * step)
     if nb <= 0:
         return envelopes, np.zeros((0, dots, plan.n_channels), dtype=dtype)
-    tdt = torch.float64 if np.dtype(dtype) == np.float64 else torch.float32
-    out, flag = engine.dense_frames(res["env_t"], dots, step, 0, nb, normalize=True, out_dtype=tdt)
-    host = _to_host(out)
-    if int(flag.item()) != 0:
-        raise ValueError("values must all be positive")  # Training.py:18-20
-    return envelopes, host
+    return envelopes, _normalised_frames(res["env_t"], dots, step, 0, nb, True, dtype)
 
 
 _networks = OrderedDict()
+
+
+def _check_cnn_geometry(radius, coefs):
+    """coefs as float64, after checking that the tensor-core network takes this geometry."""
+    coefs = np.asarray(coefs, dtype=np.float64)
+    if radius != 5 or coefs.shape[0] != 128:
+        raise ValueError("the tensor-core network is built for RADIUS = 5 and 128 channels")
+    return coefs
 
 
 def _network_for(weights):
@@ -736,18 +693,13 @@ def cnn_evaluate(wave, coefs, weights, LPF=False, CUTOFF=100, radius=5, step=160
     (csrc/f2_cnn.cu), without materialising the (nb, 11, 128) frame tensor.  weights: the 12 arrays of
     Keras' model.get_weights() or an f2cnn_b200.cnn.F2CNN module.  Returns (scores (nb, 2) float32,
     envelopes (C, n) float64 or None).  Only the configured geometry (RADIUS = 5, 128 channels)."""
-    coefs = np.asarray(coefs, dtype=np.float64)
-    if radius != 5 or coefs.shape[0] != 128:
-        raise ValueError("the tensor-core network is built for RADIUS = 5 and 128 channels")
+    coefs = _check_cnn_geometry(radius, coefs)
     net = _network_for(weights)
     if with_envelopes:
         envelopes, env_t = evaluate_front_end(wave, coefs, LPF, CUTOFF, radius, step, frames=False)
     else:
-        w = _as_wave(wave)
-        plan = engine.plan_for(coefs)
-        envelopes = None
-        env_t = plan.batch([int(w.shape[0])], step=step).run(_to_device(w, plan.device), lpf=LPF, cutoff=CUTOFF,
-                                                             env_t=True)["env_t"]
+        w, plan, _ = _utterance(wave, coefs)
+        envelopes, env_t = None, _run_utterance(plan, w, step=step, lpf=LPF, cutoff=CUTOFF, env_t=True)["env_t"]
     scores = net.predict_envelope(env_t, step)
     return _to_host(scores), envelopes
 
@@ -774,10 +726,7 @@ def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, 
     coefs, flat_in, waves, lengths, nb, offsets, sel = _scoring_corpus(waves, coefs, radius, step, shard, out is not None,
                                                                        "cnn_evaluate_corpus")
     total = int(offsets[-1])
-    if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags["C_CONTIGUOUS"]
-                                and out.shape == (total, 2)):
-        raise ValueError("out must be a C-contiguous float32 array of shape %s" % ((total, 2),))
-    scores = np.empty((total, 2), dtype=np.float32) if out is None else out
+    scores = np.empty((total, 2), dtype=np.float32) if out is None else _check_out(out, (total, 2))
     for _ in _scored_sub_batches(flat_in, waves, lengths, nb, sel, coefs, weights, LPF, CUTOFF, int(step),
                                  scores, offsets):
         pass
@@ -787,20 +736,13 @@ def cnn_evaluate_corpus(waves, coefs, weights, LPF=False, CUTOFF=100, radius=5, 
 def _scoring_corpus(waves, coefs, radius, step, shard, shared_out, caller):
     """The arguments common to the corpus scoring calls, checked -> (coefs, flat host tensor or None, list of waves
     or None, lengths, frames per utterance nb, score offsets, the utterances this call scores)."""
-    coefs = np.asarray(coefs, dtype=np.float64)
-    if radius != 5 or coefs.shape[0] != 128:
-        raise ValueError("the tensor-core network is built for RADIUS = 5 and 128 channels")
+    coefs = _check_cnn_geometry(radius, coefs)
     flat_in, waves, lengths = _waves_lengths(waves)
     if flat_in is not None and flat_in.device.type != "cpu":
         raise ValueError("%s takes the flat wave buffer in host memory (it is on %s)" % (caller, flat_in.device))
     nb = np.maximum(lengths - (2 * radius + 1) * int(step), 0)
     offsets = np.concatenate([[0], np.cumsum(nb)]).astype(np.int64)
-    sel = np.arange(lengths.shape[0])
-    if shard is not None:
-        rank, world = int(shard[0]), int(shard[1])
-        if not shared_out or not 0 <= rank < world:
-            raise ValueError("shard=(rank, world) needs 0 <= rank < world and the shared `out` array")
-        sel = engine.shard_utterances(lengths, world)[rank]
+    sel, _ = _shard(lengths, shard, shared_out)
     return coefs, flat_in, waves, lengths, nb, offsets, sel
 
 
@@ -940,11 +882,8 @@ def cnn_label_accuracy_corpus(waves, coefs, weights, labels, LPF=False, CUTOFF=1
     if len(labels) != 3:
         raise ValueError("labels = (times, classes, counts)")
     times, classes, loff = _label_arrays(*labels, n_utts)
-    if out is not None and not (len(out) == 2 and all(
-            isinstance(a, np.ndarray) and a.dtype == np.int64 and a.flags["C_CONTIGUOUS"] and a.shape == (n_utts,)
-            for a in out)):
-        raise ValueError("out must be two C-contiguous int64 arrays of shape (%d,)" % n_utts)
-    hits, counted = (np.zeros(n_utts, np.int64), np.zeros(n_utts, np.int64)) if out is None else out
+    hits, counted = (np.zeros(n_utts, np.int64), np.zeros(n_utts, np.int64)) if out is None else _check_out(
+        out, (n_utts,), np.int64, count=2, message="out must be two C-contiguous int64 arrays of shape (%d,)" % n_utts)
     hits[sel] = 0
     counted[sel] = 0
     scores = np.empty((int(offsets[-1]), 2), dtype=np.float32) if with_scores else None

@@ -190,6 +190,14 @@ class Batch:
     def workspace_bytes(self):
         return int(_native.lib().f2_batch_workspace_bytes(self._h, 0, 0))
 
+    def _check_wave(self, wave_dev):
+        if wave_dev.numel() != self.total_samples:
+            raise ValueError("wave has %d samples, batch expects %d" % (wave_dev.numel(), self.total_samples))
+        if wave_dev.device != self.plan.device:
+            raise ValueError("wave is on %s, plan on %s" % (wave_dev.device, self.plan.device))
+        if not wave_dev.is_contiguous() or wave_dev.dtype not in _T2F2:
+            raise ValueError("wave must be a contiguous int16 / float32 / float64 tensor")
+
     def grid_windows(self, dots=11):
         """The label grid of LabelDataGenerator.py:38-50 on this batch's decimated frames: utterance
         u has nb = max(n // step - dots - 1, 0) windows, window k = frames k .. k+dots-1.  Returns the
@@ -213,12 +221,7 @@ class Batch:
         row_offsets[u] + k); a stand-alone output mode, see grid_windows()."""
         plan = self.plan
         C = plan.n_channels
-        if wave_dev.numel() != self.total_samples:
-            raise ValueError("wave has %d samples, batch expects %d" % (wave_dev.numel(), self.total_samples))
-        if wave_dev.device != plan.device:
-            raise ValueError("wave is on %s, plan on %s" % (wave_dev.device, plan.device))
-        if not wave_dev.is_contiguous() or wave_dev.dtype not in _T2F2:
-            raise ValueError("wave must be a contiguous int16 / float32 / float64 tensor")
+        self._check_wave(wave_dev)
         res = {} if out is None else dict(out)
         # the C ABI takes bare pointers: whatever the caller preallocated is checked here
         want = {"gfb": (C * self.total_samples, (torch.float32, torch.float64)),
@@ -256,18 +259,16 @@ class Batch:
             offs, dots = windows[0], int(windows[1])
             if offs.dtype != torch.int64 or offs.device != plan.device or offs.numel() != len(self.lengths) + 1:
                 raise ValueError("windows offsets: int64 device tensor of n_utts+1 entries")
+            rows = self._grid_rows.get(int(offs.data_ptr()))
+            if rows is None:  # offsets that did not come from grid_windows(): one small D2H read
+                rows = int(offs[-1].item())
             if len(windows) > 2 and windows[2] is not None:
                 res["windows"] = windows[2]
             elif "windows" not in res:
-                rows = self._grid_rows.get(int(offs.data_ptr()))
-                rows = int(offs[-1].item()) if rows is None else rows
                 res["windows"] = torch.empty((rows, dots, C), dtype=torch.float32, device=plan.device)
             w = res["windows"]
             if w.dtype != torch.float32 or not w.is_contiguous() or w.device != plan.device:
                 raise ValueError("windows output: contiguous float32 tensor on the plan's device")
-            rows = self._grid_rows.get(int(offs.data_ptr()))
-            if rows is None:  # offsets that did not come from grid_windows(): one small D2H read
-                rows = int(offs[-1].item())
             if w.numel() < rows * dots * C:
                 raise ValueError("windows output holds %d floats, the offsets ask for %d rows x %d x %d" %
                                  (w.numel(), rows, dots, C))
@@ -289,12 +290,7 @@ class Batch:
         C = plan.n_channels
         hz = cutoff_settings(cutoffs)
         K = len(hz)
-        if wave_dev.numel() != self.total_samples:
-            raise ValueError("wave has %d samples, batch expects %d" % (wave_dev.numel(), self.total_samples))
-        if wave_dev.device != plan.device:
-            raise ValueError("wave is on %s, plan on %s" % (wave_dev.device, plan.device))
-        if not wave_dev.is_contiguous() or wave_dev.dtype not in _T2F2:
-            raise ValueError("wave must be a contiguous int16 / float32 / float64 tensor")
+        self._check_wave(wave_dev)
         if out is None:
             out = torch.empty((K, self.total_frames, C), dtype=torch.float32, device=plan.device)
         mapped = out.device.type == "cpu" and out.is_pinned()
@@ -484,6 +480,14 @@ class _PinnedBlock:
             pass
 
 
+def _block_array(block, nbytes, dtype, count):
+    """`count` elements of `dtype` at the start of an f2_host_alloc block, as a numpy array that keeps the block
+    (its mapping and registration) alive as long as the array or a tensor on it is."""
+    buf = (ctypes.c_char * nbytes).from_address(block.ptr.value)
+    buf._f2_block = block
+    return np.frombuffer(buf, dtype=dtype, count=count)
+
+
 def _pinned_empty(n, dtype):
     """Flat pinned host tensor of n elements; falls back to torch's pinned allocator where registering
     fails (memlock limits, exotic platforms)."""
@@ -493,10 +497,7 @@ def _pinned_empty(n, dtype):
         block = _PinnedBlock(n * esz)
     except Exception:
         return torch.empty(n, dtype=dtype, pin_memory=True)
-    buf = (ctypes.c_char * (n * esz)).from_address(block.ptr.value)
-    buf._f2_block = block   # the registration lives as long as the ctypes view numpy (and the tensor) hold on to
-    np_dt = torch.empty(0, dtype=dtype).numpy().dtype
-    return torch.from_numpy(np.frombuffer(buf, dtype=np_dt, count=n))
+    return torch.from_numpy(_block_array(block, n * esz, torch.empty(0, dtype=dtype).numpy().dtype, n))
 
 
 class WindowPipeline:
@@ -624,7 +625,7 @@ class WindowPipeline:
         edges = np.searchsorted(which, np.arange(len(self.subs) + 1))
         return [np.ascontiguousarray(runs[edges[i]:edges[i + 1]]) for i in range(len(self.subs))]
 
-    def run(self, wave_host, runs, out_host, keep_frames=False):
+    def run(self, wave_host, runs, out_host):
         """wave_host: flat host tensor (int16 / float32 / float64; pinned for full speed -- pageable
         input is staged through a pinned buffer sub-batch by sub-batch) or a list of per-utterance
         numpy arrays; runs: (n, 3) int64 from engine.window_runs on this pipeline's frame_offsets;
@@ -638,12 +639,12 @@ class WindowPipeline:
         gc_was_on = gc.isenabled()
         gc.disable()
         try:
-            return self._run(wave_host, runs, out_host, keep_frames, gc_was_on)
+            return self._run(wave_host, runs, out_host, gc_was_on)
         finally:
             if gc_was_on:
                 gc.enable()
 
-    def _run(self, wave_host, runs, out_host, keep_frames, gc_was_on):
+    def _run(self, wave_host, runs, out_host, gc_was_on):
         caller = torch.cuda.current_stream(self.plan.device)
         dev = self.plan.device
         listed =isinstance(wave_host, (list, tuple))
@@ -1010,7 +1011,4 @@ def host_empty(shape, dtype=np.float32):
     shape = tuple(int(s) for s in shape)
     dt = np.dtype(dtype)
     nbytes = int(np.prod(shape, dtype=np.int64)) * dt.itemsize
-    block = _HostBlock(nbytes)
-    buf = (ctypes.c_char * max(nbytes, 1)).from_address(block.ptr.value)
-    buf._f2_block = block  # the mapping lives as long as the ctypes view numpy holds on to
-    return np.frombuffer(buf, dtype=dt, count=int(np.prod(shape, dtype=np.int64))).reshape(shape)
+    return _block_array(_HostBlock(nbytes), max(nbytes, 1), dt, int(np.prod(shape, dtype=np.int64))).reshape(shape)
